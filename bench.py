@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- BEM assemble + GMRES solve, seconds per frequency (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one frequency of the sweep: dense TBEM assembly of the system matrix + restarted
 GMRES(50) solve to 1e-10 on that matrix.  Default workload = BASELINE.json configs[1]: rigid
@@ -19,6 +19,9 @@ e2e    : the same metric through the public host-buffer API (bem.build_tbem_syst
          bem.gmres): mesh H2D staging, rhs D2H, b H2D and x D2H inside the timed region.
 --impl reference : the CPU oracle (restatement of the reference; the Rust reference cannot be
          built in this image) on the host cores, bounded samples, rank 0 only.
+--dump-outputs DIR : after the timed steps, rank 0 of the native arm writes what the last timed step
+         returned as float64 DIR/<name>.npy (see dump_outputs); the inputs depend on the arguments only,
+         so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -818,6 +821,29 @@ def run_config3(ctx, rank, world, dev, reps=2):
     return block
 
 
+DUMP_SEED = 2024
+DUMP_MATRIX_BYTES = 32 << 20  # the sampled matrix rows; with x and the GMRES figures well under 64 MB for every workload
+
+
+def dump_outputs(out_dir: Path, x: np.ndarray, sol: dict, matrix) -> None:
+    """--dump-outputs: the arrays a caller of the timed path receives for its last step, as float64 .npy files.
+    x.npy                 GMRES solution, n x [re, im]
+    gmres.npy             [iterations, restarts, residual, converged]
+    matrix_rows.npy       rows of the assembled system matrix, k x n x [re, im]: a fixed seeded sample of this rank's
+                          rows (all of them when they fit in DUMP_MATRIX_BYTES)
+    matrix_row_index.npy  the k row indices of matrix_rows.npy, ascending"""
+    n = x.shape[0]
+    r0, r1 = matrix.local_rows
+    k = min(r1 - r0, max(1, DUMP_MATRIX_BYTES // (16 * n)))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(np.arange(r0, r1), size=k, replace=False))
+    a = np.stack([matrix.rows(int(r), int(r) + 1)[0] for r in rows])
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "x.npy", x.view(np.float64).reshape(n, 2))
+    np.save(out_dir / "gmres.npy", np.array([sol["iterations"], sol["restarts"], sol["residual"], sol["converged"]], dtype=np.float64))
+    np.save(out_dir / "matrix_rows.npy", a.view(np.float64).reshape(k, n, 2))
+    np.save(out_dir / "matrix_row_index.npy", rows.astype(np.float64))
+
+
 # -------------------------------------------------------------------------------------------
 # native arm
 # -------------------------------------------------------------------------------------------
@@ -937,6 +963,9 @@ def run_native(args):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     total_ms = float(ms.item())
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # the last timed case was assembled into the driver's buffer (steps - 1) % 2 and solved into x_dev
+        dump_outputs(Path(args.dump_outputs), x_dev.cpu().numpy(), sols[-1], driver.buffers[(args.steps - 1) % 2].matrix)
     stats = []
     for i, sd in enumerate(sols):
         stats.append(dict(sd, **{f"asm_{k}": v for k, v in driver.asm_stats[i].items()},
@@ -1207,7 +1236,12 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="do not overlap assembly(f+1) with solve(f)")
     ap.add_argument("--schedule", choices=["auto", "pipelined", "sequential"], default="auto",
                     help="auto: pipelined sweep on 1 GPU, sequential (persistent fused solver) from 2 GPUs on")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (native arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native arm")
     if args.warmup < 3 and args.impl == "native":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

@@ -24,10 +24,15 @@ tests need the oracle at these sizes at run time:
                      sides (32 independent gmres() calls, the reference's semantics) and the LAPACK solutions of columns
                      0, 13 and 31.
 
-    python tests/golden/make_golden_large.py [config4] [config2] [config3] [config5]
+  rowdot_fsum.npz    the whole-row dot products of config4_rows.npz and config3_rows.npz again, summed with exact_dot: the
+                     same bits on every CPU, where np.dot's summation order follows the BLAS kernel chosen for the processor.
+                     The rows are re-assembled and checked against those two fixtures first.
+
+    python tests/golden/make_golden_large.py [config4] [config2] [config3] [config5] [rowdot]
 
 config2 takes ~8 minutes per frequency on 8 cores (assembly 92 s, LU 4-5 min, GMRES 25 s).
 """
+import math
 import sys
 import time
 from pathlib import Path
@@ -207,8 +212,37 @@ def make_config5():
     print(f"config5: {time.time() - t0:.0f} s, iterations {its}")
 
 
+def exact_dot(a: np.ndarray, x: np.ndarray) -> complex:
+    """sum_j a_j x_j with every product rounded once and each of the two real sums correctly rounded (math.fsum)."""
+    return complex(math.fsum(np.concatenate([a.real * x.real, -(a.imag * x.imag)])),
+                   math.fsum(np.concatenate([a.real * x.imag, a.imag * x.real])))
+
+
+def make_rowdot_fsum():
+    out = {}
+    for name in ("config4", "config3"):
+        g = np.load(OUT / f"{name}_rows.npz")
+        if name == "config4":
+            mesh = generate_geodesic_sphere_mesh(float(g["a"]), int(g["nu"]))
+            ph = PhysicsParams.from_wave_number(float(g["k"]))
+            beta, _ = ph.burton_miller_beta_adaptive(float(g["a"]))
+        else:
+            mesh = cabinet_mesh(1.0)
+            ph = PhysicsParams.new(1000.0, 343.0, 1.21, False)
+            beta = ph.burton_miller_beta()
+        xprobe = config4_probe_vector(mesh.num_dofs)
+        out[name] = np.zeros(len(g["rows"]), dtype=np.complex128)
+        for i, r in enumerate(g["rows"]):
+            A, rh, _ = orc.assemble(mesh, ph.wave_number, beta, row_begin=int(r), row_end=int(r) + 1)
+            assert np.array_equal(A[0, g["cols"][i]], g["vals"][i]) and rh[0] == g["rhs"][i], (name, i)
+            out[name][i] = exact_dot(A[0], xprobe)
+            assert abs(out[name][i] - g["rowdot"][i]) <= 1e-12 * abs(g["rowdot"][i]), (name, i)
+    np.savez_compressed(OUT / "rowdot_fsum.npz", **out)
+    print(f"rowdot_fsum: {len(out['config4'])} + {len(out['config3'])} rows")
+
+
 if __name__ == "__main__":
-    what = sys.argv[1:] or ["config4", "config2", "config3", "config5"]
+    what = sys.argv[1:] or ["config4", "config2", "config3", "config5", "rowdot"]
     if "config5" in what:
         make_config5()
     if "config3" in what:
@@ -217,3 +251,5 @@ if __name__ == "__main__":
         make_config4()
     if "config2" in what:
         make_config2()
+    if "rowdot" in what:
+        make_rowdot_fsum()

@@ -12,6 +12,9 @@ import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 GOLD = ROOT / "tests" / "golden"
+sys.path.insert(0, str(GOLD))
+
+from make_golden_large import exact_dot  # noqa: E402  (the summation rowdot_fsum.npz was made with)
 
 
 def _run_bench(*args, env=None):
@@ -43,6 +46,13 @@ def test_reference_arm_respects_its_budget():
     assert line["steps"] == 2 and line["steps_requested"] == 50  # never fewer than two complete frequencies
 
 
+def test_bench_rejects_no_steps_and_a_dump_of_the_reference_arm(tmp_path):
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "out")]):
+        p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "sphere1k", *args], capture_output=True, text=True, timeout=300)
+        assert p.returncode == 2 and p.stdout == "" and "error:" in p.stderr, args
+    assert not (tmp_path / "out").exists()
+
+
 def test_both_arms_share_the_config_object():
     sys.path.insert(0, str(ROOT))
     import bench
@@ -68,11 +78,12 @@ def test_config4_golden_rows_match_the_oracle():
     assert abs(beta - complex(g["beta"])) == 0.0
     rng = np.random.default_rng(1234)
     xprobe = rng.standard_normal(mesh.num_dofs) + 1j * rng.standard_normal(mesh.num_dofs)
+    rowdot = np.load(GOLD / "rowdot_fsum.npz")["config4"]
     for i in (5, 31):
         r = int(g["rows"][i])
         A, _, _ = orc.assemble(mesh, ph.wave_number, beta, row_begin=r, row_end=r + 1)
         assert np.array_equal(A[0, g["cols"][i]], g["vals"][i])
-        assert np.dot(A[0], xprobe) == g["rowdot"][i]
+        assert exact_dot(A[0], xprobe) == rowdot[i]
         assert r in g["cols"][i][:256]  # the self term is among the nearest columns
 
 
@@ -105,11 +116,12 @@ def test_config3_golden_rows_match_the_oracle():
     rng = np.random.default_rng(1234)
     xprobe = rng.standard_normal(mesh.num_dofs) + 1j * rng.standard_normal(mesh.num_dofs)
     assert np.max(np.abs(g["rhs"])) > 0.0
+    rowdot = np.load(GOLD / "rowdot_fsum.npz")["config3"]
     for i in (1, len(g["rows"]) - 1):
         r = int(g["rows"][i])
         A, rhs, _ = orc.assemble(mesh, ph.wave_number, beta, row_begin=r, row_end=r + 1)
         assert np.array_equal(A[0, g["cols"][i]], g["vals"][i])
-        assert np.dot(A[0], xprobe) == g["rowdot"][i] and rhs[0] == g["rhs"][i]
+        assert exact_dot(A[0], xprobe) == rowdot[i] and rhs[0] == g["rhs"][i]
 
 
 def test_config3_and_config5_solution_fixtures_are_consistent():

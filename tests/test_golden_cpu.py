@@ -1,6 +1,7 @@
 """CPU suite: the oracle against the committed golden fixtures, the host-side logic, and the
 C-ABI library surface (load + exported symbols; no compute without a GPU)."""
 import ctypes as C
+import os
 import re
 from pathlib import Path
 
@@ -13,6 +14,16 @@ from math_audio_b200.types import PhysicsParams
 
 ROOT = Path(__file__).resolve().parent.parent
 GOLD = ROOT / "tests" / "golden"
+
+
+def reference_tree():
+    """The Rust math-audio source tree this port restates, if MATH_AUDIO_REFERENCE names a checkout of it.  It is not part of
+    this repository, so the checks that read it skip without one."""
+    p = os.environ.get("MATH_AUDIO_REFERENCE")
+    return Path(p) if p and Path(p).is_dir() else None
+
+
+NO_REFERENCE = "set MATH_AUDIO_REFERENCE to a checkout of the math-audio Rust sources"
 
 
 def box_piston_mesh():
@@ -209,11 +220,12 @@ def test_rust_manifests_resolve_against_the_reference_workspace():
     assert deps["bem-b200-sys"]["path"] == "../bem-b200-sys"
     expected = {"math-solvers": "math_audio_solvers", "math-bem": "math_audio_bem"}
     src = (root / "rust" / "math-bem-b200" / "src" / "lib.rs").read_text() + (root / "rust" / "math-bem-b200" / "examples" / "frequency_sweep_b200.rs").read_text()
+    reference = reference_tree()
     for pkg, libname in expected.items():
         assert deps[pkg]["path"].endswith(pkg)
         assert re.search(rf"\buse {libname}::", src), libname
-        ref = Path("/root/reference") / pkg / "Cargo.toml"
-        if ref.exists():  # this container only: the package / lib names are the reference's own
+        if reference is not None:  # the package / lib names are the reference's own
+            ref = reference / pkg / "Cargo.toml"
             m = tomllib.loads(ref.read_text())
             assert m["package"]["name"] == pkg and m["lib"]["name"] == libname
             assert "math-bem-b200" not in ref.read_text() and "bem-b200-sys" not in ref.read_text()
@@ -247,13 +259,12 @@ def test_binding_arities_match_the_header():
 
 def test_rust_imports_resolve_to_public_items_of_the_reference():
     """Every `use math_audio_{bem,solvers}::path::{Items}` of the safe crate and its example names a public item of the reference
-    source tree (this container only: /root/reference is absent on the GPU box).  No Rust compiler exists in this image, so this
-    is the nearest thing to name resolution the crates get."""
+    source tree (MATH_AUDIO_REFERENCE).  Without a Rust compiler this is the nearest thing to name resolution the crates get."""
     import re
 
-    ref = Path("/root/reference")
-    if not ref.exists():
-        pytest.skip("/root/reference is only present in the build container")
+    ref = reference_tree()
+    if ref is None:
+        pytest.skip(NO_REFERENCE)
     root = Path(__file__).resolve().parent.parent
     src = (root / "rust" / "math-bem-b200" / "src" / "lib.rs").read_text() + (root / "rust" / "math-bem-b200" / "examples" / "frequency_sweep_b200.rs").read_text()
     crates = {"math_audio_bem": ref / "math-bem" / "src", "math_audio_solvers": ref / "math-solvers" / "src"}
@@ -363,12 +374,12 @@ int main(void) {
 
 def test_qualified_reference_paths_in_the_docs_resolve():
     """Every fully qualified `math_audio_bem::...` / `math_audio_solvers::...` path quoted in INTEGRATION.md, DESIGN.md, README.md
-    and the Rust sources names a module file and a public item of the reference (this container only)."""
+    and the Rust sources names a module file and a public item of the reference (MATH_AUDIO_REFERENCE)."""
     import re
 
-    ref = Path("/root/reference")
-    if not ref.exists():
-        pytest.skip("/root/reference is only present in the build container")
+    ref = reference_tree()
+    if ref is None:
+        pytest.skip(NO_REFERENCE)
     root = Path(__file__).resolve().parent.parent
     crates = {"math_audio_bem": ref / "math-bem" / "src", "math_audio_solvers": ref / "math-solvers" / "src"}
     texts = [(root / n).read_text() for n in ("INTEGRATION.md", "DESIGN.md", "README.md")]
@@ -397,13 +408,13 @@ def test_qualified_reference_paths_in_the_docs_resolve():
 
 def test_reference_citations_resolve():
     """Every `path/file.rs:line[-line]` citation in the headers, the CUDA sources, the Python / C++ / Rust mirrors, the oracle, the
-    tests and the documents names a file of the reference that has that many lines (this container only).  The judge checks parity
+    tests and the documents names a file of the reference that has that many lines (MATH_AUDIO_REFERENCE).  Parity is checked
     through these citations; a stale one is a wrong map."""
     import re
 
-    ref = Path("/root/reference")
-    if not ref.exists():
-        pytest.skip("/root/reference is only present in the build container")
+    ref = reference_tree()
+    if ref is None:
+        pytest.skip(NO_REFERENCE)
     root = Path(__file__).resolve().parent.parent
     by_name, nlines = {}, {}
     for p in ref.rglob("*.rs"):

@@ -830,3 +830,45 @@ def test_config2_sampled_rows_and_solve(bem, orc, big, ka):
         # beta E[1] quadrature residue is O(0.1) here, exactly as in the oracle
         ones = op.apply(np.ones(n, dtype=np.complex128))
         assert np.abs(ones.real + 1.0).max() < 0.05 and np.abs(ones + 1.0).max() < 0.2
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(orc, tmp_path):
+    """bench.py --dump-outputs: float64 arrays within 64 MB holding what the last timed step computed -- the sampled rows of its
+    matrix and its GMRES solution agree with the oracle's assembly and solve of that frequency."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    from math_audio_b200.incident import IncidentField
+
+    root = Path(__file__).resolve().parent.parent
+    steps, warmup = 2, 3
+    p = subprocess.run([sys.executable, str(root / "bench.py"), "--workload", "sphere1k", "--steps", str(steps), "--warmup", str(warmup),
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, env=dict(os.environ, BENCH_NO_CONFIG5="1"), timeout=900)
+    assert p.returncode == 0, p.stderr[-3000:]
+    assert json.loads(p.stdout)["steps"] == steps
+    files = sorted(tmp_path.glob("*.npy"))
+    assert {f.stem for f in files} == {"x", "gmres", "matrix_rows", "matrix_row_index"}
+    assert sum(f.stat().st_size for f in files) <= 64 << 20
+    d = {f.stem: np.load(f) for f in files}
+    assert all(a.dtype == np.float64 for a in d.values())
+    if str(root) not in sys.path:
+        sys.path.insert(0, str(root))
+    import bench
+
+    wl = bench.workload("sphere1k")
+    mesh = wl["mesh"]
+    _, ph, beta = bench.physics_for(wl, warmup + steps - 1)
+    Ao, _, _ = orc.assemble(mesh, ph.wave_number, beta)
+    rows = d["matrix_row_index"].astype(np.int64)
+    assert len(rows) == mesh.num_dofs and (np.diff(rows) > 0).all()  # this small matrix fits the sample whole
+    A = d["matrix_rows"][..., 0] + 1j * d["matrix_rows"][..., 1]
+    assert max(entry_err(A, Ao[rows])) < ENTRY_TOL
+    b = IncidentField.plane_wave_z().compute_rhs_with_beta(mesh.center, mesh.normal, ph, beta)
+    xo, _ = orc.gmres(Ao, b, max_iterations=1000, restart=50, tolerance=1e-10)
+    x = d["x"][:, 0] + 1j * d["x"][:, 1]
+    assert np.linalg.norm(x - xo) / np.linalg.norm(xo) < X_TOL
+    _, _, residual, converged = d["gmres"]
+    assert converged == 1.0 and residual < 1e-10

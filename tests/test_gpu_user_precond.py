@@ -48,10 +48,7 @@ def test_cpp_user_preconditioner_compiles(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.xfail(strict=False, reason="first hardware run of the C++ twin (the Python wrapper of the same C entry is green on a B200)")
 def test_cpp_user_preconditioner_on_gpu(tmp_path):
-    """bemb200::Preconditioner (include/bemb200.hpp) on the device solver.  The Python wrapper of the same C entry is green on a
-    B200 (profiles/r02zz_user_precond.json); this C++ twin was added after the round's GPU minutes were spent, so its first
-    hardware run is the driver's."""
+    """bemb200::Preconditioner (include/bemb200.hpp) on the device solver: the C++ twin of the Python wrapper test above."""
     out = subprocess.run([str(_build_cpp(tmp_path))], capture_output=True, text=True, timeout=240)
     assert out.returncode == 0 and "PASS" in out.stdout, out.stdout + out.stderr
