@@ -7,12 +7,14 @@
 // Krylov basis, Hessenberg matrix, Givens rotations, convergence test, restart counter.  A
 // right-hand side that has converged simply stops taking part (its column of the block still
 // rides along in the matvec).  There is no coupling between the right-hand sides (this is
-// "batched GMRES", not block-Krylov), so results are those of nrhs separate solves.
+// "batched GMRES", not block-Krylov), so results are those of nrhs separate solves.  The host
+// arithmetic of each right-hand side's cycle is the single-RHS solver's (GmresCycle, gmres_host.h).
 #include <cmath>
 #include <cstring>
 #include <vector>
 
 #include "api_internal.h"
+#include "gmres_host.h"
 #include "linalg.h"
 #include "schwarz.h"
 
@@ -24,34 +26,11 @@ int nccl_allgather_bytes(bemb200_ctx* ctx, const void* send, void* recv, size_t 
 
 namespace {
 
-inline double tnorm(cplx a) { return std::sqrt(norm_sqr(a)); }
-void givens_rotation(cplx a, cplx b, cplx* c, cplx* s) {  // gmres.rs:589-603
-    const double tol = 1e-30;
-    if (tnorm(b) < tol) { *c = C(1, 0); *s = C(0, 0); return; }
-    if (tnorm(a) < tol) { *c = C(0, 0); *s = C(1, 0); return; }
-    double r = std::sqrt(norm_sqr(a) + norm_sqr(b));
-    *c = a * C(1.0 / r, 0.0);
-    *s = b * C(1.0 / r, 0.0);
-}
-void solve_upper_triangular(const std::vector<cplx>& h, int ldh, const std::vector<cplx>& g, int k, std::vector<cplx>& y) {
-    y.assign(k, C(0, 0));
-    for (int i = k - 1; i >= 0; --i) {
-        cplx sum = g[i];
-        for (int j = i + 1; j < k; ++j) sum -= h[i * ldh + j] * y[j];
-        cplx d = h[i * ldh + i];
-        if (tnorm(d) > 1e-30) {
-            double ns = norm_sqr(d);
-            y[i] = sum * C(d.re / ns, -d.im / ns);
-        }
-    }
-}
-
 struct Rhs {
     bool active = false;   // still iterating
     bool done = false;     // result final
     double b_norm = 0.0;
-    std::vector<cplx> h, cs, sn, g;
-    bool inner_converged = false;
+    GmresCycle cycle;
     bemb200_gmres_info info{0, 0, 0.0, 0};
 };
 
@@ -235,11 +214,7 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
                 continue;
             }
             r.active = true;
-            r.inner_converged = false;
-            r.h.assign((size_t)(mm + 1) * mm, C(0, 0));
-            r.cs.clear(); r.sn.clear();
-            r.g.assign(mm + 1, C(0, 0));
-            r.g[0] = C(beta, 0.0);
+            r.cycle.start(mm, beta);
             scale[q] = 1.0 / beta;
         }
         if (all_done()) break;
@@ -248,7 +223,6 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
         for (int q = 0; q < S; ++q) active_h[q] = R[q].active ? 1 : 0;
         BEMB_CUDA(ctx, cudaMemcpyAsync(active_d, active_h.data(), S, cudaMemcpyHostToDevice, s));
         BEMB_CUDA(ctx, cudaStreamSynchronize(s));  // `scale` lives on the host stack
-        const int ldh = mm;
         for (int j = 0; j < mm; ++j) {
             bool any_active = false;
             for (int q = 0; q < S; ++q) any_active = any_active || R[q].active;
@@ -265,28 +239,11 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
                 Rhs& r = R[q];
                 if (!r.active) continue;
                 r.info.iterations += 1;
-                const cplx* hc = hcol_h.data() + (size_t)q * hstride;
-                for (int i = 0; i <= j; ++i) r.h[i * ldh + j] = hc[i];
-                const double w_norm = hc[j + 1].re;
-                r.h[(j + 1) * ldh + j] = C(w_norm, 0.0);
-                if (w_norm < 1e-14) r.inner_converged = true;
-                for (int i = 0; i < j; ++i) {
-                    cplx temp = conj(r.cs[i]) * r.h[i * ldh + j] + conj(r.sn[i]) * r.h[(i + 1) * ldh + j];
-                    r.h[(i + 1) * ldh + j] = C(0, 0) - r.sn[i] * r.h[i * ldh + j] + r.cs[i] * r.h[(i + 1) * ldh + j];
-                    r.h[i * ldh + j] = temp;
-                }
-                cplx c, sg;
-                givens_rotation(r.h[j * ldh + j], r.h[(j + 1) * ldh + j], &c, &sg);
-                r.cs.push_back(c); r.sn.push_back(sg);
-                r.h[j * ldh + j] = conj(c) * r.h[j * ldh + j] + conj(sg) * r.h[(j + 1) * ldh + j];
-                r.h[(j + 1) * ldh + j] = C(0, 0);
-                cplx temp = conj(c) * r.g[j] + conj(sg) * r.g[j + 1];
-                r.g[j + 1] = C(0, 0) - sg * r.g[j] + c * r.g[j + 1];
-                r.g[j] = temp;
-                const double rel_res = tnorm(r.g[j + 1]) / r.b_norm;
-                if (rel_res < tolerance || r.inner_converged) {
+                bool breakdown = false;
+                const double rel_res = r.cycle.add_column(j, hcol_h.data() + (size_t)q * hstride, r.b_norm, &breakdown);
+                if (rel_res < tolerance || breakdown) {
                     std::vector<cplx> y;
-                    solve_upper_triangular(r.h, ldh, r.g, j + 1, y);
+                    r.cycle.solve(j + 1, y);
                     for (int i = 0; i < (int)y.size(); ++i) ycoef_h[(size_t)q * mm + i] = y[i];
                     cnt_h[q] = (int)y.size();
                     r.active = false;
@@ -310,7 +267,7 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
             Rhs& r = R[q];
             if (!r.active) continue;
             std::vector<cplx> y;
-            solve_upper_triangular(r.h, ldh, r.g, mm, y);
+            r.cycle.solve(mm, y);
             for (int i = 0; i < (int)y.size(); ++i) ycoef_h[(size_t)q * mm + i] = y[i];
             cnt_h[q] = (int)y.size();
             r.info.restarts += 1;

@@ -1,8 +1,9 @@
 // gmres.cu -- operator application and restarted GMRES on a device-resident, row-sharded
 // matrix.  Host control flow restates math-solvers/src/iterative/gmres.rs:105-277 (restart
-// semantics, iteration counting, Givens with conj(c), conj(s), relative residual vs ||b||,
-// breakdown 1e-14, zero-RHS early return); all O(N) and O(N^2) work runs in the kernels of
-// linalg.cu.
+// semantics, iteration counting, relative residual vs ||b||, zero-RHS early return); the
+// Hessenberg / Givens arithmetic of a cycle (conj(c), conj(s), breakdown 1e-14) is GmresCycle
+// of gmres_host.h, shared with the batched solver.  All O(N) and O(N^2) work runs in the
+// kernels of linalg.cu.
 //
 // Multi-GPU layout ("sharded matvec, replicated Arnoldi"): rank p owns rows
 // [p*chunk,(p+1)*chunk) of A; after the local GEMV the slices of y are all-gathered (NCCL,
@@ -18,6 +19,7 @@
 
 #include "api_internal.h"
 #include "gmres_fused.h"
+#include "gmres_host.h"
 #include "linalg.h"
 #include "schwarz.h"
 
@@ -270,38 +272,10 @@ static void accumulate_matvec_time(bemb200_matrix* m) {
     else cudaGetLastError();
 }
 
-static double g_dbg_launch_us = 0.0, g_dbg_wait_us = 0.0;  // host-side phase timers (diagnostics)
-static double g_dbg_post_ms = 0.0, g_dbg_gap_ms = 0.0;     // device: zgemv-end -> column-on-host, and iteration-to-iteration gap
-static double g_dbg_mgs_ms = 0.0;
-static const bool g_dbg_split = std::getenv("BEMB200_DEBUG_SPLIT") != nullptr;
 static const bool g_speculate = []() {
     const char* v = std::getenv("BEMB200_GMRES_SPECULATE");
     return v ? (std::atoi(v) != 0) : true;
 }();
-
-// ---- host-side pieces of gmres.rs ----------------------------------------------------------
-static inline double tnorm(cplx a) { return std::sqrt(norm_sqr(a)); }  // ComplexField::norm (traits.rs:93-95)
-static void givens_rotation(cplx a, cplx b, cplx* c, cplx* s) {        // gmres.rs:589-603
-    const double tol = 1e-30;
-    if (tnorm(b) < tol) { *c = C(1, 0); *s = C(0, 0); return; }
-    if (tnorm(a) < tol) { *c = C(0, 0); *s = C(1, 0); return; }
-    double r = std::sqrt(norm_sqr(a) + norm_sqr(b));
-    *c = a * C(1.0 / r, 0.0);
-    *s = b * C(1.0 / r, 0.0);
-}
-static void solve_upper_triangular(const std::vector<cplx>& h, int ldh, const std::vector<cplx>& g, int k,
-                                   std::vector<cplx>& y) {  // gmres.rs:606-621
-    y.assign(k, C(0, 0));
-    for (int i = k - 1; i >= 0; --i) {
-        cplx sum = g[i];
-        for (int j = i + 1; j < k; ++j) sum -= h[i * ldh + j] * y[j];
-        cplx d = h[i * ldh + i];
-        if (tnorm(d) > 1e-30) {
-            double ns = norm_sqr(d);
-            y[i] = sum * C(d.re / ns, -d.im / ns);
-        }
-    }
-}
 
 static int norm_of(bemb200_matrix* m, const cplx* b, const cplx* ax, cplx* r, double* out, const cplx* pinv = nullptr) {
     bemb200_ctx* ctx = m->ctx;
@@ -314,27 +288,6 @@ static int norm_of(bemb200_matrix* m, const cplx* b, const cplx* ax, cplx* r, do
     return BEMB200_OK;
 }
 
-// dst (npad, device) = M^-1 src for the Schwarz preconditioner: every rank solves on its slab, then the slabs are gathered
-static int schwarz_full(bemb200_matrix* m, const bemb200_precond* sp, const cplx* src, cplx* dst) {
-    bemb200_ctx* ctx = m->ctx;
-    GmresWorkspace* ws = m->ws;
-    const uint64_t off = ctx->nranks > 1 ? (uint64_t)ctx->rank * ws->chunk : m->r0;
-    BEMB_CUDA(ctx, schwarz_apply_local(sp, src + m->r0, dst + off, ctx->stream));
-    m->last_launches += schwarz_apply_launches(sp);
-    if (ctx->nranks > 1) return nccl_allgather_bytes(ctx, dst + off, dst, ws->chunk * sizeof(cplx));
-    return BEMB200_OK;
-}
-// r = M^-1 (b - A x) with A x in ws->w; *out = ||r||  (gmres.rs:473-476)
-static int schwarz_residual(bemb200_matrix* m, const bemb200_precond* sp, const cplx* b, double* out) {
-    bemb200_ctx* ctx = m->ctx;
-    GmresWorkspace* ws = m->ws;
-    BEMB_CUDA(ctx, launch_residual(b, ws->w, ws->r, m->n_rows, ws->scal_d, nullptr, ctx->stream));  // r = b - A x
-    m->last_launches += 1;
-    int rc = schwarz_full(m, sp, ws->r, ws->w);
-    if (rc != BEMB200_OK) return rc;
-    return norm_of(m, ws->w, nullptr, ws->r, out);  // r = M^-1 (b - A x), its norm
-}
-
 // ---- user preconditioner (bemb200_gmres_callback): Preconditioner::apply (traits.rs:366-371) supplied by the caller as a host
 // function.  The Arnoldi process stays on the device; only M^-1 makes the round trip through two pinned host vectors.
 struct UserPrecond {
@@ -344,28 +297,60 @@ struct UserPrecond {
     cplx* z_h = nullptr;  // pinned, n
     uint64_t calls = 0;
 };
-// dst (device, n) = M^-1 src (device, n); src == dst allowed.  Single rank only (checked by the entry point).
-static int user_full(bemb200_matrix* m, UserPrecond* up, const cplx* src, cplx* dst) {
+
+// The left preconditioner of gmres_preconditioned_with_guess (gmres.rs:434-585); `left` = false is plain gmres_with_guess.
+// With `left`, at most one of the other members is set, and none of them means IdentityPreconditioner.
+struct LeftPrecond {
+    bool left = false;
+    const cplx* pinv = nullptr;                // DiagonalPreconditioner: inverse diagonal on the device, applied inside the
+                                               // residual and Gram-Schmidt kernels
+    const bemb200_precond* schwarz = nullptr;  // additive Schwarz / block-Jacobi (schwarz.cu)
+    UserPrecond* user = nullptr;               // the caller's host function
+    // M^-1 is a step of its own between the matvec and the exchange; the fused kernel and peer mode have no room for it
+    bool own_step() const { return schwarz || user; }
+};
+
+// dst (npad, device) = M^-1 src for a preconditioner with a step of its own; src_loc points at this rank's rows of src.
+// Schwarz: every rank solves on its slab, then the slabs are gathered.  Callback: single rank only (checked by the entry
+// point), so the slab is the whole vector; src_loc == dst allowed.
+static int precond_apply(bemb200_matrix* m, const LeftPrecond& P, const cplx* src_loc, cplx* dst) {
     bemb200_ctx* ctx = m->ctx;
+    GmresWorkspace* ws = m->ws;
+    if (P.schwarz) {
+        const uint64_t off = ctx->nranks > 1 ? (uint64_t)ctx->rank * ws->chunk : m->r0;
+        BEMB_CUDA(ctx, schwarz_apply_local(P.schwarz, src_loc, dst + off, ctx->stream));
+        m->last_launches += schwarz_apply_launches(P.schwarz);
+        if (ctx->nranks > 1) return nccl_allgather_bytes(ctx, dst + off, dst, ws->chunk * sizeof(cplx));
+        return BEMB200_OK;
+    }
+    UserPrecond* up = P.user;
     const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(up->r_h, src, nb, cudaMemcpyDeviceToHost, ctx->stream));
+    BEMB_CUDA(ctx, cudaMemcpyAsync(up->r_h, src_loc, nb, cudaMemcpyDeviceToHost, ctx->stream));
     BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     up->calls += 1;
     const int urc = up->fn(up->user, reinterpret_cast<const double*>(up->r_h), reinterpret_cast<double*>(up->z_h), m->n_rows);
     if (urc != 0) return set_error(ctx, BEMB200_ECALLBACK, "the preconditioner callback returned a non-zero code");
-    // z_h is not touched again before the next user_full has synchronised the stream, i.e. after this copy has completed
+    // z_h is not touched again before the next call has synchronised the stream, i.e. after this copy has completed
     BEMB_CUDA(ctx, cudaMemcpyAsync(dst, up->z_h, nb, cudaMemcpyHostToDevice, ctx->stream));
     return BEMB200_OK;
 }
-// r = M^-1 (b - A x) with A x in ws->w; *out = ||r||  (gmres.rs:473-476)
-static int user_residual(bemb200_matrix* m, UserPrecond* up, const cplx* b, double* out) {
+
+// *out = ||M^-1 (b - A x)|| with A x in ax = ws->w, and M^-1 (b - A x) left in ws->r (gmres.rs:473-476); with ax = nullptr
+// *out = ||M^-1 b|| (gmres.rs:455-457).  M = I without a left preconditioner.
+static int residual_norm(bemb200_matrix* m, const LeftPrecond& P, const cplx* b, const cplx* ax, double* out) {
     bemb200_ctx* ctx = m->ctx;
     GmresWorkspace* ws = m->ws;
-    BEMB_CUDA(ctx, launch_residual(b, ws->w, ws->r, m->n_rows, ws->scal_d, nullptr, ctx->stream));  // r = b - A x
-    m->last_launches += 1;
-    int rc = user_full(m, up, ws->r, ws->w);
+    cplx* r = ax ? ws->r : nullptr;
+    if (!P.own_step()) return norm_of(m, b, ax, r, out, P.pinv);
+    const cplx* src = b;
+    if (ax) {
+        BEMB_CUDA(ctx, launch_residual(b, ax, ws->r, m->n_rows, ws->scal_d, nullptr, ctx->stream));  // r = b - A x
+        m->last_launches += 1;
+        src = ws->r;
+    }
+    int rc = precond_apply(m, P, src + m->r0, ws->w);
     if (rc != BEMB200_OK) return rc;
-    return norm_of(m, ws->w, nullptr, ws->r, out);  // r = M^-1 (b - A x), its norm
+    return norm_of(m, ws->w, nullptr, r, out);
 }
 
 static int update_x(bemb200_matrix* m, cplx* x, const std::vector<cplx>& y) {
@@ -703,45 +688,32 @@ extern "C" void bemb200_debug_fused_times(double* total_ms, double* matvec_ms, d
     g_fused_rounds = 0;
 }
 
-// gmres_with_guess (gmres.rs:105-277) with device vectors b, x (x holds x0 on entry).
-// `precond` selects the left-preconditioned variant gmres_preconditioned_with_guess
-// (gmres.rs:434-585): pinv = inverse diagonal on the device (DiagonalPreconditioner) or nullptr
-// with precond = true (IdentityPreconditioner).
-// `sp`: additive Schwarz / block-Jacobi preconditioner (schwarz.cu) instead of a diagonal one: M^-1 acts on the rank's slab of
-// A v between the ZGEMV and the exchange; the Gram-Schmidt kernel then sees an already preconditioned vector.
+// gmres_with_guess (gmres.rs:105-277) with device vectors b, x (x holds x0 on entry), or with P.left its left-preconditioned
+// variant.  A Schwarz or callback preconditioner acts on the rank's slab of A v between the ZGEMV and the exchange; the
+// Gram-Schmidt kernel then sees an already preconditioned vector.  A diagonal one is applied by that kernel (pinv).
 static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iterations, uint32_t restart, double tol,
-                      bemb200_gmres_info* info, bool precond = false, const cplx* pinv = nullptr, const bemb200_precond* sp = nullptr,
-                      UserPrecond* up = nullptr) {
+                      bemb200_gmres_info* info, const LeftPrecond& P) {
     bemb200_ctx* ctx = m->ctx;
     GmresWorkspace* ws = m->ws;
     const uint64_t n = m->n_rows;
     const int mm = (int)restart;
     cudaStream_t s = ctx->stream;
-    if (!sp && !up) {
+    if (!P.own_step()) {
         bool used = false;
-        int frc = gmres_fused_solve(m, b, x, max_iterations, restart, tol, info, precond, pinv, &used);
+        int frc = gmres_fused_solve(m, b, x, max_iterations, restart, tol, info, P.left, P.pinv, &used);
         if (frc != BEMB200_OK || used) return frc;
     }
     double b_norm = 0.0;
-    int rc = BEMB200_OK;
-    if (sp) {
-        rc = schwarz_full(m, sp, b, ws->w);  // M^-1 b
-        if (rc == BEMB200_OK) rc = norm_of(m, ws->w, nullptr, nullptr, &b_norm);
-    } else if (up) {
-        rc = user_full(m, up, b, ws->w);  // M^-1 b
-        if (rc == BEMB200_OK) rc = norm_of(m, ws->w, nullptr, nullptr, &b_norm);
-    } else {
-        rc = norm_of(m, b, nullptr, nullptr, &b_norm, pinv);  // ||b|| resp. ||M^-1 b|| (gmres.rs:455-457)
-    }
+    int rc = residual_norm(m, P, b, nullptr, &b_norm);  // ||b|| resp. ||M^-1 b||
     if (rc != BEMB200_OK) return rc;
-    const int direct_scale = precond ? 1 : 0;
+    const int direct_scale = P.left ? 1 : 0;
     if (b_norm < 1e-15) {
         *info = bemb200_gmres_info{0, 0, 0.0, 1};
         return BEMB200_OK;
     }
     uint64_t total_iterations = 0, restarts = 0;
-    const int ldh = mm;
-    std::vector<cplx> h, cs, sn, g, y;
+    GmresCycle cycle;
+    std::vector<cplx> y;
     const bool allow_grid = ctx->shared_gpu.load() == 0;
     if (allow_grid) {  // same value on every rank (collective call sequence)
         rc = ensure_peer_exchange(ctx, ws->npad);
@@ -765,7 +737,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
         if (!every) ctx->px.ok = false;
         if (ctx->px.err_h) *ctx->px.err_h = 0;
     }
-    const bool peer_fused = !sp && !up && allow_grid && ctx->nranks > 1 && ctx->px.ok && ctx->px.npad >= ws->npad && ws->npad == ws->chunk * (uint64_t)ctx->nranks &&
+    const bool peer_fused = !P.own_step() && allow_grid && ctx->nranks > 1 && ctx->px.ok && ctx->px.npad >= ws->npad && ws->npad == ws->chunk * (uint64_t)ctx->nranks &&
                             mgs_peer_wait_capable(n, restart, allow_grid);
     static const unsigned long long peer_timeout_ns = []() {
         const char* v = std::getenv("BEMB200_PEER_TIMEOUT_MS");
@@ -780,7 +752,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
         rc = matvec(m, x, ws->w, true);
         if (rc != BEMB200_OK) return rc;
         double beta = 0.0;
-        rc = sp ? schwarz_residual(m, sp, b, &beta) : (up ? user_residual(m, up, b, &beta) : norm_of(m, b, ws->w, ws->r, &beta, pinv));
+        rc = residual_norm(m, P, b, ws->w, &beta);
         if (rc != BEMB200_OK) return rc;
         accumulate_matvec_time(m);
         double rel = beta / b_norm;
@@ -790,11 +762,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
         }
         BEMB_CUDA(ctx, launch_scale(ws->r, 1.0 / beta, ws->V, n, s));
         m->last_launches += 1;
-        h.assign((size_t)(mm + 1) * mm, C(0, 0));
-        cs.clear(); sn.clear();
-        g.assign(mm + 1, C(0, 0));
-        g[0] = C(beta, 0.0);
-        bool inner_converged = false;
+        cycle.start(mm, beta);
         // One Arnoldi iteration = ZGEMV (+ all-gather) + ONE cluster MGS kernel + a (j+2)-number
         // D2H copy.  Iteration j+1 is enqueued BEFORE the host waits for column j, so the GPU never
         // idles on the host round trip; if column j turns out to converge, the speculative
@@ -822,28 +790,20 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
                 pw.timeout_ns = peer_timeout_ns;
             } else {
                 cplx* yloc = ws->w + (ctx->nranks > 1 ? (uint64_t)ctx->rank * ws->chunk : m->r0);
-                BEMB_CUDA(ctx, launch_zgemv(m->A, m->n_cols, nloc, m->n_cols, ws->V + (uint64_t)j * ws->npad, sp ? sp->tmp : yloc, s));
+                cplx* av = P.schwarz ? P.schwarz->tmp : yloc;  // Schwarz: A v_j into scratch, M^-1 writes the rank's rows of w
+                BEMB_CUDA(ctx, launch_zgemv(m->A, m->n_cols, nloc, m->n_cols, ws->V + (uint64_t)j * ws->npad, av, s));
                 BEMB_CUDA(ctx, cudaEventRecord(ws->it_ev1[j], s));
-                if (sp) {  // w = M^-1 (A v_j) on this rank's rows (gmres.rs:513-514)
-                    BEMB_CUDA(ctx, schwarz_apply_local(sp, sp->tmp, yloc, s));
-                    m->last_launches += schwarz_apply_launches(sp);
-                }
-                if (up) {  // w = M^-1 (A v_j) through the caller's function (host round trip of one vector)
-                    int rc3 = user_full(m, up, yloc, yloc);
-                    if (rc3 != BEMB200_OK) return rc3;
-                }
-                if (ctx->nranks > 1) {
-                    int rc2 = nccl_allgather_bytes(ctx, yloc, ws->w, ws->chunk * sizeof(cplx));
-                    if (rc2 != BEMB200_OK) return rc2;
-                }
+                int rc2 = BEMB200_OK;
+                if (P.own_step()) rc2 = precond_apply(m, P, av, ws->w);  // w = M^-1 (A v_j) (gmres.rs:513-514)
+                else if (ctx->nranks > 1) rc2 = nccl_allgather_bytes(ctx, yloc, ws->w, ws->chunk * sizeof(cplx));
+                if (rc2 != BEMB200_OK) return rc2;
             }
             cplx* hd = ws->hcol_d + (size_t)j * ws->ldh_slot;
             bool wrote_host = false;
-            BEMB_CUDA(ctx, launch_mgs(ws->V, ws->npad, const_cast<cplx*>(wvec), j, n, hd, ws->V + (uint64_t)(j + 1) * ws->npad, pinv,
+            BEMB_CUDA(ctx, launch_mgs(ws->V, ws->npad, const_cast<cplx*>(wvec), j, n, hd, ws->V + (uint64_t)(j + 1) * ws->npad, P.pinv,
                                       direct_scale, ws->lmat_d, (int)ws->restart + 1,
                                       ws->lmat_d + (size_t)(ws->restart + 1) * (ws->restart + 1),
                                       ws->hcol_h + (size_t)j * ws->ldh_slot, &wrote_host, allow_grid, pw, ctx->nranks > 1, s));
-            if (g_dbg_split) BEMB_CUDA(ctx, cudaEventRecord(ws->ev0, s));
             if (!wrote_host)
                 BEMB_CUDA(ctx, cudaMemcpyAsync(ws->hcol_h + (size_t)j * ws->ldh_slot, hd, (j + 2) * sizeof(cplx),
                                                cudaMemcpyDeviceToHost, s));
@@ -854,36 +814,22 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
         };
         for (int j = 0; j < mm; ++j) {
             total_iterations += 1;
-            auto tp0 = std::chrono::steady_clock::now();
             if (!ws->launched[j]) {
                 rc = enqueue_iteration(j);
                 if (rc != BEMB200_OK) return rc;
             }
-            if (g_speculate && !up && j + 1 < mm && !ws->launched[j + 1]) {
+            // (never with a callback: the caller's apply runs exactly as often as in the reference)
+            if (g_speculate && !P.user && j + 1 < mm && !ws->launched[j + 1]) {
                 rc = enqueue_iteration(j + 1);
                 if (rc != BEMB200_OK) return rc;
             }
-            auto tp1 = std::chrono::steady_clock::now();
             BEMB_CUDA(ctx, cudaEventSynchronize(ws->it_done[j]));
-            auto tp2 = std::chrono::steady_clock::now();
             {
                 float ms = 0.f;
                 if (cudaEventElapsedTime(&ms, ws->it_ev0[j], ws->it_ev1[j]) == cudaSuccess) m->last_matvec_ms += ms;
                 else cudaGetLastError();
                 m->last_matvecs += 1;  // matvecs whose duration is in last_matvec_ms
-                if (cudaEventElapsedTime(&ms, ws->it_ev1[j], ws->it_done[j]) == cudaSuccess) g_dbg_post_ms += ms;
-                else cudaGetLastError();
-                if (g_dbg_split && !g_speculate) {
-                    if (cudaEventElapsedTime(&ms, ws->it_ev1[j], ws->ev0) == cudaSuccess) g_dbg_mgs_ms += ms;
-                    else cudaGetLastError();
-                }
-                if (j > 0 && ws->launched[j - 1]) {
-                    if (cudaEventElapsedTime(&ms, ws->it_done[j - 1], ws->it_ev0[j]) == cudaSuccess) g_dbg_gap_ms += ms;
-                    else cudaGetLastError();
-                }
             }
-            g_dbg_launch_us += std::chrono::duration<double, std::micro>(tp1 - tp0).count();
-            g_dbg_wait_us += std::chrono::duration<double, std::micro>(tp2 - tp1).count();
             if (peer_err.check()) {
                 // this solve is lost (the peers run into their own bounded waits); later solves of this context use the
                 // NCCL all-gather, which the ranks agree on at the start of the next solve
@@ -891,34 +837,17 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
                 *ctx->px.err_h = 0;
                 return set_error(ctx, BEMB200_ENCCL, "peer-memory exchange timed out waiting for another rank's slab of A v");
             }
-            const cplx* hcol = ws->hcol_h + (size_t)j * ws->ldh_slot;
-            for (int i = 0; i <= j; ++i) h[i * ldh + j] = hcol[i];
-            const double w_norm = hcol[j + 1].re;
-            h[(j + 1) * ldh + j] = C(w_norm, 0.0);
-            if (w_norm < 1e-14) inner_converged = true;  // breakdown: v_{j+1} not formed (gmres.rs:194-202)
-            for (int i = 0; i < j; ++i) {
-                cplx temp = conj(cs[i]) * h[i * ldh + j] + conj(sn[i]) * h[(i + 1) * ldh + j];
-                h[(i + 1) * ldh + j] = C(0, 0) - sn[i] * h[i * ldh + j] + cs[i] * h[(i + 1) * ldh + j];
-                h[i * ldh + j] = temp;
-            }
-            cplx c, sgiv;
-            givens_rotation(h[j * ldh + j], h[(j + 1) * ldh + j], &c, &sgiv);
-            cs.push_back(c); sn.push_back(sgiv);
-            h[j * ldh + j] = conj(c) * h[j * ldh + j] + conj(sgiv) * h[(j + 1) * ldh + j];
-            h[(j + 1) * ldh + j] = C(0, 0);
-            cplx temp = conj(c) * g[j] + conj(sgiv) * g[j + 1];
-            g[j + 1] = C(0, 0) - sgiv * g[j] + c * g[j + 1];
-            g[j] = temp;
-            const double rel_res = tnorm(g[j + 1]) / b_norm;
-            if (rel_res < tol || inner_converged) {
-                solve_upper_triangular(h, ldh, g, j + 1, y);
+            bool breakdown = false;
+            const double rel_res = cycle.add_column(j, ws->hcol_h + (size_t)j * ws->ldh_slot, b_norm, &breakdown);
+            if (rel_res < tol || breakdown) {
+                cycle.solve(j + 1, y);
                 rc = update_x(m, x, y);
                 if (rc != BEMB200_OK) return rc;
                 *info = bemb200_gmres_info{total_iterations, restarts, rel_res, 1};
                 return BEMB200_OK;
             }
         }
-        solve_upper_triangular(h, ldh, g, mm, y);
+        cycle.solve(mm, y);
         rc = update_x(m, x, y);
         if (rc != BEMB200_OK) return rc;
         restarts += 1;
@@ -926,7 +855,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
     rc = matvec(m, x, ws->w, true);
     if (rc != BEMB200_OK) return rc;
     double rn = 0.0;
-    rc = sp ? schwarz_residual(m, sp, b, &rn) : (up ? user_residual(m, up, b, &rn) : norm_of(m, b, ws->w, ws->r, &rn, pinv));
+    rc = residual_norm(m, P, b, ws->w, &rn);
     if (rc != BEMB200_OK) return rc;
     accumulate_matvec_time(m);
     *info = bemb200_gmres_info{total_iterations, restarts, rn / b_norm, 0};
@@ -940,7 +869,15 @@ static inline cplx cdiv(cplx a, cplx b) {
     return C((a.re * b.re + a.im * b.im) / ns, (a.im * b.re - a.re * b.im) / ns);
 }
 
-// b, x: device vectors of n (x is overwritten; the reference starts from x = 0).  Workspace rows
+// the first cnt device scalars of BiCGSTAB / CGS (ws->hcol_d) into their pinned mirror (ws->hcol_h)
+static int fetch_scalars(bemb200_matrix* m, int cnt) {
+    bemb200_ctx* ctx = m->ctx;
+    BEMB_CUDA(ctx, cudaMemcpyAsync(m->ws->hcol_h, m->ws->hcol_d, cnt * sizeof(cplx), cudaMemcpyDeviceToHost, ctx->stream));
+    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return BEMB200_OK;
+}
+
+// b, x: device vectors of n (x = 0 on entry, as the reference starts).  Workspace rows
 // V[0..6] hold r, r0, p, v, s, t; two A-products per iteration through the same (row-sharded)
 // matvec as GMRES; every vector update is fused with the inner products that follow it and the
 // scalars (4 small D2H reads per iteration) drive the reference's control flow on the host.
@@ -957,12 +894,6 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
     cplx* t = ws->V + 5 * ws->npad;
     cplx* dsc = ws->hcol_d;                 // device scalars
     cplx* hsc = ws->hcol_h;                 // pinned mirror
-    auto fetch = [&](int cnt) -> int {
-        BEMB_CUDA(ctx, cudaMemcpyAsync(hsc, dsc, cnt * sizeof(cplx), cudaMemcpyDeviceToHost, s));
-        BEMB_CUDA(ctx, cudaStreamSynchronize(s));
-        return BEMB200_OK;
-    };
-    BEMB_CUDA(ctx, cudaMemsetAsync(x, 0, n * sizeof(cplx), s));
     // r = r0 = b, p = v = 0; (b, b) gives ||b|| and the first rho_new = (r0, r)
     BEMB_CUDA(ctx, cudaMemcpyAsync(r, b, n * sizeof(cplx), cudaMemcpyDeviceToDevice, s));
     BEMB_CUDA(ctx, cudaMemcpyAsync(r0, b, n * sizeof(cplx), cudaMemcpyDeviceToDevice, s));
@@ -970,7 +901,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
     BEMB_CUDA(ctx, cudaMemsetAsync(v, 0, ws->npad * sizeof(cplx), s));
     BEMB_CUDA(ctx, launch_bicg_dot(b, b, n, dsc, s));
     m->last_launches += 1;
-    int rc = fetch(1);
+    int rc = fetch_scalars(m, 1);
     if (rc != BEMB200_OK) return rc;
     const double b_norm = std::sqrt(hsc[0].re);
     if (b_norm < 1e-15) {
@@ -992,7 +923,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
         if (rc != BEMB200_OK) return rc;
         BEMB_CUDA(ctx, launch_bicg_dot(r0, v, n, dsc, s));
         m->last_launches += 2;
-        rc = fetch(1);
+        rc = fetch_scalars(m, 1);
         if (rc != BEMB200_OK) return rc;
         accumulate_matvec_time(m);
         const cplx r0v = hsc[0];
@@ -1003,7 +934,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
         alpha = cdiv(rho, r0v);
         BEMB_CUDA(ctx, launch_bicg_s(r, v, alpha, sv, n, dsc, s));
         m->last_launches += 1;
-        rc = fetch(1);
+        rc = fetch_scalars(m, 1);
         if (rc != BEMB200_OK) return rc;
         const double s_norm = std::sqrt(hsc[0].re);
         if (s_norm / b_norm < tol) {
@@ -1017,7 +948,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
         if (rc != BEMB200_OK) return rc;
         BEMB_CUDA(ctx, launch_bicg_tt(t, sv, n, dsc, s));
         m->last_launches += 1;
-        rc = fetch(2);
+        rc = fetch_scalars(m, 2);
         if (rc != BEMB200_OK) return rc;
         accumulate_matvec_time(m);
         const cplx tt = hsc[0];
@@ -1028,7 +959,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
         omega = cdiv(hsc[1], tt);
         BEMB_CUDA(ctx, launch_bicg_update(x, p, sv, t, r, r0, alpha, omega, n, dsc, s));
         m->last_launches += 1;
-        rc = fetch(2);
+        rc = fetch_scalars(m, 2);
         if (rc != BEMB200_OK) return rc;
         r_norm = std::sqrt(hsc[0].re);
         rho_new = hsc[1];
@@ -1047,7 +978,7 @@ static int bicgstab_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max
 }
 
 // ---- cgs (math-solvers/src/iterative/cgs.rs:46-155) with device vectors ------------------------
-// Workspace rows V[0..7] hold r, r0, p, u, q, v, u+q, w; two A-products per iteration; three fused
+// x = 0 on entry.  Workspace rows V[0..7] hold r, r0, p, u, q, v, u+q, w; two A-products per iteration; three fused
 // vector kernels; 2 scalar read-backs per iteration drive the reference's control flow on the host
 // (including its test of the OLD rho after rho_new has been formed, cgs.rs:122).
 static int cgs_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iterations, double tol, bemb200_gmres_info* info) {
@@ -1065,12 +996,6 @@ static int cgs_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iter
     cplx* w = ws->V + 7 * ws->npad;
     cplx* dsc = ws->hcol_d;
     cplx* hsc = ws->hcol_h;
-    auto fetch = [&](int cnt) -> int {
-        BEMB_CUDA(ctx, cudaMemcpyAsync(hsc, dsc, cnt * sizeof(cplx), cudaMemcpyDeviceToHost, s));
-        BEMB_CUDA(ctx, cudaStreamSynchronize(s));
-        return BEMB200_OK;
-    };
-    BEMB_CUDA(ctx, cudaMemsetAsync(x, 0, n * sizeof(cplx), s));
     // r = r0 = p = u = b; (b, b) gives ||b|| and the first rho = (r0, r)
     for (cplx* dst : {r, r0, p, u}) {
         BEMB_CUDA(ctx, cudaMemsetAsync(dst, 0, ws->npad * sizeof(cplx), s));
@@ -1079,7 +1004,7 @@ static int cgs_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iter
     BEMB_CUDA(ctx, cudaMemsetAsync(uq, 0, ws->npad * sizeof(cplx), s));
     BEMB_CUDA(ctx, launch_bicg_dot(b, b, n, dsc, s));
     m->last_launches += 1;
-    int rc = fetch(1);
+    int rc = fetch_scalars(m, 1);
     if (rc != BEMB200_OK) return rc;
     const double b_norm = std::sqrt(hsc[0].re);
     if (b_norm < 1e-15) {
@@ -1093,7 +1018,7 @@ static int cgs_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iter
         if (rc != BEMB200_OK) return rc;
         BEMB_CUDA(ctx, launch_bicg_dot(r0, v, n, dsc, s));
         m->last_launches += 1;
-        rc = fetch(1);
+        rc = fetch_scalars(m, 1);
         if (rc != BEMB200_OK) return rc;
         accumulate_matvec_time(m);
         const cplx sigma = hsc[0];
@@ -1107,7 +1032,7 @@ static int cgs_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_iter
         if (rc != BEMB200_OK) return rc;
         BEMB_CUDA(ctx, launch_cgs_update(x, uq, w, r, r0, alpha, n, dsc, s));
         m->last_launches += 2;
-        rc = fetch(2);
+        rc = fetch_scalars(m, 2);
         if (rc != BEMB200_OK) return rc;
         accumulate_matvec_time(m);
         r_norm = std::sqrt(hsc[0].re);
@@ -1141,17 +1066,6 @@ static int check_partition(bemb200_matrix* m) {
     return BEMB200_OK;
 }
 
-extern "C" void bemb200_debug_times(double* launch_us, double* wait_us) {
-    *launch_us = g_dbg_launch_us;
-    *wait_us = g_dbg_wait_us;
-    g_dbg_launch_us = g_dbg_wait_us = 0.0;
-}
-extern "C" void bemb200_debug_times2(double* post_ms, double* gap_ms) {
-    *post_ms = g_dbg_post_ms;
-    *gap_ms = g_dbg_mgs_ms > 0.0 ? g_dbg_mgs_ms : g_dbg_gap_ms;
-    g_dbg_post_ms = g_dbg_gap_ms = g_dbg_mgs_ms = 0.0;
-}
-
 static void reset_stats(bemb200_matrix* m) {
     m->last_launches = 0;
     m->last_matvecs = 0;
@@ -1159,22 +1073,58 @@ static void reset_stats(bemb200_matrix* m) {
     m->last_solve_ms = 0.0;
 }
 
-extern "C" {
+// workspace rows V[0..7] of BiCGSTAB and CGS (what GMRES sizes by its restart length)
+constexpr uint32_t BICG_ROWS = 8;
 
-int bemb200_gmres_device(const bemb200_matrix* cm, const double* b_dev, const double* x0_dev, uint32_t max_iterations,
-                         uint32_t restart, double tolerance, double* x_dev, bemb200_gmres_info* info) {
-    bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !b_dev || !x_dev || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+// Argument checks of the solver entry points: `args` = every pointer argument the call needs is non-NULL; `restart` = the
+// GMRES restart length (BICG_ROWS for BiCGSTAB / CGS).
+static int check_solver_args(const bemb200_matrix* m, bool args, const char* solver, uint32_t restart) {
+    if (!m || !args) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    if (m->n_rows != m->n_cols) return set_error(m->ctx, BEMB200_EINVAL, std::string(solver) + " needs a square operator");
+    if (restart == 0) return set_error(m->ctx, BEMB200_EINVAL, "restart must be >= 1");
+    return BEMB200_OK;
+}
+
+// The start of a solver or operator call after its argument checks, with ctx->mu held: device, partition check, a
+// workspace for `restart` Krylov vectors, fresh statistics.
+static int begin_call(bemb200_matrix* m, uint32_t restart) {
     bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "gmres needs a square operator");
-    if (restart == 0) return set_error(ctx, BEMB200_EINVAL, "restart must be >= 1");
-    std::lock_guard<std::mutex> lk(ctx->mu);
     BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
     int rc = check_partition(m);
     if (rc != BEMB200_OK) return rc;
     rc = ensure_workspace(m, restart);
     if (rc != BEMB200_OK) return rc;
     reset_stats(m);
+    return BEMB200_OK;
+}
+
+// A solve on host vectors: b and x0 (NULL: x = 0) into the workspace, core(b, x) on the device, x back to x_out.
+template <class Core>
+static int solve_host_vectors(bemb200_matrix* m, const double* b, const double* x0, double* x_out, Core core) {
+    bemb200_ctx* ctx = m->ctx;
+    GmresWorkspace* ws = m->ws;
+    const size_t nb = m->n_rows * sizeof(cplx);
+    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
+    if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
+    else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
+    const int rc = core(ws->bin, ws->xout);
+    if (rc != BEMB200_OK) return rc;
+    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
+    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return BEMB200_OK;
+}
+
+extern "C" {
+
+int bemb200_gmres_device(const bemb200_matrix* cm, const double* b_dev, const double* x0_dev, uint32_t max_iterations,
+                         uint32_t restart, double tolerance, double* x_dev, bemb200_gmres_info* info) {
+    bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
+    int rc = check_solver_args(m, b_dev && x_dev && info, "gmres", restart);
+    if (rc != BEMB200_OK) return rc;
+    bemb200_ctx* ctx = m->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    rc = begin_call(m, restart);
+    if (rc != BEMB200_OK) return rc;
     const size_t nb = m->n_rows * sizeof(cplx);
     if (x0_dev) {
         if ((const void*)x0_dev != (const void*)x_dev)
@@ -1182,7 +1132,7 @@ int bemb200_gmres_device(const bemb200_matrix* cm, const double* b_dev, const do
     } else {
         BEMB_CUDA(ctx, cudaMemsetAsync(x_dev, 0, nb, ctx->stream));
     }
-    rc = gmres_core(m, (const cplx*)b_dev, (cplx*)x_dev, max_iterations, restart, tolerance, info);
+    rc = gmres_core(m, (const cplx*)b_dev, (cplx*)x_dev, max_iterations, restart, tolerance, info, LeftPrecond{});
     cudaStreamSynchronize(ctx->stream);
     return rc;
 }
@@ -1190,153 +1140,90 @@ int bemb200_gmres_device(const bemb200_matrix* cm, const double* b_dev, const do
 int bemb200_gmres(const bemb200_matrix* cm, const double* b, const double* x0, uint32_t max_iterations, uint32_t restart,
                   double tolerance, double* x_out, bemb200_gmres_info* info) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
-    bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "gmres needs a square operator");
-    if (restart == 0) return set_error(ctx, BEMB200_EINVAL, "restart must be >= 1");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = check_solver_args(m, b && x_out && info, "gmres", restart);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, restart);
+    std::lock_guard<std::mutex> lk(m->ctx->mu);
+    rc = begin_call(m, restart);
     if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
-    const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
-    rc = gmres_core(m, ws->bin, ws->xout, max_iterations, restart, tolerance, info);
-    if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    return solve_host_vectors(m, b, x0, x_out, [&](const cplx* bd, cplx* xd) {
+        return gmres_core(m, bd, xd, max_iterations, restart, tolerance, info, LeftPrecond{});
+    });
 }
 
 int bemb200_bicgstab(const bemb200_matrix* cm, const double* b, uint32_t max_iterations, double tolerance, double* x_out,
                      bemb200_gmres_info* info) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
-    bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "bicgstab needs a square operator");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = check_solver_args(m, b && x_out && info, "bicgstab", BICG_ROWS);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, 8);
+    std::lock_guard<std::mutex> lk(m->ctx->mu);
+    rc = begin_call(m, BICG_ROWS);
     if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
-    const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    rc = bicgstab_core(m, ws->bin, ws->xout, max_iterations, tolerance, info);
-    if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    return solve_host_vectors(m, b, nullptr, x_out, [&](const cplx* bd, cplx* xd) {
+        return bicgstab_core(m, bd, xd, max_iterations, tolerance, info);
+    });
 }
 
 int bemb200_cgs(const bemb200_matrix* cm, const double* b, uint32_t max_iterations, double tolerance, double* x_out,
                 bemb200_gmres_info* info) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
-    bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "cgs needs a square operator");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = check_solver_args(m, b && x_out && info, "cgs", BICG_ROWS);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, 8);
+    std::lock_guard<std::mutex> lk(m->ctx->mu);
+    rc = begin_call(m, BICG_ROWS);
     if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
-    const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    rc = cgs_core(m, ws->bin, ws->xout, max_iterations, tolerance, info);
-    if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    return solve_host_vectors(m, b, nullptr, x_out, [&](const cplx* bd, cplx* xd) {
+        return cgs_core(m, bd, xd, max_iterations, tolerance, info);
+    });
 }
 
 int bemb200_gmres_preconditioned(const bemb200_matrix* cm, const double* inv_diag, const double* b, const double* x0,
                                  uint32_t max_iterations, uint32_t restart, double tolerance, double* x_out,
                                  bemb200_gmres_info* info) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    int rc = check_solver_args(m, b && x_out && info, "gmres", restart);
+    if (rc != BEMB200_OK) return rc;
     bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "gmres needs a square operator");
-    if (restart == 0) return set_error(ctx, BEMB200_EINVAL, "restart must be >= 1");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    rc = begin_call(m, restart);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, restart);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
-    const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
-    const cplx* pinv = nullptr;
-    if (inv_diag) {
-        BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xin, inv_diag, nb, cudaMemcpyHostToDevice, ctx->stream));
-        pinv = ws->xin;
-    }
-    rc = gmres_core(m, ws->bin, ws->xout, max_iterations, restart, tolerance, info, true, pinv);
-    if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    return solve_host_vectors(m, b, x0, x_out, [&](const cplx* bd, cplx* xd) {
+        LeftPrecond P{true};  // inv_diag == NULL: IdentityPreconditioner
+        if (inv_diag) {
+            BEMB_CUDA(ctx, cudaMemcpyAsync(m->ws->xin, inv_diag, m->n_rows * sizeof(cplx), cudaMemcpyHostToDevice, ctx->stream));
+            P.pinv = m->ws->xin;
+        }
+        return gmres_core(m, bd, xd, max_iterations, restart, tolerance, info, P);
+    });
 }
 
 int bemb200_gmres_schwarz(const bemb200_matrix* cm, const bemb200_precond* precond, const double* b, const double* x0,
                           uint32_t max_iterations, uint32_t restart, double tolerance, double* x_out, bemb200_gmres_info* info) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !precond || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    int rc = check_solver_args(m, precond && b && x_out && info, "gmres", restart);
+    if (rc != BEMB200_OK) return rc;
     bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "gmres needs a square operator");
-    if (restart == 0) return set_error(ctx, BEMB200_EINVAL, "restart must be >= 1");
     if (precond->ctx != ctx || precond->n != m->n_rows || precond->r0 != m->r0 || precond->r1 != m->r1)
         return set_error(ctx, BEMB200_EINVAL, "preconditioner was built for another operator shape / context");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    rc = begin_call(m, restart);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, restart);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
-    const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
-    rc = gmres_core(m, ws->bin, ws->xout, max_iterations, restart, tolerance, info, true, nullptr, precond);
-    if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    return solve_host_vectors(m, b, x0, x_out, [&](const cplx* bd, cplx* xd) {
+        return gmres_core(m, bd, xd, max_iterations, restart, tolerance, info, LeftPrecond{true, nullptr, precond});
+    });
 }
 
 int bemb200_gmres_callback(const bemb200_matrix* cm, bemb200_precond_fn apply, void* user, const double* b, const double* x0,
                            uint32_t max_iterations, uint32_t restart, double tolerance, double* x_out, bemb200_gmres_info* info,
                            uint64_t* precond_calls) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
-    if (!m || !apply || !b || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    int rc = check_solver_args(m, apply && b && x_out && info, "gmres", restart);
+    if (rc != BEMB200_OK) return rc;
     bemb200_ctx* ctx = m->ctx;
-    if (m->n_rows != m->n_cols) return set_error(ctx, BEMB200_EINVAL, "gmres needs a square operator");
-    if (restart == 0) return set_error(ctx, BEMB200_EINVAL, "restart must be >= 1");
     if (ctx->nranks != 1 || m->r0 != 0 || m->r1 != m->n_rows)
         return set_error(ctx, BEMB200_EUNSUPPORTED, "bemb200_gmres_callback: a host preconditioner acts on whole vectors -- single-rank operators only");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    rc = begin_call(m, restart);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, restart);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
-    GmresWorkspace* ws = m->ws;
     const size_t nb = m->n_rows * sizeof(cplx);
     struct Pinned {  // the two host vectors of the round trip
         cplx* p = nullptr;
@@ -1351,18 +1238,12 @@ int bemb200_gmres_callback(const bemb200_matrix* cm, bemb200_precond_fn apply, v
     up.user = user;
     up.r_h = rbuf.p;
     up.z_h = zbuf.p;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
-    if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
-    rc = gmres_core(m, ws->bin, ws->xout, max_iterations, restart, tolerance, info, true, nullptr, nullptr, &up);
+    rc = solve_host_vectors(m, b, x0, x_out, [&](const cplx* bd, cplx* xd) {
+        return gmres_core(m, bd, xd, max_iterations, restart, tolerance, info, LeftPrecond{true, nullptr, nullptr, &up});
+    });
     if (precond_calls) *precond_calls = up.calls;
-    if (rc != BEMB200_OK) {
-        cudaStreamSynchronize(ctx->stream);  // nothing of this solve may still be reading the pinned vectors when they go
-        return rc;
-    }
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_out, ws->xout, nb, cudaMemcpyDeviceToHost, ctx->stream));
-    BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return BEMB200_OK;
+    if (rc != BEMB200_OK) cudaStreamSynchronize(ctx->stream);  // nothing of this solve may still be reading the pinned vectors when they go
+    return rc;
 }
 
 int bemb200_matrix_diagonal(const bemb200_matrix* cm, double* out) {
@@ -1395,12 +1276,8 @@ int bemb200_apply_device(const bemb200_matrix* cm, const double* x_dev, double* 
     if (!m || !x_dev || !y_dev) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
     bemb200_ctx* ctx = m->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = begin_call(m, 1);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, 1);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
     GmresWorkspace* ws = m->ws;
     if (ctx->nranks == 1) {
         // write straight into the caller's vector
@@ -1424,12 +1301,8 @@ int bemb200_apply(const bemb200_matrix* cm, const double* x, double* y) {
     if (!m || !x || !y) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
     bemb200_ctx* ctx = m->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = begin_call(m, 1);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, 1);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
     GmresWorkspace* ws = m->ws;
     BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xin, x, m->n_cols * sizeof(cplx), cudaMemcpyHostToDevice, ctx->stream));
     rc = matvec(m, ws->xin, ws->w, true);
@@ -1446,12 +1319,8 @@ int bemb200_apply_transpose(const bemb200_matrix* cm, const double* x, double* y
     bemb200_ctx* ctx = m->ctx;
     if (ctx->nranks > 1) return set_error(ctx, BEMB200_EUNSUPPORTED, "apply_transpose on a row-sharded matrix is not implemented");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = check_partition(m);
+    int rc = begin_call(m, 1);
     if (rc != BEMB200_OK) return rc;
-    rc = ensure_workspace(m, 1);
-    if (rc != BEMB200_OK) return rc;
-    reset_stats(m);
     GmresWorkspace* ws = m->ws;
     // y = A^T x : x has num_rows entries, y has num_cols entries
     BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xin, x, m->n_rows * sizeof(cplx), cudaMemcpyHostToDevice, ctx->stream));
