@@ -269,6 +269,12 @@ int bemb200_gmres_batched(const bemb200_matrix* m, const double* b_all, uint32_t
 int bemb200_gmres_batched_schwarz(const bemb200_matrix* m, const bemb200_precond* precond, const double* b_all, uint32_t nrhs,
                                   uint32_t max_iterations, uint32_t restart, double tolerance, double* x_all,
                                   bemb200_gmres_info* infos, double* block_matvec_ms, uint64_t* block_matvecs);
+/* bemb200_gmres_batched (precond == NULL) / bemb200_gmres_batched_schwarz with DEVICE vectors: b_dev and x_dev are nrhs
+ * vectors of num_rows complex128, each contiguous, in memory of the matrix's device (BEMB200_EINVAL otherwise).  Same
+ * limits and the same results; B is interleaved straight from b_dev and X written straight to x_dev. */
+int bemb200_gmres_batched_device(const bemb200_matrix* m, const bemb200_precond* precond, const double* b_dev, uint32_t nrhs,
+                                 uint32_t max_iterations, uint32_t restart, double tolerance, double* x_dev,
+                                 bemb200_gmres_info* infos, double* block_matvec_ms, uint64_t* block_matvecs);
 /* Y = A X for nrhs (<= 32) vectors at once with the tensor-core block kernel; kernel_ms (may be
  * NULL) receives the device time of one block matvec.  Row-sharded operators: collective, every rank multiplies its row
  * block and receives the whole Y.  (bemb200_gmres_batched: up to 196 608 unknowns, also row-sharded.) */
@@ -297,6 +303,28 @@ int bemb200_scattered_field(const bemb200_staged_mesh* sm, const bemb200_physics
  * (the reference indexes it by boundary-element enumeration, identical for sequential dof maps). */
 int bemb200_compute_rcs(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t n_dirs, const double* dirs,
                         const double* surface_pressure, double* rcs_out);
+/* ---- several right-hand sides / solutions of one mesh (plane waves from many directions, point sources) ----------------
+ * Block layout: nrhs (or nsol) vectors of num_dofs complex128, each contiguous, in DOF order (that of bemb200_gmres_batched).
+ * Device arrays belong to the staged mesh's device (BEMB200_EINVAL otherwise).  Row s of every result has the bits of the
+ * single-vector call on vector s. */
+/* nrhs (1..4096) calls of bemb200_incident_rhs: right-hand side s sums the sources [src_ptr[s], src_ptr[s+1]) (src_ptr[0] = 0,
+ * non-decreasing, src_ptr[nrhs] <= 65536 sources in all; kinds / vecs / amps as there).  system != NULL (a matrix of the staged
+ * mesh's device) adds TbemSystem.rhs -- b = TbemSystem.rhs + incident, the b of bemb200_sweep_next; on a row-sharded operator
+ * the rhs is gathered as bemb200_rhs_download_full gathers it, so the call is collective.  Result [nrhs * num_dofs] to b_host
+ * and/or b_dev (either may be NULL). */
+int bemb200_incident_rhs_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re, double beta_im,
+                               uint32_t nrhs, const uint32_t* src_ptr, const int32_t* kinds, const double* vecs, const double* amps,
+                               const bemb200_matrix* system, double* b_host, double* b_dev);
+/* bemb200_compute_rcs for nsol (1..4096) surface solutions at once (on_device = 0: host array, 1: device array);
+ * rcs_out [nsol * n_dirs] (host), solution-major. */
+int bemb200_compute_rcs_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                              const double* surface_pressure, int on_device, uint32_t n_dirs, const double* dirs,
+                              double* rcs_out);
+/* bemb200_scattered_field for nsol (1..4096) surface solutions at once (surface_velocity may be NULL; on_device as above);
+ * out [nsol * n_eval] complex128 (host), solution-major. */
+int bemb200_scattered_field_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                                  const double* surface_pressure, const double* surface_velocity, int on_device,
+                                  uint64_t n_eval, const double* eval_pts, double* out);
 
 /* ---- room-acoustics dense path (SURVEY 8f rank 3): math-bem/src/room_acoustics/solver.rs -------
  * Point collocation on a RoomMesh (math-xem-common/src/types.rs:185-192): nodes [n_nodes*3],
@@ -353,6 +381,19 @@ int bemb200_sweep_submit(bemb200_sweep* sw, const bemb200_physics* phys, double 
                          uint32_t max_iterations, uint32_t restart, double tolerance);
 /* x_out: num_dofs complex128 (host); stats and rhs_out (the b that was solved) may be NULL */
 int bemb200_sweep_next(bemb200_sweep* sw, double* x_out, bemb200_gmres_info* info, bemb200_assembly_stats* stats, double* rhs_out);
+/* Queue a frequency with nrhs (1..32) incident right-hand sides (sources as bemb200_incident_rhs_batch).  The incident block
+ * is built on the device right after the frequency's assembly; b = TbemSystem.rhs + incident is formed on the device.
+ * nrhs = 1 solves as bemb200_sweep_submit with rhs_extra = that incident vector (same bits); nrhs > 1 with the batched solver
+ * (bemb200_gmres_batched / _schwarz; overlapping subdomains fail in next_batch with BEMB200_EUNSUPPORTED and the frequency is
+ * consumed).  bemb200_sweep_next on a frequency with nrhs > 1 returns BEMB200_EINVAL and leaves it queued. */
+int bemb200_sweep_submit_incident(bemb200_sweep* sw, const bemb200_physics* phys, double beta_re, double beta_im, uint32_t nrhs,
+                                  const uint32_t* src_ptr, const int32_t* kinds, const double* vecs, const double* amps,
+                                  uint32_t max_iterations, uint32_t restart, double tolerance);
+/* Solve the oldest queued frequency, whichever call submitted it: x_out [capacity * num_dofs] complex128 and infos[capacity]
+ * (host) receive its *nrhs_out (1 for bemb200_sweep_submit) solutions.  A frequency of more than `capacity` right-hand sides
+ * returns BEMB200_EINVAL and stays queued.  stats may be NULL. */
+int bemb200_sweep_next_batch(bemb200_sweep* sw, uint32_t capacity, double* x_out, bemb200_gmres_info* infos, uint32_t* nrhs_out,
+                             bemb200_assembly_stats* stats);
 uint64_t bemb200_sweep_boosts(const bemb200_sweep* sw);
 /* Solve every frequency returned from now on with gmres_preconditioned (gmres.rs:282) and the block-Jacobi / additive Schwarz
  * preconditioner of bemb200_schwarz_create, rebuilt from each frequency's matrix (arguments as there; num_subdomains = 0

@@ -111,11 +111,17 @@ SYMBOLS = {
                                         C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "bemb200_gmres_batched_schwarz": (C.c_int, [_VP, _VP, _VP, C.c_uint32, C.c_uint32, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo),
                                                 C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
+    "bemb200_gmres_batched_device": (C.c_int, [_VP, _VP, _VP, C.c_uint32, C.c_uint32, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo),
+                                               C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "bemb200_apply_block": (C.c_int, [_VP, _VP, C.c_uint32, _VP, C.POINTER(C.c_double)]),
     "bemb200_solver_stats": (C.c_int, [_VP, C.POINTER(C.c_uint64), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "bemb200_incident_rhs": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_double, C.c_double, C.c_uint32, _VP, _VP, _VP, _VP, _VP]),
     "bemb200_scattered_field": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint64, _VP, _VP, _VP, _VP]),
     "bemb200_compute_rcs": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, _VP]),
+    "bemb200_incident_rhs_batch": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_double, C.c_double, C.c_uint32, _VP, _VP, _VP, _VP, _VP, _VP,
+                                             _VP]),
+    "bemb200_compute_rcs_batch": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, C.c_int, C.c_uint32, _VP, _VP]),
+    "bemb200_scattered_field_batch": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, C.c_int, C.c_uint64, _VP, _VP]),
     "bemb200_bicgstab": (C.c_int, [_VP, _VP, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo)]),
     "bemb200_cgs": (C.c_int, [_VP, _VP, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo)]),
     "bemb200_lu_solve": (C.c_int, [_VP, _VP, _VP, C.c_int, C.POINTER(C.c_double)]),
@@ -134,6 +140,9 @@ SYMBOLS = {
     "bemb200_sweep_num_dofs": (C.c_uint64, [_VP]),
     "bemb200_sweep_submit": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_double, C.c_double, _VP, C.c_uint32, C.c_uint32, C.c_double]),
     "bemb200_sweep_next": (C.c_int, [_VP, _VP, C.POINTER(CGmresInfo), C.POINTER(CAssemblyStats), _VP]),
+    "bemb200_sweep_submit_incident": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_double, C.c_double, C.c_uint32, _VP, _VP, _VP, _VP,
+                                                C.c_uint32, C.c_uint32, C.c_double]),
+    "bemb200_sweep_next_batch": (C.c_int, [_VP, C.c_uint32, _VP, C.POINTER(CGmresInfo), C.POINTER(C.c_uint32), C.POINTER(CAssemblyStats)]),
     "bemb200_sweep_boosts": (C.c_uint64, [_VP]),
     "bemb200_sweep_set_block_jacobi": (C.c_int, [_VP, C.c_uint32, _VP, _VP]),
     "bemb200_sweep_destroy": (None, [_VP]),

@@ -495,6 +495,143 @@ def incident_rhs_device(staged: StagedMesh, physics: PhysicsParams, beta: comple
     return out
 
 
+def source_groups(incidents, max_groups: int = 4096) -> tuple:
+    """``(src_ptr, kinds, vecs, amps)`` of a sequence of IncidentField objects, one group per field: its plane waves, then its
+    point sources (the source order of ``incident_rhs_device``).  Raises ValueError for anything else."""
+    if isinstance(incidents, (str, bytes)) or not hasattr(incidents, "__len__") or len(incidents) == 0:
+        raise ValueError("incidents must be a non-empty sequence of IncidentField objects")
+    src_ptr, kinds, vecs, amps = [0], [], [], []
+    for f in incidents:
+        if not (hasattr(f, "plane_waves") and hasattr(f, "point_sources")):
+            raise ValueError(f"incidents must hold IncidentField objects, got {type(f).__name__}")
+        for kind, group in ((0, f.plane_waves), (1, f.point_sources)):
+            for v, a in group:
+                v = np.asarray(v, dtype=np.float64)
+                if v.shape != (3,):
+                    raise ValueError("a source direction / position must have 3 components")
+                kinds.append(kind); vecs.append(v); amps.append(complex(a))
+        src_ptr.append(len(kinds))
+    return check_source_groups(np.asarray(src_ptr, dtype=np.uint32), np.asarray(kinds, dtype=np.int32),
+                               np.asarray(vecs, dtype=np.float64).reshape(-1, 3), np.asarray(amps, dtype=np.complex128),
+                               max_groups)
+
+
+def check_source_groups(src_ptr, kinds, vecs, amps, max_groups: int = 4096) -> tuple:
+    """Validate the source groups of ``bemb200_incident_rhs_batch`` / ``bemb200_sweep_submit_incident`` before they reach the
+    library: src_ptr[0] = 0, non-decreasing, at most ``max_groups`` groups and 65536 sources, kinds 0 / 1, vecs (ns, 3),
+    amps (ns,).  Returns the contiguous arrays."""
+    src_ptr = np.ascontiguousarray(src_ptr)
+    if src_ptr.ndim != 1 or src_ptr.size < 2 or not np.issubdtype(src_ptr.dtype, np.integer):
+        raise ValueError("src_ptr must be a 1-D integer array of nrhs + 1 entries")
+    nrhs = src_ptr.size - 1
+    if nrhs > max_groups:
+        raise ValueError(f"at most {max_groups} right-hand sides per call")
+    if src_ptr[0] != 0 or np.any(np.diff(src_ptr.astype(np.int64)) < 0):
+        raise ValueError("src_ptr must start at 0 and be non-decreasing")
+    ns = int(src_ptr[-1])
+    if ns > 65536:
+        raise ValueError("at most 65536 sources in all")
+    kinds = np.ascontiguousarray(kinds, dtype=np.int32)
+    vecs = np.ascontiguousarray(vecs, dtype=np.float64)
+    amps = np.ascontiguousarray(amps, dtype=np.complex128)
+    if kinds.shape != (ns,) or vecs.shape != (ns, 3) or amps.shape != (ns,):
+        raise ValueError("kinds / vecs / amps must have src_ptr[-1] entries (vecs: 3 per source)")
+    if np.any((kinds != 0) & (kinds != 1)):
+        raise ValueError("source kind must be 0 (plane wave) or 1 (point source)")
+    if ns == 0:  # the library takes no NULL arrays: one unused entry each
+        kinds, vecs, amps = np.zeros(1, np.int32), np.zeros((1, 3)), np.zeros(1, np.complex128)
+    return np.ascontiguousarray(src_ptr, dtype=np.uint32), kinds, vecs, amps
+
+
+def _device_ptr(p, what: str) -> int:
+    if isinstance(p, (bool, np.bool_)) or not isinstance(p, (int, np.integer)) or int(p) <= 0:
+        raise ValueError(f"{what} must be a device pointer (a positive int)")
+    return int(p)
+
+
+def incident_rhs_batch(staged: StagedMesh, physics: PhysicsParams, beta: complex, incidents, system: Optional[TbemSystem] = None,
+                       b_dev: int = 0, fetch: bool = True) -> Optional[np.ndarray]:
+    """``incident_rhs_device`` for every IncidentField of ``incidents`` in one launch: row s of the (nrhs, n) result (DOF order)
+    has the bits of ``incident_rhs_device(staged, physics, beta, incidents[s])``.  ``system``: add TbemSystem.rhs (b = rhs +
+    incident, as the sweep forms it).  ``b_dev``: device pointer receiving the block; ``fetch=False`` returns None."""
+    src_ptr, kinds, vecs, amps = source_groups(incidents)
+    nrhs = src_ptr.size - 1
+    if b_dev:
+        b_dev = _device_ptr(b_dev, "b_dev")
+    if not fetch and not b_dev:
+        raise ValueError("fetch=False needs b_dev")
+    if system is not None and not isinstance(system, TbemSystem):
+        raise ValueError("system must be a TbemSystem")
+    out = np.empty((nrhs, staged.num_dofs), dtype=np.complex128) if fetch else None
+    ph = _cphys(physics)
+    beta = complex(beta)
+    _capi.check(_capi.lib().bemb200_incident_rhs_batch(staged._h, C.byref(ph), beta.real, beta.imag, nrhs, _capi.ptr(src_ptr),
+                                                       _capi.ptr(kinds), _capi.ptr(vecs), _capi.ptr(amps),
+                                                       system.matrix._h if system is not None else None,
+                                                       _capi.ptr(out) if fetch else None, C.c_void_p(b_dev or None)), staged.ctx._h)
+    return out
+
+
+def _solutions_arg(values, staged: StagedMesh, nsol: Optional[int], what: str, allow_none: bool = False):
+    """(pointer, on_device, nsol, keep-alive) of surface values given as an (nsol, n) host array (entry j of a row belongs to
+    the j-th non-evaluation element, re-addressed to DOF order) or a device pointer to nsol DOF-ordered vectors."""
+    if values is None:
+        if allow_none:
+            return None, nsol, None
+        raise ValueError(f"{what} is required")
+    if isinstance(values, (int, np.integer)) and not isinstance(values, (bool, np.bool_)):
+        if nsol is None or not 1 <= int(nsol) <= 4096:
+            raise ValueError(f"{what} as a device pointer needs nsol in 1..4096")
+        return C.c_void_p(_device_ptr(values, what)), int(nsol), True
+    a = np.ascontiguousarray(values, dtype=np.complex128)
+    if a.ndim != 2 or a.shape[1] != staged.num_dofs or not 1 <= a.shape[0] <= 4096:
+        raise ValueError(f"{what} must be an (nsol, num_dofs) array with 1 <= nsol <= 4096, got shape {a.shape}")
+    if nsol is not None and int(nsol) != a.shape[0]:
+        raise ValueError(f"nsol = {nsol} does not match {what} with {a.shape[0]} rows")
+    if staged.enum_to_dof is not None:
+        b = np.empty_like(a)
+        b[:, staged.enum_to_dof] = a
+        a = b
+    return a, a.shape[0], False
+
+
+def compute_rcs_batch(surface_pressure, staged: StagedMesh, directions, physics: PhysicsParams, nsol: Optional[int] = None) -> np.ndarray:
+    """``compute_rcs`` of nsol solutions over the (M, 3) ``directions`` in one launch -> (nsol, M); row s has the bits of
+    ``compute_rcs(surface_pressure[s], ...)``.  ``surface_pressure``: (nsol, n) host array in the order ``compute_rcs`` takes,
+    or a device pointer (int) to nsol DOF-ordered vectors, as ``gmres_batched_device`` leaves them, with ``nsol``."""
+    ps, nsol, on_dev = _solutions_arg(surface_pressure, staged, nsol, "surface_pressure")
+    d = np.ascontiguousarray(directions, dtype=np.float64)
+    if d.ndim != 2 or d.shape[1] != 3:
+        raise ValueError("directions must be an (M, 3) array")
+    out = np.empty((nsol, d.shape[0]), dtype=np.float64)
+    ph = _cphys(physics)
+    _capi.check(_capi.lib().bemb200_compute_rcs_batch(staged._h, C.byref(ph), nsol, ps if on_dev else _capi.ptr(ps), 1 if on_dev else 0,
+                                                      d.shape[0], _capi.ptr(d), _capi.ptr(out)), staged.ctx._h)
+    return out
+
+
+def compute_scattered_field_batch(eval_points, staged: StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                                  nsol: Optional[int] = None) -> np.ndarray:
+    """``compute_scattered_field`` of nsol solutions at the (M, 3) ``eval_points`` in one launch -> (nsol, M) complex; row s has
+    the bits of ``compute_scattered_field(eval_points, staged, surface_pressure[s], surface_velocity[s], physics)``.  Surface
+    values: (nsol, n) host arrays as ``compute_scattered_field`` takes them, or device pointers (ints, DOF order) with ``nsol``;
+    ``surface_velocity`` may be None, and is given the same way as ``surface_pressure``."""
+    ps, nsol, on_dev = _solutions_arg(surface_pressure, staged, nsol, "surface_pressure")
+    vs, _, v_dev = _solutions_arg(surface_velocity, staged, nsol, "surface_velocity", allow_none=True)
+    if vs is not None and v_dev != on_dev:
+        raise ValueError("surface_pressure and surface_velocity must both be host arrays or both device pointers")
+    pts = np.ascontiguousarray(eval_points, dtype=np.float64)
+    if pts.ndim != 2 or pts.shape[1] != 3:
+        raise ValueError("eval_points must be an (M, 3) array")
+    out = np.empty((nsol, pts.shape[0]), dtype=np.complex128)
+    ph = _cphys(physics)
+    vptr = None if vs is None else (vs if on_dev else _capi.ptr(vs))
+    _capi.check(_capi.lib().bemb200_scattered_field_batch(staged._h, C.byref(ph), nsol, ps if on_dev else _capi.ptr(ps), vptr,
+                                                          1 if on_dev else 0, pts.shape[0], _capi.ptr(pts), _capi.ptr(out)),
+                staged.ctx._h)
+    return out
+
+
 def compute_scattered_field(eval_points: np.ndarray, staged: StagedMesh, surface_pressure: np.ndarray,
                             surface_velocity: Optional[np.ndarray], physics: PhysicsParams) -> np.ndarray:
     """postprocess/pressure.rs:81-137 on the device.  Surface values as the reference takes them: entry j belongs to the j-th
@@ -936,6 +1073,28 @@ def gmres_batched(operator: DenseOperator, b_all: np.ndarray, config: GmresConfi
                                                               config.restart, config.tolerance, _capi.ptr(x_all), infos, C.byref(ms),
                                                               C.byref(cnt)), operator.matrix.ctx._h)
     sols = [GmresSolution(x=x_all[i], iterations=int(infos[i].iterations), restarts=int(infos[i].restarts),
+                          residual=float(infos[i].residual), converged=bool(infos[i].converged)) for i in range(nrhs)]
+    return sols, dict(block_matvec_ms=float(ms.value), block_matvecs=int(cnt.value))
+
+
+def gmres_batched_device(operator: DenseOperator, b_dev: int, nrhs: int, config: GmresConfig, x_dev: int,
+                         precond: "Optional[AdditiveSchwarzPreconditioner]" = None):
+    """``gmres_batched`` on DEVICE vectors: ``b_dev`` / ``x_dev`` point to nrhs (1..32) vectors of num_rows complex128, each
+    contiguous, on the operator's device.  Same solutions and infos as ``gmres_batched`` on the same B; returns
+    (list of GmresSolution with x=None, stats dict)."""
+    b_dev, x_dev = _device_ptr(b_dev, "b_dev"), _device_ptr(x_dev, "x_dev")
+    if isinstance(nrhs, (bool, np.bool_)) or not isinstance(nrhs, (int, np.integer)) or not 1 <= int(nrhs) <= 32:
+        raise ValueError("nrhs must be an int in 1..32")
+    if precond is not None and not isinstance(precond, AdditiveSchwarzPreconditioner):
+        raise ValueError("precond must be a block-Jacobi AdditiveSchwarzPreconditioner or None")
+    nrhs = int(nrhs)
+    infos = (_capi.CGmresInfo * nrhs)()
+    ms, cnt = C.c_double(), C.c_uint64()
+    _capi.check(_capi.lib().bemb200_gmres_batched_device(operator.matrix._h, precond._h if precond is not None else None,
+                                                         C.c_void_p(b_dev), nrhs, config.max_iterations, config.restart,
+                                                         config.tolerance, C.c_void_p(x_dev), infos, C.byref(ms), C.byref(cnt)),
+                operator.matrix.ctx._h)
+    sols = [GmresSolution(x=None, iterations=int(infos[i].iterations), restarts=int(infos[i].restarts),
                           residual=float(infos[i].residual), converged=bool(infos[i].converged)) for i in range(nrhs)]
     return sols, dict(block_matvec_ms=float(ms.value), block_matvecs=int(cnt.value))
 

@@ -115,6 +115,17 @@ int set_error(bemb200_ctx* ctx, int code, const std::string& msg);
 int cuda_fail(bemb200_ctx* ctx, cudaError_t e, const char* what);
 void free_workspace(bemb200_matrix* m);
 void free_peer_exchange(bemb200_ctx* ctx, bool collective);
+// true when p is device (or managed) memory of `device` (postprocess.cu)
+bool device_ptr_on(int device, const void* p);
+// out[s n + i] = sys[i] + inc[s n + i] for s < nrhs (out may be inc) on stream s (postprocess.cu)
+cudaError_t launch_add_system_rhs(const cplx* sys, const cplx* inc, uint64_t n, uint32_t nrhs, cplx* out, cudaStream_t s);
+// TbemSystem.rhs of every row (local slices all-gathered; collective on a row-sharded operator) to `out`, a host
+// (cudaMemcpyDeviceToHost) or device (cudaMemcpyDeviceToDevice) vector of num_rows complex128 (gmres.cu)
+int rhs_full(bemb200_matrix* m, double* out, cudaMemcpyKind kind);
+// bemb200_gmres (pc == NULL) / bemb200_gmres_schwarz with b already on the device: the same operations, only the copy of b
+// into the workspace is device to device (gmres.cu)
+int gmres_solve_device_b(bemb200_matrix* m, const bemb200_precond* pc, const double* b_dev, uint32_t max_iterations, uint32_t restart,
+                         double tolerance, double* x_out, bemb200_gmres_info* info);
 }  // namespace bemb
 
 #define BEMB_CUDA(ctx, call)                                          \

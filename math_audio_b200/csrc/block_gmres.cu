@@ -55,12 +55,16 @@ struct DevBuf {
 
 // `sp` != NULL: nrhs independent gmres_preconditioned() solves (gmres.rs:282-585) with the block-Jacobi preconditioner: M^-1 acts on
 // the rank's slab of the block product before the exchange, residuals are M^-1 (B - A X), norms relative to ||M^-1 b||.
+// `device_io`: b_all / x_all are device arrays of the matrix's device; B is interleaved straight from b_all and X
+// de-interleaved straight into x_all (no staging copy, no host round trip).
 static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* sp, const double* b_all, uint32_t nrhs,
                               uint32_t max_iterations, uint32_t restart, double tolerance, double* x_all, bemb200_gmres_info* infos,
-                              double* block_matvec_ms, uint64_t* block_matvecs) {
+                              double* block_matvec_ms, uint64_t* block_matvecs, bool device_io = false) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
     if (!m || !b_all || !x_all || !infos) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
     bemb200_ctx* ctx = m->ctx;
+    if (device_io && (!device_ptr_on(ctx->device, b_all) || !device_ptr_on(ctx->device, x_all)))
+        return set_error(ctx, BEMB200_EINVAL, "b_dev / x_dev are not device memory of the matrix's device");
     if (sp && (sp->ctx != ctx || sp->n != m->n_rows || sp->r0 != m->r0 || sp->r1 != m->r1))
         return set_error(ctx, BEMB200_EINVAL, "preconditioner was built for another operator shape / context");
     if (sp && !sp->disjoint)
@@ -96,7 +100,7 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
     BEMB_CUDA(ctx, buf.alloc(&Bblk, npad * S));
     BEMB_CUDA(ctx, buf.alloc(&Rblk, npad * S));
     BEMB_CUDA(ctx, buf.alloc(&Xsol, npad * S));
-    BEMB_CUDA(ctx, buf.alloc(&stage, (size_t)nrhs * n));
+    BEMB_CUDA(ctx, buf.alloc(&stage, device_io ? 0 : (size_t)nrhs * n));
     cplx* Pslab = nullptr;  // this rank's slab of a block before M^-1
     if (sp) BEMB_CUDA(ctx, buf.alloc(&Pslab, (nloc ? nloc : 1) * (size_t)S));
     BEMB_CUDA(ctx, buf.alloc(&hcol_d, (size_t)S * hstride));
@@ -119,8 +123,12 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
     BEMB_CUDA(ctx, cudaMemsetAsync(Xblk, 0, npad * S * sizeof(cplx), s));
     BEMB_CUDA(ctx, cudaMemsetAsync(Yblk, 0, npad * S * sizeof(cplx), s));
     BEMB_CUDA(ctx, cudaMemsetAsync(Xsol, 0, npad * S * sizeof(cplx), s));
-    BEMB_CUDA(ctx, cudaMemcpyAsync(stage, b_all, (size_t)nrhs * n * sizeof(cplx), cudaMemcpyHostToDevice, s));
-    BEMB_CUDA(ctx, launch_interleave(stage, Bblk, n, (int)nrhs, S, 1, s));
+    if (device_io) {
+        BEMB_CUDA(ctx, launch_interleave((const cplx*)b_all, Bblk, n, (int)nrhs, S, 1, s));
+    } else {
+        BEMB_CUDA(ctx, cudaMemcpyAsync(stage, b_all, (size_t)nrhs * n * sizeof(cplx), cudaMemcpyHostToDevice, s));
+        BEMB_CUDA(ctx, launch_interleave(stage, Bblk, n, (int)nrhs, S, 1, s));
+    }
 
     bool precond_in_matvec = false;  // on inside the Arnoldi loop; the residual products need the bare A X
     // Z (npad x S) = M^-1 R for a whole block: every rank solves on its slab, the slabs are gathered
@@ -294,8 +302,12 @@ static int gmres_batched_impl(const bemb200_matrix* cm, const bemb200_precond* s
                 R[q].done = true;
             }
     }
-    BEMB_CUDA(ctx, launch_interleave(Xsol, stage, n, (int)nrhs, S, 0, s));
-    BEMB_CUDA(ctx, cudaMemcpyAsync(x_all, stage, (size_t)nrhs * n * sizeof(cplx), cudaMemcpyDeviceToHost, s));
+    if (device_io) {
+        BEMB_CUDA(ctx, launch_interleave(Xsol, (cplx*)x_all, n, (int)nrhs, S, 0, s));
+    } else {
+        BEMB_CUDA(ctx, launch_interleave(Xsol, stage, n, (int)nrhs, S, 0, s));
+        BEMB_CUDA(ctx, cudaMemcpyAsync(x_all, stage, (size_t)nrhs * n * sizeof(cplx), cudaMemcpyDeviceToHost, s));
+    }
     BEMB_CUDA(ctx, cudaStreamSynchronize(s));
     for (uint32_t q = 0; q < nrhs; ++q) infos[q] = R[q].info;
     if (block_matvec_ms) *block_matvec_ms = mv_ms;
@@ -314,6 +326,13 @@ extern "C" int bemb200_gmres_batched_schwarz(const bemb200_matrix* cm, const bem
                                              bemb200_gmres_info* infos, double* block_matvec_ms, uint64_t* block_matvecs) {
     if (!precond) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
     return gmres_batched_impl(cm, precond, b_all, nrhs, max_iterations, restart, tolerance, x_all, infos, block_matvec_ms, block_matvecs);
+}
+
+extern "C" int bemb200_gmres_batched_device(const bemb200_matrix* cm, const bemb200_precond* precond, const double* b_dev, uint32_t nrhs,
+                                            uint32_t max_iterations, uint32_t restart, double tolerance, double* x_dev,
+                                            bemb200_gmres_info* infos, double* block_matvec_ms, uint64_t* block_matvecs) {
+    return gmres_batched_impl(cm, precond, b_dev, nrhs, max_iterations, restart, tolerance, x_dev, infos, block_matvec_ms, block_matvecs,
+                              true);
 }
 
 // Y = A X for a block of nrhs right-hand sides (each contiguous on the host): the tensor-core

@@ -1099,12 +1099,14 @@ static int begin_call(bemb200_matrix* m, uint32_t restart) {
 }
 
 // A solve on host vectors: b and x0 (NULL: x = 0) into the workspace, core(b, x) on the device, x back to x_out.
+// `b_kind` = cudaMemcpyDeviceToDevice: b is a device vector (the sweep's right-hand sides formed on the device).
 template <class Core>
-static int solve_host_vectors(bemb200_matrix* m, const double* b, const double* x0, double* x_out, Core core) {
+static int solve_host_vectors(bemb200_matrix* m, const double* b, const double* x0, double* x_out, Core core,
+                              cudaMemcpyKind b_kind = cudaMemcpyHostToDevice) {
     bemb200_ctx* ctx = m->ctx;
     GmresWorkspace* ws = m->ws;
     const size_t nb = m->n_rows * sizeof(cplx);
-    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, cudaMemcpyHostToDevice, ctx->stream));
+    BEMB_CUDA(ctx, cudaMemcpyAsync(ws->bin, b, nb, b_kind, ctx->stream));
     if (x0) BEMB_CUDA(ctx, cudaMemcpyAsync(ws->xout, x0, nb, cudaMemcpyHostToDevice, ctx->stream));
     else BEMB_CUDA(ctx, cudaMemsetAsync(ws->xout, 0, nb, ctx->stream));
     const int rc = core(ws->bin, ws->xout);
@@ -1372,6 +1374,12 @@ int bemb200_row_sum_correction(bemb200_matrix* m, double* avg) {
 int bemb200_rhs_download_full(const bemb200_matrix* cm, double* out) {
     bemb200_matrix* m = const_cast<bemb200_matrix*>(cm);
     if (!m || !out) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    return rhs_full(m, out, cudaMemcpyDeviceToHost);
+}
+
+}  // extern "C"
+
+int bemb::rhs_full(bemb200_matrix* m, double* out, cudaMemcpyKind kind) {
     bemb200_ctx* ctx = m->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -1384,10 +1392,30 @@ int bemb200_rhs_download_full(const bemb200_matrix* cm, double* out) {
     BEMB_CUDA(ctx, cudaMemcpyAsync(loc, m->rhs, (m->r1 - m->r0) * sizeof(cplx), cudaMemcpyDeviceToDevice, ctx->stream));
     rc = nccl_allgather_bytes(ctx, loc, ws->r, ws->chunk * sizeof(cplx));
     if (rc != BEMB200_OK) return rc;
-    BEMB_CUDA(ctx, cudaMemcpyAsync(out, ws->r, m->n_rows * sizeof(cplx), cudaMemcpyDeviceToHost, ctx->stream));
+    BEMB_CUDA(ctx, cudaMemcpyAsync(out, ws->r, m->n_rows * sizeof(cplx), kind, ctx->stream));
     BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return BEMB200_OK;
 }
+
+int bemb::gmres_solve_device_b(bemb200_matrix* m, const bemb200_precond* pc, const double* b_dev, uint32_t max_iterations,
+                               uint32_t restart, double tolerance, double* x_out, bemb200_gmres_info* info) {
+    int rc = check_solver_args(m, b_dev && x_out && info, "gmres", restart);
+    if (rc != BEMB200_OK) return rc;
+    bemb200_ctx* ctx = m->ctx;
+    if (pc && (pc->ctx != ctx || pc->n != m->n_rows || pc->r0 != m->r0 || pc->r1 != m->r1))
+        return set_error(ctx, BEMB200_EINVAL, "preconditioner was built for another operator shape / context");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    rc = begin_call(m, restart);
+    if (rc != BEMB200_OK) return rc;
+    return solve_host_vectors(
+        m, b_dev, nullptr, x_out,
+        [&](const cplx* bd, cplx* xd) {
+            return gmres_core(m, bd, xd, max_iterations, restart, tolerance, info, pc ? LeftPrecond{true, nullptr, pc} : LeftPrecond{});
+        },
+        cudaMemcpyDeviceToDevice);
+}
+
+extern "C" {
 
 int bemb200_solver_stats(const bemb200_matrix* m, uint64_t* kernel_launches, double* matvec_ms, uint64_t* matvecs) {
     if (!m) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");

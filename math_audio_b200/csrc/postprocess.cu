@@ -3,6 +3,12 @@
 //   scattered_field_kernel   compute_scattered_field                 math-bem/src/core/postprocess/pressure.rs:81-259
 //   rcs_kernel               compute_rcs                             math-bem/src/core/postprocess/pressure.rs:438-478
 // All work on the staged (DOF-ordered) mesh so that a frequency sweep never leaves the device.
+//
+// The *_batch kernels serve several right-hand sides / solutions of one mesh (plane waves from many directions, DESIGN.md
+// section 4.7).  What depends only on the geometry -- sincos(-k c.d) and n.d of the RCS, the 7-point Green's function of the
+// field -- is evaluated once and applied to every solution of a chunk.  Per solution they repeat the single kernels'
+// expressions, thread-to-element mapping and reduction order, so row s of a batch has the bits of the single call on
+// solution s (this unit is compiled with -fmad=false: no contraction can differ between the two).
 #include <vector>
 
 #include "api_internal.h"
@@ -149,7 +155,182 @@ rcs_kernel(const double* __restrict__ src, const double* __restrict__ area, uint
     }
 }
 
+// Column s of a batch: incident_rhs_kernel over the sources [grp[s], grp[s+1]) (same per-entry arithmetic and source order);
+// `sys` != NULL (TbemSystem.rhs, all rows) adds it as one IEEE add, sys + incident, the b of bemb200_sweep_next.
+__global__ void incident_rhs_batch_kernel(const double* __restrict__ src, uint32_t n, const Source* __restrict__ sources,
+                                          const uint32_t* __restrict__ grp, double k, double gamma, double tau, cplx beta,
+                                          const cplx* __restrict__ sys, cplx* __restrict__ rhs) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t s0 = grp[blockIdx.y], s1 = grp[blockIdx.y + 1];
+    const double* p = src + 8ull * i;
+    const double* nr = p + 3;
+    cplx pinc = C(0, 0), dpdn = C(0, 0);
+    for (uint32_t s = s0; s < s1; ++s) {
+        const Source sc = sources[s];
+        if (sc.kind == 0) {
+            const double kdotx = k * (sc.v[0] * p[0] + sc.v[1] * p[1] + sc.v[2] * p[2]);
+            const double kdotn = k * (sc.v[0] * nr[0] + sc.v[1] * nr[1] + sc.v[2] * nr[2]);
+            double sn, cs;
+            sincos(kdotx, &sn, &cs);
+            const cplx pw = sc.amp * C(cs, sn);
+            pinc += pw;
+            dpdn += C(0.0, kdotn) * pw;
+        } else {
+            const double dx = p[0] - sc.v[0], dy = p[1] - sc.v[1], dz = p[2] - sc.v[2];
+            const double r = sqrt(dx * dx + dy * dy + dz * dz);
+            if (r > 1e-10) {
+                double sn, cs;
+                sincos(k * r, &sn, &cs);
+                const cplx g = C(cs, sn) / (4.0 * PI * r);
+                pinc += sc.amp * g;
+                const cplx dgdr = (C(0.0, k) - C(1.0 / r, 0.0)) * g;
+                const double drdn = (dx * nr[0] + dy * nr[1] + dz * nr[2]) / r;
+                dpdn += sc.amp * dgdr * drdn;
+            }
+        }
+    }
+    const cplx v = -(pinc * gamma + beta * C(tau, 0.0) * dpdn);
+    rhs[(uint64_t)blockIdx.y * n + i] = sys ? sys[i] + v : v;
+}
+
+constexpr int SOL_CHUNK = 8;  // solutions per block of the batch kernels (grid dimension y runs over chunks)
+
+// Warp shuffle + 8-warp sum of every solution of the chunk, in the order of the single kernels; thread c < cnt returns
+// the block total of solution c (other threads: undefined).
+__device__ __forceinline__ cplx block_sum_chunk(cplx (&acc)[SOL_CHUNK], int cnt) {
+    __shared__ double red[2][SOL_CHUNK][8];
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) {
+#pragma unroll
+        for (int m = 16; m >= 1; m >>= 1) {
+            acc[c].re += __shfl_xor_sync(0xffffffffu, acc[c].re, m);
+            acc[c].im += __shfl_xor_sync(0xffffffffu, acc[c].im, m);
+        }
+        if ((threadIdx.x & 31) == 0) { red[0][c][threadIdx.x >> 5] = acc[c].re; red[1][c][threadIdx.x >> 5] = acc[c].im; }
+    }
+    __syncthreads();
+    cplx t = C(0, 0);
+    if ((int)threadIdx.x < cnt)
+        for (int w = 0; w < 8; ++w) { t.re += red[0][threadIdx.x][w]; t.im += red[1][threadIdx.x][w]; }
+    return t;
+}
+
+// scattered_field_kernel for solutions [SOL_CHUNK * blockIdx.y, +SOL_CHUNK) of ps / vs ([nsol][n], DOF order): the geometry
+// and Green's function of a (point, element, quadrature point) are computed once for the whole chunk.
+__global__ void __launch_bounds__(256)
+scattered_field_batch_kernel(const double* __restrict__ coords, uint32_t n, const double* __restrict__ eval, uint32_t n_eval,
+                             uint32_t nsol, const cplx* __restrict__ ps, const cplx* __restrict__ vs, double wavruim,
+                             cplx* __restrict__ out) {
+    const double x0 = eval[3 * blockIdx.x], x1 = eval[3 * blockIdx.x + 1], x2 = eval[3 * blockIdx.x + 2];
+    const uint32_t s0 = blockIdx.y * SOL_CHUNK;
+    const int cnt = (int)min((uint32_t)SOL_CHUNK, nsol - s0);
+    cplx acc[SOL_CHUNK];
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) acc[c] = C(0, 0);
+    for (uint32_t j = threadIdx.x; j < n; j += blockDim.x) {
+        const double* c_ = coords + 12ull * j;
+        const double e1[3] = {c_[3] - c_[0], c_[4] - c_[1], c_[5] - c_[2]};
+        const double e2[3] = {c_[6] - c_[0], c_[7] - c_[1], c_[8] - c_[2]};
+        const double nv[3] = {e1[1] * e2[2] - e1[2] * e2[1], e1[2] * e2[0] - e1[0] * e2[2], e1[0] * e2[1] - e1[1] * e2[0]};
+        const double jac = sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]);
+        if (jac < 1e-15) continue;
+        const double en[3] = {nv[0] / jac, nv[1] / jac, nv[2] / jac};
+        cplx p_surf[SOL_CHUNK], v_surf[SOL_CHUNK];
+        bool has_v[SOL_CHUNK];
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c) {
+            const uint64_t at = (uint64_t)(s0 + c) * n + j;
+            p_surf[c] = c < cnt ? ps[at] : C(0, 0);
+            v_surf[c] = (vs && c < cnt) ? vs[at] : C(0, 0);
+            has_v[c] = sqrt(v_surf[c].re * v_surf[c].re + v_surf[c].im * v_surf[c].im) > 1e-15;
+        }
+        cplx res[SOL_CHUNK];
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c) res[c] = C(0, 0);
+#pragma unroll
+        for (int q = 0; q < 7; ++q) {
+            const double xi = d_tr7[q][0], eta = d_tr7[q][1], wq = d_tr7[q][2] * 0.5;
+            const double l0 = 1.0 - xi - eta;
+            const double rv[3] = {l0 * c_[0] + xi * c_[3] + eta * c_[6] - x0, l0 * c_[1] + xi * c_[4] + eta * c_[7] - x1,
+                                  l0 * c_[2] + xi * c_[5] + eta * c_[8] - x2};
+            const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
+            if (r < 1e-15) continue;
+            const double vjacwe = jac * wq;
+            double sn, cs;
+            sincos(wavruim * r, &sn, &cs);
+            const double re1 = 4.0 * PI * r;
+            const cplx zg = C(cs / re1, sn / re1);
+            const cplx zgikr = zg * C(-1.0 / r, wavruim);
+            const double drdn = (rv[0] * en[0] + rv[1] * en[1] + rv[2] * en[2]) / r;
+            const cplx dgdn = zgikr * drdn;
+#pragma unroll
+            for (int c = 0; c < SOL_CHUNK; ++c) {
+                res[c] += p_surf[c] * dgdn * vjacwe;
+                if (has_v[c]) res[c] -= v_surf[c] * zg * vjacwe;
+            }
+        }
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c) acc[c] += res[c];
+    }
+    const cplx t = block_sum_chunk(acc, cnt);
+    if ((int)threadIdx.x < cnt) out[(uint64_t)(s0 + threadIdx.x) * n_eval + blockIdx.x] = t;
+}
+
+// rcs_kernel for solutions [SOL_CHUNK * blockIdx.y, +SOL_CHUNK): sincos(-k c_j.d) and n_j.d once per (element, direction).
+__global__ void __launch_bounds__(256, 2)  // (256) alone lets ptxas cap it at 64 registers and spill the accumulators
+rcs_batch_kernel(const double* __restrict__ src, const double* __restrict__ area, uint32_t n, const double* __restrict__ dirs,
+                 uint32_t n_dirs, uint32_t nsol, const cplx* __restrict__ ps, double k, double* __restrict__ out) {
+    const double d0 = dirs[3 * blockIdx.x], d1 = dirs[3 * blockIdx.x + 1], d2 = dirs[3 * blockIdx.x + 2];
+    const uint32_t s0 = blockIdx.y * SOL_CHUNK;
+    const int cnt = (int)min((uint32_t)SOL_CHUNK, nsol - s0);
+    cplx acc[SOL_CHUNK];
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) acc[c] = C(0, 0);
+    for (uint32_t j = threadIdx.x; j < n; j += blockDim.x) {
+        const double* c_ = src + 8ull * j;
+        const double phase = -k * (c_[0] * d0 + c_[1] * d1 + c_[2] * d2);
+        double sn, cs;
+        sincos(phase, &sn, &cs);
+        const double n_dot_d = c_[3] * d0 + c_[4] * d1 + c_[5] * d2;
+        const double a = area[j];
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c) {
+            if (c < cnt) {
+                const cplx t = ((ps[(uint64_t)(s0 + c) * n + j] * C(cs, sn)) * a) * C(0.0, k);
+                acc[c] += t * n_dot_d;
+            }
+        }
+    }
+    const cplx t = block_sum_chunk(acc, cnt);
+    if ((int)threadIdx.x < cnt) out[(uint64_t)(s0 + threadIdx.x) * n_dirs + blockIdx.x] = 4.0 * 3.14159265358979323846 * (t.re * t.re + t.im * t.im);
+}
+
+// b[s] = sys + inc[s] for the nrhs columns of a block (in place: out may be inc), the one IEEE add of bemb200_sweep_next
+__global__ void add_system_rhs_kernel(const cplx* __restrict__ sys, const cplx* inc, uint64_t n, uint64_t total, cplx* out) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x)
+        out[i] = sys[i % n] + inc[i];
+}
+
 }  // namespace
+
+cudaError_t bemb::launch_add_system_rhs(const cplx* sys, const cplx* inc, uint64_t n, uint32_t nrhs, cplx* out, cudaStream_t s) {
+    const uint64_t total = n * nrhs;
+    if (total == 0) return cudaSuccess;
+    const uint64_t blocks = (total + 255) / 256;
+    add_system_rhs_kernel<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, s>>>(sys, inc, n, total, out);
+    return cudaGetLastError();
+}
+
+// true when p is device (or managed) memory of `device`
+bool bemb::device_ptr_on(int device, const void* p) {
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == device;
+}
 
 extern "C" int bemb200_incident_rhs(const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re, double beta_im,
                                     uint32_t n_sources, const int32_t* kinds, const double* vecs, const double* amps,
@@ -244,5 +425,164 @@ extern "C" int bemb200_compute_rcs(const bemb200_staged_mesh* sm, const bemb200_
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     cudaFreeAsync(ddirs, s); cudaFreeAsync(dout, s); cudaFreeAsync(dps, s);
     if (e != cudaSuccess) return cuda_fail(ctx, e, "compute_rcs");
+    return BEMB200_OK;
+}
+
+namespace {
+
+// Surface values of nsol solutions ([nsol][n] complex128, DOF order) on the device: the caller's device array, or an upload of
+// the host array into *tmp.
+cudaError_t solutions_on_device(const double* values, int on_device, size_t count, cudaStream_t s, cplx** tmp, const cplx** out) {
+    if (on_device) {
+        *out = (const cplx*)values;
+        return cudaSuccess;
+    }
+    cudaError_t e = cudaMallocAsync((void**)tmp, (count ? count : 1) * sizeof(cplx), s);
+    if (e == cudaSuccess && count) e = cudaMemcpyAsync(*tmp, values, count * sizeof(cplx), cudaMemcpyHostToDevice, s);
+    *out = *tmp;
+    return e;
+}
+
+}  // namespace
+
+extern "C" int bemb200_incident_rhs_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re, double beta_im,
+                                          uint32_t nrhs, const uint32_t* src_ptr, const int32_t* kinds, const double* vecs,
+                                          const double* amps, const bemb200_matrix* system, double* b_host, double* b_dev) {
+    if (!sm || !phys || !src_ptr || !kinds || !vecs || !amps || (!b_host && !b_dev)) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    bemb200_ctx* ctx = sm->ctx;
+    if (nrhs == 0 || nrhs > 4096) return set_error(ctx, BEMB200_EINVAL, "need 1..4096 right-hand sides");
+    if (src_ptr[0] != 0) return set_error(ctx, BEMB200_EINVAL, "src_ptr[0] must be 0");
+    for (uint32_t s = 0; s < nrhs; ++s)
+        if (src_ptr[s + 1] < src_ptr[s]) return set_error(ctx, BEMB200_EINVAL, "src_ptr must be non-decreasing");
+    const uint32_t n_sources = src_ptr[nrhs];
+    if (n_sources > 65536) return set_error(ctx, BEMB200_EINVAL, "at most 65536 sources in all");
+    for (uint32_t s = 0; s < n_sources; ++s)
+        if (kinds[s] != 0 && kinds[s] != 1) return set_error(ctx, BEMB200_EINVAL, "source kind must be 0 (plane wave) or 1 (point source)");
+    const uint32_t n = sm->dm.n;
+    if (system) {
+        if (system->n_rows != n || system->n_cols != n) return set_error(ctx, BEMB200_EINVAL, "system does not match the staged mesh");
+        if (system->ctx->device != ctx->device) return set_error(ctx, BEMB200_EINVAL, "system lives on another device than the staged mesh");
+    }
+    if (b_dev && !device_ptr_on(ctx->device, b_dev)) return set_error(ctx, BEMB200_EINVAL, "b_dev is not device memory of the staged mesh's device");
+    std::vector<Source> hs(n_sources ? n_sources : 1);
+    for (uint32_t s = 0; s < n_sources; ++s) {
+        hs[s].kind = kinds[s];
+        for (int d = 0; d < 3; ++d) hs[s].v[d] = vecs[3 * s + d];
+        hs[s].amp = C(amps[2 * s], amps[2 * s + 1]);
+    }
+    // TbemSystem.rhs of every row, gathered as bemb200_rhs_download_full gathers it (collective on a row-sharded operator)
+    struct DevMem {
+        cudaStream_t s;
+        void* p = nullptr;
+        ~DevMem() { if (p) cudaFreeAsync(p, s); }  // after the kernel on the staged mesh's stream
+    } sys{ctx->stream};
+    if (system) {
+        BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+        BEMB_CUDA(ctx, cudaMallocAsync(&sys.p, (size_t)(n ? n : 1) * sizeof(cplx), ctx->stream));
+        BEMB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the system's stream writes it next
+        int rc = rhs_full(const_cast<bemb200_matrix*>(system), (double*)sys.p, cudaMemcpyDeviceToDevice);
+        if (rc != BEMB200_OK) return set_error(ctx, rc, bemb200_last_error(system->ctx));
+    }
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t total = (size_t)nrhs * n;
+    cudaStream_t st = ctx->stream;
+    Source* dsrc = nullptr;
+    uint32_t* dgrp = nullptr;
+    cplx* dout = (cplx*)b_dev;
+    cplx* tmp = nullptr;
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dsrc, hs.size() * sizeof(Source), st));
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dgrp, (nrhs + 1) * sizeof(uint32_t), st));
+    if (!dout) {
+        BEMB_CUDA(ctx, cudaMallocAsync((void**)&tmp, (total ? total : 1) * sizeof(cplx), st));
+        dout = tmp;
+    }
+    cudaError_t e = cudaMemcpyAsync(dsrc, hs.data(), hs.size() * sizeof(Source), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dgrp, src_ptr, (nrhs + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n) {
+        incident_rhs_batch_kernel<<<dim3((n + 255) / 256, nrhs), 256, 0, st>>>(sm->dm.src, n, dsrc, dgrp, phys->wave_number, phys->gamma,
+                                                                            phys->tau, C(beta_re, beta_im), (const cplx*)sys.p, dout);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess && b_host && total) e = cudaMemcpyAsync(b_host, dout, total * sizeof(cplx), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    cudaFreeAsync(dsrc, st);
+    cudaFreeAsync(dgrp, st);
+    if (tmp) cudaFreeAsync(tmp, st);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "incident_rhs_batch");
+    return BEMB200_OK;
+}
+
+extern "C" int bemb200_compute_rcs_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                                         const double* surface_pressure, int on_device, uint32_t n_dirs, const double* dirs,
+                                         double* rcs_out) {
+    if (!sm || !phys || !surface_pressure || !dirs || !rcs_out) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    bemb200_ctx* ctx = sm->ctx;
+    if (nsol == 0 || nsol > 4096) return set_error(ctx, BEMB200_EINVAL, "need 1..4096 solutions");
+    if (on_device != 0 && on_device != 1) return set_error(ctx, BEMB200_EINVAL, "on_device must be 0 (host arrays) or 1 (device arrays)");
+    if (n_dirs > 0x7fffffffu) return set_error(ctx, BEMB200_EINVAL, "too many directions");
+    if (on_device && !device_ptr_on(ctx->device, surface_pressure))
+        return set_error(ctx, BEMB200_EINVAL, "surface_pressure is not device memory of the staged mesh's device");
+    if (n_dirs == 0) return BEMB200_OK;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const uint32_t n = sm->dm.n;
+    const size_t nout = (size_t)nsol * n_dirs;
+    double *ddirs = nullptr, *dout = nullptr;
+    cplx* tmp = nullptr;
+    const cplx* dps = nullptr;
+    cudaStream_t s = ctx->stream;
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&ddirs, (size_t)n_dirs * 3 * sizeof(double), s));
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dout, nout * sizeof(double), s));
+    cudaError_t e = solutions_on_device(surface_pressure, on_device, (size_t)nsol * n, s, &tmp, &dps);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ddirs, dirs, (size_t)n_dirs * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) {
+        rcs_batch_kernel<<<dim3(n_dirs, (nsol + SOL_CHUNK - 1) / SOL_CHUNK), 256, 0, s>>>(sm->dm.src, sm->dm.area, n, ddirs, n_dirs, nsol,
+                                                                                         dps, phys->wave_number, dout);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(rcs_out, dout, nout * sizeof(double), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaFreeAsync(ddirs, s); cudaFreeAsync(dout, s);
+    if (tmp) cudaFreeAsync(tmp, s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "compute_rcs_batch");
+    return BEMB200_OK;
+}
+
+extern "C" int bemb200_scattered_field_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                                             const double* surface_pressure, const double* surface_velocity, int on_device,
+                                             uint64_t n_eval, const double* eval_pts, double* out) {
+    if (!sm || !phys || !surface_pressure || !eval_pts || !out) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    bemb200_ctx* ctx = sm->ctx;
+    if (nsol == 0 || nsol > 4096) return set_error(ctx, BEMB200_EINVAL, "need 1..4096 solutions");
+    if (on_device != 0 && on_device != 1) return set_error(ctx, BEMB200_EINVAL, "on_device must be 0 (host arrays) or 1 (device arrays)");
+    if (n_eval > 0x7fffffffull) return set_error(ctx, BEMB200_EINVAL, "too many evaluation points");
+    if (on_device && (!device_ptr_on(ctx->device, surface_pressure) || (surface_velocity && !device_ptr_on(ctx->device, surface_velocity))))
+        return set_error(ctx, BEMB200_EINVAL, "surface values are not device memory of the staged mesh's device");
+    if (n_eval == 0) return BEMB200_OK;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const uint32_t n = sm->dm.n;
+    const size_t nout = (size_t)nsol * n_eval;
+    double* dev = nullptr;
+    cplx *dout = nullptr, *tmp_p = nullptr, *tmp_v = nullptr;
+    const cplx *dps = nullptr, *dvs = nullptr;
+    cudaStream_t s = ctx->stream;
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dev, n_eval * 3 * sizeof(double), s));
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dout, nout * sizeof(cplx), s));
+    cudaError_t e = solutions_on_device(surface_pressure, on_device, (size_t)nsol * n, s, &tmp_p, &dps);
+    if (e == cudaSuccess && surface_velocity) e = solutions_on_device(surface_velocity, on_device, (size_t)nsol * n, s, &tmp_v, &dvs);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dev, eval_pts, n_eval * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) {
+        scattered_field_batch_kernel<<<dim3((unsigned)n_eval, (nsol + SOL_CHUNK - 1) / SOL_CHUNK), 256, 0, s>>>(
+            sm->dm.coords, n, dev, (uint32_t)n_eval, nsol, dps, dvs, phys->wave_number * phys->harmonic_factor, dout);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaFreeAsync(dev, s); cudaFreeAsync(dout, s);
+    if (tmp_p) cudaFreeAsync(tmp_p, s);
+    if (tmp_v) cudaFreeAsync(tmp_v, s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "scattered_field_batch");
     return BEMB200_OK;
 }

@@ -14,6 +14,7 @@
 #include <cstring>
 #include <deque>
 #include <memory>
+#include <string>
 #include <thread>
 
 #include "api_internal.h"
@@ -27,6 +28,11 @@ struct SweepJob {
     bemb200_physics phys;
     double beta_re, beta_im;
     std::vector<double> rhs_extra;  // 2 n doubles or empty
+    // bemb200_sweep_submit_incident: nrhs > 0 incident right-hand sides, built by the worker into the slot's device buffer
+    uint32_t nrhs = 0;
+    std::vector<uint32_t> src_ptr;
+    std::vector<int32_t> kinds;
+    std::vector<double> vecs, amps;
     uint32_t max_iterations, restart;
     double tolerance;
     int slot = 0;
@@ -59,7 +65,26 @@ struct bemb200_sweep {
     uint32_t pc_subdomains = 0;
     std::vector<uint64_t> pc_ptr, pc_idx;
     double pc_setup_ms = 0.0;  // device time of the last preconditioner set-up
+    // per matrix slot: the incident block of the job owning the slot (nrhs x n complex128, device of ctx_asm, grow-only)
+    bemb::cplx* inc[2] = {nullptr, nullptr};
+    size_t inc_cap[2] = {0, 0};
 };
+
+// The incident block of `job` into its slot's buffer, on the assembly context right after the job's assembly (the worker
+// thread): next_batch() then only adds TbemSystem.rhs and never waits for the assembly context behind the next frequency.
+static int build_incident_block(bemb200_sweep* sw, SweepJob* job) {
+    const size_t need = (size_t)job->nrhs * sw->n;
+    if (sw->inc_cap[job->slot] < need) {
+        cudaFree(sw->inc[job->slot]);
+        sw->inc[job->slot] = nullptr;
+        sw->inc_cap[job->slot] = 0;
+        cudaError_t e = cudaMalloc((void**)&sw->inc[job->slot], (need ? need : 1) * sizeof(bemb::cplx));
+        if (e != cudaSuccess) return cuda_fail(sw->ctx_asm, e, "sweep incident block");
+        sw->inc_cap[job->slot] = need;
+    }
+    return bemb200_incident_rhs_batch(sw->staged, &job->phys, job->beta_re, job->beta_im, job->nrhs, job->src_ptr.data(), job->kinds.data(),
+                                      job->vecs.data(), job->amps.data(), nullptr, nullptr, (double*)sw->inc[job->slot]);
+}
 
 static void sweep_worker(bemb200_sweep* sw) {
     cudaSetDevice(sw->ctx_asm->device);
@@ -87,6 +112,7 @@ static void sweep_worker(bemb200_sweep* sw) {
             rc = bemb200_matrix_set_context(sw->buf[job->slot], sw->ctx_solve);  // the solver owns the handle from now on
             sw->buf_handed[job->slot] = rc == BEMB200_OK;
         }
+        if (rc == BEMB200_OK && job->nrhs > 0) rc = build_incident_block(sw, job.get());
         {
             std::lock_guard<std::mutex> lk(sw->mu);
             job->rc = rc;
@@ -153,13 +179,58 @@ int bemb200_sweep_submit(bemb200_sweep* sw, const bemb200_physics* phys, double 
     return BEMB200_OK;
 }
 
-int bemb200_sweep_next(bemb200_sweep* sw, double* x_out, bemb200_gmres_info* info, bemb200_assembly_stats* stats, double* rhs_out) {
-    if (!sw || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+int bemb200_sweep_submit_incident(bemb200_sweep* sw, const bemb200_physics* phys, double beta_re, double beta_im, uint32_t nrhs,
+                                  const uint32_t* src_ptr, const int32_t* kinds, const double* vecs, const double* amps,
+                                  uint32_t max_iterations, uint32_t restart, double tolerance) {
+    if (!sw || !phys || !src_ptr || !kinds || !vecs || !amps) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    if (restart == 0) return set_error(sw->ctx_solve, BEMB200_EINVAL, "restart must be >= 1");
+    if (nrhs == 0 || nrhs > 32) return set_error(sw->ctx_solve, BEMB200_EINVAL, "need 1..32 right-hand sides per frequency");
+    if (src_ptr[0] != 0) return set_error(sw->ctx_solve, BEMB200_EINVAL, "src_ptr[0] must be 0");
+    for (uint32_t s = 0; s < nrhs; ++s)
+        if (src_ptr[s + 1] < src_ptr[s]) return set_error(sw->ctx_solve, BEMB200_EINVAL, "src_ptr must be non-decreasing");
+    const uint32_t ns = src_ptr[nrhs];
+    if (ns > 65536) return set_error(sw->ctx_solve, BEMB200_EINVAL, "at most 65536 sources in all");
+    for (uint32_t s = 0; s < ns; ++s)
+        if (kinds[s] != 0 && kinds[s] != 1) return set_error(sw->ctx_solve, BEMB200_EINVAL, "source kind must be 0 (plane wave) or 1 (point source)");
+    auto job = std::make_shared<SweepJob>();
+    job->phys = *phys;
+    job->beta_re = beta_re;
+    job->beta_im = beta_im;
+    job->nrhs = nrhs;
+    job->src_ptr.assign(src_ptr, src_ptr + nrhs + 1);
+    job->kinds.assign(kinds, kinds + ns);
+    job->vecs.assign(vecs, vecs + 3 * (size_t)ns);
+    job->amps.assign(amps, amps + 2 * (size_t)ns);
+    job->max_iterations = max_iterations;
+    job->restart = restart;
+    job->tolerance = tolerance;
+    {
+        std::lock_guard<std::mutex> lk(sw->mu);
+        job->slot = (int)(sw->submitted & 1u);
+        sw->submitted += 1;
+        sw->queue.push_back(job);
+    }
+    sw->cv.notify_all();
+    return BEMB200_OK;
+}
+
+}  // extern "C"
+
+// The oldest queued job: wait for its assembly, solve it, hand its slot back.  A job of more than `capacity` right-hand
+// sides stays queued (BEMB200_EINVAL).  x_out / infos hold `capacity` solutions; rhs_out (may be NULL) receives b of a
+// single right-hand side.
+static int sweep_take(bemb200_sweep* sw, uint32_t capacity, double* x_out, bemb200_gmres_info* infos, uint32_t* nrhs_out,
+                      bemb200_assembly_stats* stats, double* rhs_out) {
     std::shared_ptr<SweepJob> job;
     {
         std::unique_lock<std::mutex> lk(sw->mu);
         if (sw->queue.empty()) return set_error(sw->ctx_solve, BEMB200_EINVAL, "bemb200_sweep_next: nothing submitted");
         job = sw->queue.front();
+        const uint32_t nrhs = job->nrhs > 0 ? job->nrhs : 1;
+        if (nrhs > capacity)
+            return set_error(sw->ctx_solve, BEMB200_EINVAL,
+                             "the oldest job has " + std::to_string(nrhs) + " right-hand sides, more than the " + std::to_string(capacity) +
+                                 " the caller has room for (bemb200_sweep_next_batch takes it)");
         sw->cv.wait(lk, [&] { return job->assembled; });
         if (job->rc != BEMB200_OK) {
             sw->queue.pop_front();
@@ -172,33 +243,79 @@ int bemb200_sweep_next(bemb200_sweep* sw, double* x_out, bemb200_gmres_info* inf
         // kernels of the assembly context run beside this solve whenever another job is queued behind this one
         bemb200_ctx_set_shared_gpu(sw->ctx_solve, (sw->overlap && sw->queue.size() > 1) ? 1 : 0);
     }
+    if (nrhs_out) *nrhs_out = job->nrhs > 0 ? job->nrhs : 1;
     bemb200_matrix* m = sw->buf[job->slot];
     int rc = BEMB200_OK;
     if (stats) rc = bemb200_assembly_stats_get(m, stats);
-    std::vector<double> b(2 * sw->n);
-    if (rc == BEMB200_OK) rc = bemb200_rhs_download_full(m, b.data());  // TbemSystem.rhs (all rows)
-    if (rc == BEMB200_OK) {
-        if (!job->rhs_extra.empty())
-            for (size_t i = 0; i < b.size(); ++i) b[i] += job->rhs_extra[i];
-        if (rhs_out) std::memcpy(rhs_out, b.data(), b.size() * sizeof(double));
-        bool use_pc;
-        uint32_t nsub;
-        std::vector<uint64_t> pptr, pidx;
-        {
-            std::lock_guard<std::mutex> lk(sw->mu);
-            use_pc = sw->precond; nsub = sw->pc_subdomains; pptr = sw->pc_ptr; pidx = sw->pc_idx;
+    bool use_pc;
+    uint32_t nsub;
+    std::vector<uint64_t> pptr, pidx;
+    {
+        std::lock_guard<std::mutex> lk(sw->mu);
+        use_pc = sw->precond; nsub = sw->pc_subdomains; pptr = sw->pc_ptr; pidx = sw->pc_idx;
+    }
+    // solve(pc): the job's solve, pc = NULL or the block-Jacobi preconditioner of THIS frequency's matrix
+    auto with_precond = [&](auto solve) -> int {
+        if (!use_pc) return solve((const bemb200_precond*)nullptr);
+        bemb200_precond* pc = nullptr;  // gmres_preconditioned with the block-Jacobi preconditioner of THIS frequency's matrix
+        int r = bemb200_schwarz_create(m, nsub, pptr.empty() ? nullptr : pptr.data(), pptr.empty() ? nullptr : pidx.data(), &pc);
+        if (r == BEMB200_OK) {
+            bemb200_precond_stats st{};
+            if (bemb200_precond_stats_get(pc, &st) == BEMB200_OK) sw->pc_setup_ms = st.factor_ms;
+            r = solve(pc);
         }
-        if (!use_pc) {
-            rc = bemb200_gmres(m, b.data(), nullptr, job->max_iterations, job->restart, job->tolerance, x_out, info);
-        } else {  // gmres_preconditioned with the block-Jacobi preconditioner of THIS frequency's matrix
-            bemb200_precond* pc = nullptr;
-            rc = bemb200_schwarz_create(m, nsub, pptr.empty() ? nullptr : pptr.data(), pptr.empty() ? nullptr : pidx.data(), &pc);
+        bemb200_precond_free(pc);
+        return r;
+    };
+    if (rc == BEMB200_OK && job->nrhs == 0) {  // bemb200_sweep_submit: b = TbemSystem.rhs + rhs_extra on the host
+        std::vector<double> b(2 * sw->n);
+        rc = bemb200_rhs_download_full(m, b.data());  // TbemSystem.rhs (all rows)
+        if (rc == BEMB200_OK) {
+            if (!job->rhs_extra.empty())
+                for (size_t i = 0; i < b.size(); ++i) b[i] += job->rhs_extra[i];
+            if (rhs_out) std::memcpy(rhs_out, b.data(), b.size() * sizeof(double));
+            rc = with_precond([&](const bemb200_precond* pc) {
+                return pc ? bemb200_gmres_schwarz(m, pc, b.data(), nullptr, job->max_iterations, job->restart, job->tolerance, x_out, infos)
+                          : bemb200_gmres(m, b.data(), nullptr, job->max_iterations, job->restart, job->tolerance, x_out, infos);
+            });
+        }
+    } else if (rc == BEMB200_OK) {  // bemb200_sweep_submit_incident: b = TbemSystem.rhs + incident block, formed on the device
+        bemb200_ctx* ctx = sw->ctx_solve;
+        cplx* bdev = sw->inc[job->slot];
+        const size_t nb = (size_t)job->nrhs * sw->n * sizeof(cplx);
+        // stream-ordered: a cudaFree would wait for the next frequency's assembly running beside this solve
+        struct DevMem {
+            cudaStream_t s;
+            void* p = nullptr;
+            ~DevMem() { if (p) cudaFreeAsync(p, s); }
+        } sysv{ctx->stream}, xdev{ctx->stream};
+        cudaError_t e = cudaSetDevice(ctx->device);
+        if (e == cudaSuccess) e = cudaMallocAsync(&sysv.p, (sw->n ? sw->n : 1) * sizeof(cplx), ctx->stream);
+        if (e == cudaSuccess && job->nrhs > 1) e = cudaMallocAsync(&xdev.p, nb ? nb : 1, ctx->stream);
+        if (e != cudaSuccess) rc = cuda_fail(ctx, e, "sweep right-hand side block");
+        if (rc == BEMB200_OK) rc = rhs_full(m, (double*)sysv.p, cudaMemcpyDeviceToDevice);  // TbemSystem.rhs (all rows)
+        if (rc == BEMB200_OK) {
+            std::lock_guard<std::mutex> lk(ctx->mu);
+            e = launch_add_system_rhs((const cplx*)sysv.p, bdev, sw->n, job->nrhs, bdev, ctx->stream);
+            if (e == cudaSuccess && rhs_out) e = cudaMemcpyAsync(rhs_out, bdev, nb, cudaMemcpyDeviceToHost, ctx->stream);
+            if (e == cudaSuccess && rhs_out) e = cudaStreamSynchronize(ctx->stream);
+            if (e != cudaSuccess) rc = cuda_fail(ctx, e, "sweep right-hand side block");
+        }
+        if (rc == BEMB200_OK && job->nrhs == 1) {
+            rc = with_precond([&](const bemb200_precond* pc) {
+                return gmres_solve_device_b(m, pc, (const double*)bdev, job->max_iterations, job->restart, job->tolerance, x_out, infos);
+            });
+        } else if (rc == BEMB200_OK) {
+            rc = with_precond([&](const bemb200_precond* pc) {
+                return bemb200_gmres_batched_device(m, pc, (const double*)bdev, job->nrhs, job->max_iterations, job->restart, job->tolerance,
+                                                    (double*)xdev.p, infos, nullptr, nullptr);
+            });
             if (rc == BEMB200_OK) {
-                bemb200_precond_stats st{};
-                if (bemb200_precond_stats_get(pc, &st) == BEMB200_OK) sw->pc_setup_ms = st.factor_ms;
-                rc = bemb200_gmres_schwarz(m, pc, b.data(), nullptr, job->max_iterations, job->restart, job->tolerance, x_out, info);
+                std::lock_guard<std::mutex> lk(ctx->mu);
+                e = cudaMemcpyAsync(x_out, xdev.p, nb, cudaMemcpyDeviceToHost, ctx->stream);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+                if (e != cudaSuccess) rc = cuda_fail(ctx, e, "sweep solution block");
             }
-            bemb200_precond_free(pc);
         }
     }
     bool boost = false;
@@ -222,6 +339,19 @@ int bemb200_sweep_next(bemb200_sweep* sw, double* x_out, bemb200_gmres_info* inf
         if (nxt && sw->buf[nxt->slot] && bemb200_matrix_boost_assembly(sw->buf[nxt->slot], sw->ctx_solve) == BEMB200_OK) sw->boosts += 1;
     }
     return rc;
+}
+
+extern "C" {
+
+int bemb200_sweep_next(bemb200_sweep* sw, double* x_out, bemb200_gmres_info* info, bemb200_assembly_stats* stats, double* rhs_out) {
+    if (!sw || !x_out || !info) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    return sweep_take(sw, 1, x_out, info, nullptr, stats, rhs_out);
+}
+
+int bemb200_sweep_next_batch(bemb200_sweep* sw, uint32_t capacity, double* x_out, bemb200_gmres_info* infos, uint32_t* nrhs_out,
+                             bemb200_assembly_stats* stats) {
+    if (!sw || !x_out || !infos || !nrhs_out) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    return sweep_take(sw, capacity, x_out, infos, nrhs_out, stats, nullptr);
 }
 
 uint64_t bemb200_sweep_boosts(const bemb200_sweep* sw) { return sw ? sw->boosts : 0; }
@@ -248,6 +378,10 @@ void bemb200_sweep_destroy(bemb200_sweep* sw) {
     }
     sw->cv.notify_all();
     if (sw->worker.joinable()) sw->worker.join();
+    if (sw->inc[0] || sw->inc[1]) {
+        cudaSetDevice(sw->ctx_asm->device);
+        for (int i = 0; i < 2; ++i) cudaFree(sw->inc[i]);
+    }
     for (int i = 0; i < 2; ++i)
         if (sw->buf[i]) bemb200_matrix_free(sw->buf[i]);
     if (sw->staged) bemb200_staged_mesh_free(sw->staged);

@@ -71,6 +71,33 @@ class Sweep:
                                 converged=bool(info.converged))
         return sol, {k: getattr(st, k) for k, _ in st._fields_}, b
 
+    def submit_incident(self, physics: PhysicsParams, beta: complex, incidents, config: "bem.GmresConfig") -> None:
+        """Queue a frequency with one right-hand side per IncidentField of ``incidents`` (1..32): b = TbemSystem.rhs +
+        incident, built on the device right after the frequency's assembly.  ``next_batch`` returns its solutions."""
+        src_ptr, kinds, vecs, amps = bem.source_groups(incidents, max_groups=32)
+        ph = bem._cphys(physics)
+        beta = complex(beta)
+        self._capi.check(self._lib.bemb200_sweep_submit_incident(self._h, self._C.byref(ph), beta.real, beta.imag, src_ptr.size - 1,
+                                                                 self._capi.ptr(src_ptr), self._capi.ptr(kinds), self._capi.ptr(vecs),
+                                                                 self._capi.ptr(amps), config.max_iterations, config.restart,
+                                                                 config.tolerance), None)
+
+    def next_batch(self, capacity: int = 32):
+        """The oldest queued frequency, submitted by ``submit`` (one solution) or ``submit_incident``: (list of GmresSolution,
+        assembly stats).  A frequency with more than ``capacity`` right-hand sides raises and stays queued."""
+        if isinstance(capacity, bool) or not isinstance(capacity, (int, np.integer)) or capacity < 1:
+            raise ValueError("capacity must be a positive int")
+        capacity = int(capacity)
+        x = np.empty((capacity, self.n), dtype=np.complex128)
+        infos = (self._capi.CGmresInfo * capacity)()
+        got = self._C.c_uint32(0)
+        st = self._capi.CAssemblyStats()
+        self._capi.check(self._lib.bemb200_sweep_next_batch(self._h, capacity, self._capi.ptr(x), infos, self._C.byref(got),
+                                                            self._C.byref(st)), None)
+        sols = [bem.GmresSolution(x=x[i], iterations=int(infos[i].iterations), restarts=int(infos[i].restarts),
+                                  residual=float(infos[i].residual), converged=bool(infos[i].converged)) for i in range(got.value)]
+        return sols, {k: getattr(st, k) for k, _ in st._fields_}
+
     def solve_all(self, cases, config: "bem.GmresConfig") -> list:
         """cases: sequence of (physics, beta, rhs_extra); two frequencies are kept in flight."""
         out = []

@@ -95,6 +95,18 @@ extern "C" {
     pub fn bemb200_gmres_batched_schwarz(m: *const bemb200_matrix, precond: *const bemb200_precond, b_all: *const f64, nrhs: u32,
                                          max_iterations: u32, restart: u32, tolerance: f64, x_all: *mut f64,
                                          infos: *mut bemb200_gmres_info, block_matvec_ms: *mut f64, block_matvecs: *mut u64) -> c_int;
+    pub fn bemb200_gmres_batched_device(m: *const bemb200_matrix, precond: *const bemb200_precond, b_dev: *const f64, nrhs: u32,
+                                        max_iterations: u32, restart: u32, tolerance: f64, x_dev: *mut f64,
+                                        infos: *mut bemb200_gmres_info, block_matvec_ms: *mut f64, block_matvecs: *mut u64) -> c_int;
+    pub fn bemb200_incident_rhs_batch(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, beta_re: f64, beta_im: f64,
+                                      nrhs: u32, src_ptr: *const u32, kinds: *const i32, vecs: *const f64, amps: *const f64,
+                                      system: *const bemb200_matrix, b_host: *mut f64, b_dev: *mut f64) -> c_int;
+    pub fn bemb200_compute_rcs_batch(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, nsol: u32,
+                                     surface_pressure: *const f64, on_device: c_int, n_dirs: u32, dirs: *const f64,
+                                     rcs_out: *mut f64) -> c_int;
+    pub fn bemb200_scattered_field_batch(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, nsol: u32,
+                                         surface_pressure: *const f64, surface_velocity: *const f64, on_device: c_int,
+                                         n_eval: u64, eval_pts: *const f64, out: *mut f64) -> c_int;
     pub fn bemb200_incident_rhs(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, beta_re: f64, beta_im: f64,
                                 n_sources: u32, kinds: *const i32, vecs: *const f64, amps: *const f64, rhs_host: *mut f64,
                                 rhs_dev: *mut f64) -> c_int;
@@ -110,6 +122,11 @@ extern "C" {
                                 rhs_extra: *const f64, max_iterations: u32, restart: u32, tolerance: f64) -> c_int;
     pub fn bemb200_sweep_next(sw: *mut bemb200_sweep, x_out: *mut f64, info: *mut bemb200_gmres_info,
                               stats: *mut bemb200_assembly_stats, rhs_out: *mut f64) -> c_int;
+    pub fn bemb200_sweep_submit_incident(sw: *mut bemb200_sweep, phys: *const bemb200_physics, beta_re: f64, beta_im: f64, nrhs: u32,
+                                         src_ptr: *const u32, kinds: *const i32, vecs: *const f64, amps: *const f64,
+                                         max_iterations: u32, restart: u32, tolerance: f64) -> c_int;
+    pub fn bemb200_sweep_next_batch(sw: *mut bemb200_sweep, capacity: u32, x_out: *mut f64, infos: *mut bemb200_gmres_info,
+                                    nrhs_out: *mut u32, stats: *mut bemb200_assembly_stats) -> c_int;
     pub fn bemb200_sweep_boosts(sw: *const bemb200_sweep) -> u64;
     pub fn bemb200_sweep_set_block_jacobi(sw: *mut bemb200_sweep, num_subdomains: u32, sub_ptr: *const u64, sub_idx: *const u64) -> c_int;
     pub fn bemb200_sweep_destroy(sw: *mut bemb200_sweep);
