@@ -140,6 +140,24 @@ int bemb200_assembly_stats_get(const bemb200_matrix* m, bemb200_assembly_stats* 
 /* dg_dn_sign heuristic of tbem.rs:108-123 for this mesh and wave number */
 double bemb200_dg_dn_sign(const bemb200_staged_mesh* sm, double wave_number);
 
+/* Options of one assembly (DESIGN.md 4.8); all zero / NULL is bemb200_assemble_staged.
+ *   dg_dn_sign       0: the heuristic above (the reference's); +1 / -1: that sign at every frequency.  The sign-consistent
+ *                    formulation (+1 with consistent_beta = 1) converges to the exact solution at every ka.
+ *   consistent_beta  0: the prescribed-velocity right-hand-side integrals use the unscaled beta = i/k (the reference's);
+ *                    1: they use the beta passed to the assembly, as the free term does.
+ *   admittance       NULL, or num_dofs complex128 in DOF order: the admittance Y_j (1/m, constant over the element) of an
+ *                    absorbing velocity-BC element, v_j = vbar_j + Y_j p_j with v = dp/dn_y.  Passive surfaces have
+ *                    Im Y <= 0 for harmonic_factor = +1.  A non-zero Y on a pressure or transfer element is BEMB200_EINVAL. */
+typedef struct bemb200_assembly_options {
+    int32_t dg_dn_sign;
+    int32_t consistent_beta;
+    const double* admittance;
+} bemb200_assembly_options;
+/* bemb200_assemble_staged with options (NULL: the same call); row-sharded ranks as there */
+int bemb200_assemble_staged_opts(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re,
+                                 double beta_im, const bemb200_assembly_options* opts, uint64_t row_begin, uint64_t row_end,
+                                 bemb200_matrix** inout);
+
 /* ---- matrix handle: TbemSystem (tbem.rs:13-31) / DenseOperator (solver/fmm_interface.rs:25-52) */
 /* wrap an existing host matrix: DenseOperator::new(Array2) -- rows [row_begin,row_end) of an n x n_cols matrix */
 int bemb200_matrix_from_host(bemb200_ctx* ctx, const double* a_rows, uint64_t n_rows_global, uint64_t n_cols,
@@ -399,6 +417,10 @@ uint64_t bemb200_sweep_boosts(const bemb200_sweep* sw);
  * preconditioner of bemb200_schwarz_create, rebuilt from each frequency's matrix (arguments as there; num_subdomains = 0
  * switches back to plain gmres).  The subdomains are copied. */
 int bemb200_sweep_set_block_jacobi(bemb200_sweep* sw, uint32_t num_subdomains, const uint64_t* sub_ptr, const uint64_t* sub_idx);
+/* Assemble every frequency submitted from now on (through either submit call) with these options; NULL restores the
+ * defaults.  The admittance is copied here and each submit takes the options current at that moment, so every frequency can
+ * carry its own Y(f). */
+int bemb200_sweep_set_assembly_options(bemb200_sweep* sw, const bemb200_assembly_options* opts);
 void bemb200_sweep_destroy(bemb200_sweep* sw);
 
 /* ---- one process, several devices (SURVEY 8b "Threading": every reference caller -- BemSolver::solve, qa_suite -- is one

@@ -317,6 +317,33 @@ inline TbemSystem build_tbem_system_with_beta(const StagedMesh& mesh, const Phys
           mesh.context().handle());
     return tbem_system_from_handle(mesh.context(), m, mesh.num_dofs());
 }
+// Options of one assembly (bemb200_assembly_options, DESIGN.md 4.8).  admittance: empty, or one Y per boundary element in
+// enumeration order (entry j <-> the j-th non-evaluation element), v = vbar + Y p on velocity-BC elements.
+struct AssemblyOptions {
+    int32_t dg_dn_sign = 0;        // 0: the reference's heuristic; +1 / -1 forced
+    bool consistent_beta = false;  // the prescribed-velocity right-hand side takes the assembly's beta
+    std::vector<Complex64> admittance;
+    static AssemblyOptions sign_consistent(std::vector<Complex64> y = {}) {
+        AssemblyOptions o;
+        o.dg_dn_sign = 1;
+        o.consistent_beta = true;
+        o.admittance = std::move(y);
+        return o;
+    }
+};
+inline TbemSystem build_tbem_system_with_beta(const StagedMesh& mesh, const PhysicsParams& physics, Complex64 beta,
+                                              const AssemblyOptions& options) {
+    if (!options.admittance.empty() && options.admittance.size() != mesh.num_dofs())
+        throw Error(BEMB200_EINVAL, "admittance needs one entry per boundary element");
+    const std::vector<Complex64> y = mesh.in_dof_order(options.admittance);
+    const bemb200_assembly_options o{options.dg_dn_sign, options.consistent_beta ? 1 : 0,
+                                     y.empty() ? nullptr : reinterpret_cast<const double*>(y.data())};
+    const bemb200_physics phys = physics_abi(physics);
+    bemb200_matrix* m = nullptr;
+    check(bemb200_assemble_staged_opts(mesh.context().handle(), mesh.handle(), &phys, beta.real(), beta.imag(), &o, 0, mesh.num_dofs(), &m),
+          mesh.context().handle());
+    return tbem_system_from_handle(mesh.context(), m, mesh.num_dofs());
+}
 inline TbemSystem build_tbem_system(const Context& ctx, const std::vector<Element>& el, const std::vector<double>& nodes,
                                     const PhysicsParams& ph) {  // tbem.rs:45-51
     return build_tbem_system_with_beta(ctx, el, nodes, ph, ph.burton_miller_beta());

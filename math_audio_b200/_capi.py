@@ -46,6 +46,10 @@ class CAssemblyStats(C.Structure):
                 ("total_launches", C.c_uint64), ("far_ms", C.c_double), ("total_ms", C.c_double)]
 
 
+class CAssemblyOptions(C.Structure):
+    _fields_ = [("dg_dn_sign", C.c_int32), ("consistent_beta", C.c_int32), ("admittance", C.c_void_p)]
+
+
 class CPrecondStats(C.Structure):
     _fields_ = [("num_subdomains", C.c_uint32), ("local_subdomains", C.c_uint32), ("min_size", C.c_uint32), ("max_size", C.c_uint32),
                 ("avg_size", C.c_double), ("inverse_bytes", C.c_uint64), ("factor_ms", C.c_double), ("disjoint", C.c_int32)]
@@ -80,6 +84,8 @@ SYMBOLS = {
     "bemb200_staged_mesh_free": (None, [_VP]),
     "bemb200_staged_num_dofs": (C.c_uint64, [_VP]),
     "bemb200_assemble_staged": (C.c_int, [_VP, _VP, C.POINTER(CPhysics), C.c_double, C.c_double, C.c_uint64, C.c_uint64, _PP]),
+    "bemb200_assemble_staged_opts": (C.c_int, [_VP, _VP, C.POINTER(CPhysics), C.c_double, C.c_double, C.POINTER(CAssemblyOptions),
+                                               C.c_uint64, C.c_uint64, _PP]),
     "bemb200_assemble": (C.c_int, [_VP, C.POINTER(CMesh), C.POINTER(CPhysics), C.c_double, C.c_double, C.c_uint64, C.c_uint64, _PP]),
     "bemb200_assembly_stats_get": (C.c_int, [_VP, C.POINTER(CAssemblyStats)]),
     "bemb200_dg_dn_sign": (C.c_double, [_VP, C.c_double]),
@@ -145,6 +151,7 @@ SYMBOLS = {
     "bemb200_sweep_next_batch": (C.c_int, [_VP, C.c_uint32, _VP, C.POINTER(CGmresInfo), C.POINTER(C.c_uint32), C.POINTER(CAssemblyStats)]),
     "bemb200_sweep_boosts": (C.c_uint64, [_VP]),
     "bemb200_sweep_set_block_jacobi": (C.c_int, [_VP, C.c_uint32, _VP, _VP]),
+    "bemb200_sweep_set_assembly_options": (C.c_int, [_VP, C.POINTER(CAssemblyOptions)]),
     "bemb200_sweep_destroy": (None, [_VP]),
     "bemb200_multi_create": (C.c_int, [C.POINTER(C.c_int), C.c_int, _PP]),
     "bemb200_multi_destroy": (None, [_VP]),

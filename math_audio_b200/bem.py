@@ -218,6 +218,7 @@ class StagedMesh:
         self.num_dofs = int(self._lib.bemb200_staged_num_dofs(self._h))
         self.nbytes_host = _capi.mesh_nbytes(mesh)
         self.enum_to_dof = enumeration_to_dof(mesh)
+        self.bc_type = surface_values_in_dof_order(self.enum_to_dof, np.asarray(mesh.bc_type, dtype=np.int32)[np.asarray(mesh.is_eval) == 0])
 
     def dg_dn_sign(self, wave_number: float) -> float:
         return float(self._lib.bemb200_dg_dn_sign(self._h, wave_number))
@@ -318,12 +319,72 @@ class TbemSystem:
         return out
 
 
+@dataclass
+class AssemblyOptions:
+    """Options of one assembly (DESIGN.md 4.8, ``bemb200_assembly_options``); the defaults are the reference's assembly.
+
+    * ``dg_dn_sign``: 0 = the reference's heuristic (tbem.rs:108-123, -1 once k * mean radius >= 0.5), or a forced +1 / -1.
+    * ``consistent_beta``: the prescribed-velocity right-hand-side integrals use the assembly's beta instead of the unscaled
+      i/k.  With ``dg_dn_sign=+1`` this is the sign-consistent Burton-Miller formulation, which converges to the exact
+      solution at every ka (the reference's formulation does not above ka = 0.5).
+    * ``admittance``: None, or one complex Y per boundary element in enumeration order (entry j <-> the j-th
+      non-evaluation element, as surface vectors are passed everywhere else).  An absorbing velocity-BC element satisfies
+      v = vbar + Y p with v = dp/dn (outward normal), Y in 1/m and constant over the element.  Passive surfaces have
+      Im Y <= 0 for harmonic_factor = +1.  Only velocity-BC elements may carry a non-zero Y.
+    """
+
+    dg_dn_sign: int = 0
+    consistent_beta: bool = False
+    admittance: Optional[np.ndarray] = None
+
+    @staticmethod
+    def sign_consistent(admittance=None) -> "AssemblyOptions":
+        return AssemblyOptions(dg_dn_sign=1, consistent_beta=True, admittance=admittance)
+
+    def to_c(self, bc_type: np.ndarray, enum_to_dof: Optional[np.ndarray] = None):
+        """(CAssemblyOptions, admittance array it points to, in DOF order) for a mesh whose boundary elements have the
+        DOF-order BC types ``bc_type``.  Raises ValueError for options the library would refuse."""
+        if self.dg_dn_sign not in (-1, 0, 1):
+            raise ValueError(f"dg_dn_sign must be 0 (heuristic), +1 or -1, not {self.dg_dn_sign!r}")
+        if self.consistent_beta not in (False, True, 0, 1):
+            raise ValueError(f"consistent_beta must be a bool, not {self.consistent_beta!r}")
+        y = None
+        if self.admittance is not None:
+            y = np.asarray(self.admittance, dtype=np.complex128)
+            if y.ndim == 0:
+                y = np.full(len(bc_type), complex(y))
+            if y.shape != (len(bc_type),):
+                raise ValueError(f"admittance has {y.size} entries, the mesh has {len(bc_type)} boundary elements")
+            y = np.ascontiguousarray(surface_values_in_dof_order(enum_to_dof, y))
+            bad = np.flatnonzero((y != 0) & (np.asarray(bc_type) != 0))
+            if bad.size:
+                raise ValueError(f"admittance is allowed on velocity-BC elements only (DOF {int(bad[0])} has bc_type {int(bc_type[bad[0]])})")
+        c = _capi.CAssemblyOptions(int(self.dg_dn_sign), 1 if self.consistent_beta else 0, _capi.ptr(y) if y is not None else None)
+        return c, y
+
+
+def surface_velocity(mesh: Mesh, admittance, p: np.ndarray, v_bar: Optional[np.ndarray] = None) -> np.ndarray:
+    """v = vbar + Y p on the boundary elements (enumeration order), the surface velocity ``compute_scattered_field`` needs
+    for a solution ``p`` of a system assembled with ``AssemblyOptions(admittance=admittance)``; vbar defaults to 0."""
+    n = int((np.asarray(mesh.is_eval) == 0).sum())
+    p = np.asarray(p, dtype=np.complex128)
+    y = np.broadcast_to(np.asarray(admittance, dtype=np.complex128), (n,))
+    if p.shape != (n,):
+        raise ValueError("p has the wrong length")
+    v = y * p
+    if v_bar is not None:
+        v = np.asarray(v_bar, dtype=np.complex128) + v
+    return v
+
+
 def build_tbem_system_with_beta(elements: Mesh | StagedMesh, physics: PhysicsParams, beta: complex,
                                 ctx: Optional[Context] = None, rows=None, reuse: Optional[TbemSystem] = None,
-                                fetch_rhs: bool = True) -> TbemSystem:
+                                fetch_rhs: bool = True, options: Optional[AssemblyOptions] = None) -> TbemSystem:
     """tbem.rs:96-222.  ``elements`` carries nodes + elements (SoA).  ``rows=(r0, r1)`` assembles
     one row block (default: this rank's canonical block, i.e. everything on one GPU).
-    ``fetch_rhs=False`` leaves TbemSystem.rhs on the device (``rhs`` is None)."""
+    ``fetch_rhs=False`` leaves TbemSystem.rhs on the device (``rhs`` is None).
+    ``options`` (``AssemblyOptions``): admittance boundaries and the sign-consistent formulation; None is the reference's
+    assembly."""
     lib = _capi.lib()
     staged = elements if isinstance(elements, StagedMesh) else StagedMesh(elements, ctx)
     ctx = staged.ctx
@@ -332,7 +393,12 @@ def build_tbem_system_with_beta(elements: Mesh | StagedMesh, physics: PhysicsPar
     h = reuse.matrix._h if reuse is not None else C.c_void_p()
     ph = _cphys(physics)
     beta = complex(beta)
-    _capi.check(lib.bemb200_assemble_staged(ctx._h, staged._h, C.byref(ph), beta.real, beta.imag, r0, r1, C.byref(h)), ctx._h)
+    if options is None:
+        _capi.check(lib.bemb200_assemble_staged(ctx._h, staged._h, C.byref(ph), beta.real, beta.imag, r0, r1, C.byref(h)), ctx._h)
+    else:
+        copts, _y = options.to_c(staged.bc_type, staged.enum_to_dof)
+        _capi.check(lib.bemb200_assemble_staged_opts(ctx._h, staged._h, C.byref(ph), beta.real, beta.imag, C.byref(copts), r0, r1,
+                                                     C.byref(h)), ctx._h)
     mat = reuse.matrix if reuse is not None else DeviceMatrix(ctx, h)
     return TbemSystem(matrix=mat, rhs=mat.rhs() if fetch_rhs else None, num_dofs=n)
 
@@ -656,7 +722,8 @@ def compute_scattered_field(eval_points: np.ndarray, staged: StagedMesh, surface
 
 def compute_rcs(surface_pressure: np.ndarray, staged: StagedMesh, direction, physics: PhysicsParams):
     """postprocess/pressure.rs:438-478 on the device.  ``direction``: one unit vector (returns a float, as the
-    reference) or an (M, 3) array (returns M values, one kernel launch)."""
+    reference) or an (M, 3) array (returns M values, one kernel launch).  The far-field integral has no surface-velocity
+    term, so it is the RCS of a rigid body only: a solution with an admittance (``AssemblyOptions``) is not covered."""
     ps = np.ascontiguousarray(surface_pressure, dtype=np.complex128)
     if ps.shape != (staged.num_dofs,):
         raise ValueError("surface_pressure must have num_dofs entries")

@@ -56,6 +56,7 @@ class BemProblem:
     incident_field: IncidentField
     bc_type: BoundaryConditionType = BoundaryConditionType.Rigid
     use_burton_miller: bool = True
+    admittance: Optional[np.ndarray] = None  # Y per element (or one for all), see with_admittance
 
     @staticmethod
     def rigid_sphere_scattering(radius: float, frequency: float, speed_of_sound: float, density: float) -> "BemProblem":
@@ -79,6 +80,15 @@ class BemProblem:
         self.bc_type = bc_type
         return self
 
+    def with_admittance(self, admittance) -> "BemProblem":
+        """An absorbing surface: v = Y p on every element (v = dp/dn, outward normal), ``admittance`` one complex Y in 1/m
+        for all elements or one per element.  Passive surfaces have Im Y <= 0.  Only this builder makes a surface
+        absorbing; ``BoundaryConditionType.Impedance`` still solves a rigid body, as the reference does.  Above ka = 0.5
+        pair it with ``BemSolver.with_sign_consistent_formulation(True)``: the reference's formulation does not converge
+        to the physical solution there (DESIGN.md 4.8)."""
+        self.admittance = admittance
+        return self
+
     def with_burton_miller(self, use_bm: bool) -> "BemProblem":
         self.use_burton_miller = use_bm
         return self
@@ -97,12 +107,15 @@ class BemSolution:
     incident_field: IncidentField
     physics: PhysicsParams
     staged: Optional[bem.StagedMesh] = field(default=None, repr=False)
+    admittance: Optional[np.ndarray] = None  # the problem's admittance: the surface velocity is Y p
 
     def evaluate_pressure_field(self, points) -> List[FieldPoint]:
-        """compute_total_field (pressure.rs:273-309): incident + scattered (device field kernel)."""
+        """compute_total_field (pressure.rs:273-309): incident + scattered (device field kernel).  With an admittance the
+        scattered field takes the surface velocity v = Y p."""
         if self.staged is None:
             self.staged = bem.StagedMesh(self.mesh)
-        return compute_total_field(points, self.staged, self.surface_pressure, None, self.incident_field, self.physics)
+        v = None if self.admittance is None else bem.surface_velocity(self.mesh, self.admittance, self.surface_pressure)
+        return compute_total_field(points, self.staged, self.surface_pressure, v, self.incident_field, self.physics)
 
     def evaluate_pressure(self, point) -> complex:
         return self.evaluate_pressure_field(np.asarray(point, dtype=np.float64).reshape(1, 3))[0].p_total
@@ -126,6 +139,7 @@ class BemSolver:
     tolerance: float = 1e-8
     verbose: bool = False
     beta_scale: float = 4.0
+    sign_consistent: bool = False
 
     @staticmethod
     def new() -> "BemSolver":
@@ -151,6 +165,12 @@ class BemSolver:
         self.verbose = verbose
         return self
 
+    def with_sign_consistent_formulation(self, on: bool) -> "BemSolver":
+        """Assemble with dg_dn_sign = +1 at every frequency and one beta throughout (``bem.AssemblyOptions.sign_consistent``)
+        instead of the reference's formulation; needed for physical answers above ka = 0.5 (DESIGN.md 4.8)."""
+        self.sign_consistent = on
+        return self
+
     # -- bem_solver.rs:320-350 ------------------------------------------------------------------
     def prepare_elements(self, problem: BemProblem) -> Mesh:
         import copy
@@ -173,7 +193,11 @@ class BemSolver:
         mesh = self.prepare_elements(problem)
         staged = bem.StagedMesh(mesh, ctx)
         beta = problem.physics.burton_miller_beta_scaled(self.beta_scale)
-        system = bem.build_tbem_system_with_beta(staged, problem.physics, beta)
+        options = None
+        if self.sign_consistent or problem.admittance is not None:
+            options = bem.AssemblyOptions(dg_dn_sign=1 if self.sign_consistent else 0, consistent_beta=self.sign_consistent,
+                                          admittance=problem.admittance)
+        system = bem.build_tbem_system_with_beta(staged, problem.physics, beta, options=options)
         n = mesh.num_dofs
         rows = mesh.is_eval == 0
         centers, normals = mesh.center[rows], mesh.normal[rows]
@@ -185,7 +209,7 @@ class BemSolver:
         x = self.solve_dense_system(system, rhs, stats)
         if self.verbose:
             print(f"Solution complete. Max surface pressure: {np.abs(x).max():.6f}")
-        return BemSolution(x, mesh, problem.incident_field, problem.physics, staged)
+        return BemSolution(x, mesh, problem.incident_field, problem.physics, staged, problem.admittance)
 
     # -- bem_solver.rs:435-463 ------------------------------------------------------------------
     def solve_dense_system(self, system, rhs: np.ndarray, stats: Optional[dict] = None) -> np.ndarray:

@@ -304,6 +304,7 @@ int bemb200_mesh_stage(bemb200_ctx* ctx, const bemb200_mesh* mesh, bemb200_stage
     STAGE_TRY(dev_alloc_copy(sm, &dm.area, area));
     STAGE_TRY(dev_alloc_copy(sm, &dm.src, src));
     STAGE_TRY(dev_alloc_copy(sm, &dm.bc_type, bctype));
+    sm->bc_type = bctype;
     STAGE_TRY(dev_alloc_copy(sm, &dm.bc_len, bclen));
     STAGE_TRY(dev_alloc_copy(sm, &dm.bc_val, bcval));
     STAGE_TRY(dev_alloc_copy(sm, &dm.nonzero_bc, nz));
@@ -395,6 +396,7 @@ void bemb200_matrix_free(bemb200_matrix* m) {
     free_workspace(m);
     if (m->A) cudaFree(m->A);
     if (m->rhs) cudaFree(m->rhs);
+    if (m->adm) cudaFree(m->adm);
     if (m->near_list) cudaFree(m->near_list);
     if (m->near_count) cudaFree(m->near_count);
     if (m->work_counters) cudaFree(m->work_counters);
@@ -405,13 +407,40 @@ void bemb200_matrix_free(bemb200_matrix* m) {
     delete m;
 }
 
+}  // extern "C" (reopened below)
+namespace bemb {
+int check_assembly_options(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, const bemb200_assembly_options* opts) {
+    if (!opts) return BEMB200_OK;
+    if (opts->dg_dn_sign != 0 && opts->dg_dn_sign != 1 && opts->dg_dn_sign != -1)
+        return set_error(ctx, BEMB200_EINVAL, "dg_dn_sign must be 0 (heuristic), +1 or -1");
+    if (opts->consistent_beta != 0 && opts->consistent_beta != 1) return set_error(ctx, BEMB200_EINVAL, "consistent_beta must be 0 or 1");
+    if (opts->admittance)
+        for (uint32_t j = 0; j < sm->dm.n; ++j)
+            if (sm->bc_type[j] != 0 && (opts->admittance[2 * j] != 0.0 || opts->admittance[2 * j + 1] != 0.0))
+                return set_error(ctx, BEMB200_EINVAL, "admittance is allowed on velocity-BC elements only (DOF " + std::to_string(j) +
+                                                          " has bc_type " + std::to_string(sm->bc_type[j]) + ")");
+    return BEMB200_OK;
+}
+}  // namespace bemb
+extern "C" {
+
 int bemb200_assemble_staged(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re,
                             double beta_im, uint64_t row_begin, uint64_t row_end, bemb200_matrix** inout) {
+    return bemb200_assemble_staged_opts(ctx, sm, phys, beta_re, beta_im, nullptr, row_begin, row_end, inout);
+}
+
+int bemb200_assemble_staged_opts(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, const bemb200_physics* phys, double beta_re,
+                                 double beta_im, const bemb200_assembly_options* opts, uint64_t row_begin, uint64_t row_end,
+                                 bemb200_matrix** inout) {
     if (!ctx) return set_error(nullptr, BEMB200_EINVAL, "ctx is NULL");
     if (!sm || !phys || !inout) return set_error(ctx, BEMB200_EINVAL, "NULL argument");
     const DeviceMesh& dm = sm->dm;
     if (row_begin > row_end || row_end > dm.n) return set_error(ctx, BEMB200_EINVAL, "row range outside [0, num_dofs]");
     if (!(phys->wave_number > 0.0)) return set_error(ctx, BEMB200_EINVAL, "wave_number must be > 0");
+    if (check_assembly_options(ctx, sm, opts) != BEMB200_OK) return BEMB200_EINVAL;
+    bool has_adm = false;
+    if (opts && opts->admittance)
+        for (uint64_t j = 0; j < 2ull * dm.n && !has_adm; ++j) has_adm = opts->admittance[j] != 0.0;
     std::lock_guard<std::mutex> lk(ctx->mu);
     BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
     bemb200_matrix* m = *inout;
@@ -431,6 +460,9 @@ int bemb200_assemble_staged(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, con
     ph.sign = bemb200_dg_dn_sign(sm, phys->wave_number);
     ph.beta = C(beta_re, beta_im);
     ph.beta_unscaled = phys->tau > 0.0 ? C(0.0, phys->harmonic_factor / phys->wave_number) : C(0.0, 0.0);  // types.rs:64-70
+    ph.adm = nullptr;
+    if (opts && opts->dg_dn_sign != 0) ph.sign = (double)opts->dg_dn_sign;
+    if (opts && opts->consistent_beta) ph.beta_unscaled = ph.beta;
     const uint64_t nloc = row_end - row_begin;
     cudaStream_t s = ctx->stream;
     int rc = BEMB200_OK;
@@ -445,6 +477,11 @@ int bemb200_assemble_staged(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, con
         if (_e != cudaSuccess) return fail(cuda_fail(ctx, _e, #call)); \
     } while (0)
     ASM_CUDA(cudaMemsetAsync(m->rhs, 0, (nloc + 1) * sizeof(cplx), s));
+    if (has_adm) {  // an all-zero admittance launches exactly the kernels of an assembly without one
+        if (!m->adm) ASM_CUDA(cudaMalloc((void**)&m->adm, (size_t)dm.n * sizeof(cplx)));
+        ASM_CUDA(cudaMemcpyAsync(m->adm, opts->admittance, (size_t)dm.n * sizeof(cplx), cudaMemcpyHostToDevice, s));
+        ph.adm = m->adm;
+    }
     if (dm.n_special) ASM_CUDA(cudaMemsetAsync(m->A, 0, nloc * dm.n * sizeof(cplx), s));  // transfer-BC columns stay 0
     ASM_CUDA(cudaEventRecord(m->ev[0], s));
     for (int attempt = 0; attempt < 2; ++attempt) {

@@ -81,6 +81,7 @@ struct bemb200_staged_mesh {
     bemb200_ctx* ctx = nullptr;
     bemb::DeviceMesh dm;
     std::vector<void*> allocs;
+    std::vector<int32_t> bc_type;  // host copy, DOF order: admittance is allowed on velocity-BC elements only
 };
 
 struct GmresWorkspace;  // gmres.cu
@@ -91,6 +92,7 @@ struct bemb200_matrix {
     uint64_t r0 = 0, r1 = 0;          // local rows
     bemb::cplx* A = nullptr;          // (r1-r0) x n_cols, row-major
     bemb::cplx* rhs = nullptr;        // r1-r0
+    bemb::cplx* adm = nullptr;        // n_cols: admittance of the last assembly with options (allocated on first use)
     uint2* near_list = nullptr;
     unsigned int near_cap = 0;
     unsigned int* near_count = nullptr;
@@ -113,6 +115,8 @@ struct bemb200_matrix {
 namespace bemb {
 int set_error(bemb200_ctx* ctx, int code, const std::string& msg);
 int cuda_fail(bemb200_ctx* ctx, cudaError_t e, const char* what);
+// BEMB200_OK, or the error (set on ctx) for options bemb200_assemble_staged_opts would refuse
+int check_assembly_options(bemb200_ctx* ctx, const bemb200_staged_mesh* sm, const bemb200_assembly_options* opts);
 void free_workspace(bemb200_matrix* m);
 void free_peer_exchange(bemb200_ctx* ctx, bool collective);
 // true when p is device (or managed) memory of `device` (postprocess.cu)

@@ -500,6 +500,15 @@ __device__ __forceinline__ cplx combine(const Acc& a, int field_bc_type, const P
     return C(0, 0);
 }
 
+// admittance column (DESIGN.md 4.8): v_j = vbar_j + Y_j p_j moves -Y_j (gamma tau G + beta H^T) to the left-hand side; G and H^T
+// are the integrals of this pair (no dg_dn_sign), beta the assembly's
+__device__ __forceinline__ cplx admittance_term(const Acc& a, cplx y, const Phys& ph) {
+    cplx gam = C(ph.gamma, 0.0), tau = C(ph.tau, 0.0);
+    return y * (a.g * gam * tau + a.ht * ph.beta);
+}
+__device__ __forceinline__ cplx admittance_of(const Phys& ph, uint32_t col) { return ph.adm ? ph.adm[col] : C(0.0, 0.0); }
+__device__ __forceinline__ bool nonzero(cplx z) { return z.re != 0.0 || z.im != 0.0; }
+
 __device__ __forceinline__ void atomic_add_cplx(cplx* p, cplx v) {
     atomicAdd(&p->re, v.re);
     atomicAdd(&p->im, v.im);
@@ -521,7 +530,10 @@ __device__ void do_pair(WarpScratch& ws, const DeviceMesh& m, const Phys& ph, ui
     for (int i = 0; i < 4; ++i) bc[i] = m.bc_val[4ull * col + i];
     Acc a = regular_integration_warp(ws, src, nx, c, et, m.area[col], ph, bc, fbl, fbt, crhs, lane);
     if (lane == 0) {
-        A[(uint64_t)(row - row_begin) * lda + col] = combine(a, fbt, ph);
+        cplx coeff = combine(a, fbt, ph);
+        const cplx y = admittance_of(ph, col);
+        if (nonzero(y)) coeff -= admittance_term(a, y, ph);
+        A[(uint64_t)(row - row_begin) * lda + col] = coeff;
         if (crhs) atomic_add_cplx(&rhs[row - row_begin], a.rhs);
     }
 }
@@ -587,6 +599,11 @@ self_kernel(DeviceMesh m, Phys ph, uint64_t row_begin, uint64_t row_end, cplx* A
                 r0 += avg * tau * 0.5;
             }
             diag += combine(a, bt, ph);
+            const cplx y = admittance_of(ph, (uint32_t)row);
+            if (nonzero(y)) {
+                diag -= admittance_term(a, y, ph);
+                diag -= y * ph.beta * tau * 0.5;
+            }
             A[(row - row_begin) * lda + row] = diag;
             if (crhs) r0 += a.rhs;
             atomic_add_cplx(&rhs[row - row_begin], r0);

@@ -56,14 +56,17 @@ __device__ double2 d_sincos_tab[SINCOS_TAB];  // (cos, sin)(i*pi/1024), filled b
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-template <int NQ, bool BIMAG, int MINB>
+// ADM: the instantiation for assemblies with admittance columns (DESIGN.md 4.8).  A tile that holds one accumulates, in the
+// same quadrature loop, T_ij = sum_q zg_q (gamma tau + beta (m rho^2 - i k m rho)) = gamma tau G_ij + beta H^T_ij and stores
+// A_ij - Y_j T_ij; its Y = 0 columns, and every column of the other tiles, keep the instruction sequence of ADM = false.
+template <int NQ, bool BIMAG, int MINB, bool ADM>
 __global__ void __launch_bounds__(TILE, MINB)
 far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, const uint8_t* __restrict__ col_class,
            const double* __restrict__ srcdat, uint32_t n, uint64_t row_begin, uint64_t row_end, uint32_t rows_per_block,
            uint32_t nchunks, uint32_t total_items, uint32_t items_per_block,
            double wavruim, CisConst cis, double k2, double cH, double beta_re, double beta_im, cplx* __restrict__ A, uint64_t lda,
            uint2* __restrict__ near_list, unsigned int near_cap, unsigned int* __restrict__ near_count,
-           unsigned int* __restrict__ work_counter) {
+           unsigned int* __restrict__ work_counter, const cplx* __restrict__ adm, double gamtau) {
     __shared__ __align__(128) double sm_k[NQ * TILE];  // kappa_q, [q][column]
     __shared__ uint32_t s_item;
     extern __shared__ __align__(16) double2 sm_tab[];  // [SINCOS_TAB] (cos, sin) table: 32 KB, dynamic (static + dynamic > 48 KB)
@@ -95,6 +98,8 @@ far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, c
     double nyx = 0, nyy = 0, nyz = 0, j4pi = 0, y0x = 0, y0y = 0, y0z = 0, thr = 0, e1x = 0, e1y = 0, e1z = 0, e2x = 0, e2y = 0,
            e2z = 0, kc = 0;
     bool active = false;
+    double yre = 0.0, yim = 0.0;  // ADM: Y of this thread's column
+    bool tile_adm = false;        // ADM: some column of the current tile has Y != 0 (block-uniform)
     uint32_t col = 0;
     const double* kq = sm_k + t;
 
@@ -134,6 +139,12 @@ far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, c
         e2x = fc[FC_E2X * TILE]; e2y = fc[FC_E2Y * TILE]; e2z = fc[FC_E2Z * TILE];
         kc = fc[FC_KC * TILE];
         active = (col < n) && (col_class[col] == want);
+        if (ADM) {
+            // per-frequency, so not part of the staged far_c record: one coalesced 16-byte load per column
+            const cplx y = col < n ? adm[col] : C(0.0, 0.0);
+            yre = y.re; yim = y.im;
+            tile_adm = __syncthreads_or(active && (yre != 0.0 || yim != 0.0)) != 0;
+        }
         {
             const uint32_t parity = loads & 1u;
             uint32_t done = 0;
@@ -195,6 +206,7 @@ far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, c
         const double c3 = bk * nn, c2 = beta_im * nn;
         const double bk3nh = bk3 * nh, b3nh = b3 * nh, bk2nh = bk2 * nh;
         double are = 0.0, aim = 0.0;
+        double tre = 0.0, tim = 0.0;  // ADM: gamma tau G + beta H^T (without J / 4 pi)
 #pragma unroll
         for (int q = 0; q < NQ; ++q) {
             const double r2 = (q == 0) ? D : fma(rc.a2[q], p1, fma(rc.b2[q], p2, D + kq[q * TILE]));
@@ -226,9 +238,30 @@ far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, c
                 are = fma(zgr, fre, fma(-zgi, fim, are));
                 aim = fma(zgr, fim, fma(zgi, fre, aim));
             }
+            if (ADM && tile_adm) {
+                // zg (gamma tau + beta (m rho^2 - i k m rho)),  zg = w rho (cs + i sn)
+                const double mr = m * rho;
+                double fr, fi;
+                if (BIMAG) {
+                    fr = fma(bk, mr, gamtau);  // beta = i b:  gamma tau + b k m rho  +  i b m rho^2
+                    fi = beta_im * (mr * rho);
+                } else {
+                    const double hr = mr * rho, hi = -(wavruim * mr);
+                    fr = fma(beta_re, hr, fma(-beta_im, hi, gamtau));
+                    fi = fma(beta_re, hi, beta_im * hr);
+                }
+                const double gw = rc.w[q] * rho;
+                tre = fma(gw, fma(cs, fr, -(sn * fi)), tre);
+                tim = fma(gw, fma(cs, fi, sn * fr), tim);
+            }
         }
         if (active) {
             double2 v = make_double2(are * j4pi, aim * j4pi);
+            if (ADM && (yre != 0.0 || yim != 0.0)) {
+                const double ur = tre * j4pi, ui = tim * j4pi;
+                v.x = v.x - (yre * ur - yim * ui);
+                v.y = v.y - (yre * ui + yim * ur);
+            }
             __stcs(reinterpret_cast<double2*>(A + (row - row_begin) * lda + col), v);
         }
     }
@@ -375,7 +408,7 @@ int env_int(const char* name, int dflt) {
     return v ? std::atoi(v) : dflt;
 }
 
-template <int NQ, bool BIMAG, int MINB>
+template <int NQ, bool BIMAG, int MINB, bool ADM>
 cudaError_t launch_far_v(const DeviceMesh& m, const Phys& ph, uint64_t row_begin, uint64_t row_end, cplx* A, uint64_t lda,
                          uint2* near_list, unsigned int near_cap, unsigned int* near_count, int background_blocks_per_sm,
                          unsigned int* work_counter, FarRelaunch* relaunch, cudaStream_t s) {
@@ -400,6 +433,8 @@ cudaError_t launch_far_v(const DeviceMesh& m, const Phys& ph, uint64_t row_begin
     const uint32_t n = m.n;
     const double wavruim = ph.wavruim, k2 = ph.k2, bre = ph.beta.re, bim = ph.beta.im;
     const CisConst cis = make_cis_const(ph.wavruim);
+    const cplx* adm = ph.adm;
+    const double gamtau = ph.gamma * ph.tau;
     constexpr size_t TAB_BYTES = SINCOS_TAB * sizeof(double2);
     {
         static std::atomic<unsigned char> attr_done[64];
@@ -407,14 +442,15 @@ cudaError_t launch_far_v(const DeviceMesh& m, const Phys& ph, uint64_t row_begin
         cudaGetDevice(&dev);
         if (dev < 0 || dev >= 64) dev = 63;
         if (!attr_done[dev].load()) {
-            cudaError_t ae = cudaFuncSetAttribute(far_kernel<NQ, BIMAG, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TAB_BYTES);
+            cudaError_t ae = cudaFuncSetAttribute(far_kernel<NQ, BIMAG, MINB, ADM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TAB_BYTES);
             if (ae != cudaSuccess) return ae;
             attr_done[dev].store(1);
         }
     }
     auto launch = [=](cudaStream_t st, unsigned int g, unsigned int* ctr) -> cudaError_t {
-        far_kernel<NQ, BIMAG, MINB><<<g, TILE, TAB_BYTES, st>>>(far_k, far_c, col_class, src, n, row_begin, row_end, rpb, nchunks, total, ipb,
-                                                       wavruim, cis, k2, cH, bre, bim, A, lda, near_list, near_cap, near_count, ctr);
+        far_kernel<NQ, BIMAG, MINB, ADM><<<g, TILE, TAB_BYTES, st>>>(far_k, far_c, col_class, src, n, row_begin, row_end, rpb, nchunks, total,
+                                                            ipb, wavruim, cis, k2, cH, bre, bim, A, lda, near_list, near_cap, near_count, ctr,
+                                                            adm, gamtau);
         return cudaGetLastError();
     };
     if (counter && relaunch) {
@@ -431,8 +467,14 @@ cudaError_t launch_far_t(const DeviceMesh& m, const Phys& ph, uint64_t row_begin
                          FarRelaunch* relaunch, cudaStream_t s) {
     const bool bimag = (ph.beta.re == 0.0);
     static const int minb = env_int("BEMB200_FAR_MINB", 4);  // read once, not on every launch
+    if (ph.adm) {  // admittance columns: one instantiation per beta form, at the default occupancy
+        if (bimag) return launch_far_v<NQ, true, 4, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
+                                                          relaunch, s);
+        return launch_far_v<NQ, false, 4, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
+                                                relaunch, s);
+    }
 #define FAR_DISPATCH(B, M) \
-    return launch_far_v<NQ, B, M>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter, relaunch, s)
+    return launch_far_v<NQ, B, M, false>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter, relaunch, s)
     if (bimag) {
         if (minb == 2) FAR_DISPATCH(true, 2);
         if (minb == 3) FAR_DISPATCH(true, 3);

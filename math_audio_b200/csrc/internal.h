@@ -47,6 +47,9 @@ struct Phys {
     double sign;     // dg_dn_sign (tbem.rs:118-123)
     cplx beta;       // coupling passed to build_tbem_system_with_beta
     cplx beta_unscaled;  // physics.burton_miller_beta() (types.rs:64-70), used inside integrators
+    // admittance Y_j of velocity-BC column j (DOF order, device) or NULL: v_j = vbar_j + Y_j p_j moves
+    // -Y_j (gamma tau G_ij + beta H^T_ij) into A[i,j] and -Y_i beta tau / 2 into A[i,i] (DESIGN.md 4.8)
+    const cplx* adm;
 };
 
 struct AssemblyStats {
@@ -65,6 +68,7 @@ typedef std::vector<std::function<cudaError_t(cudaStream_t)>> FarRelaunch;
 cudaError_t launch_far(const DeviceMesh& m, const Phys& ph, uint64_t row_begin, uint64_t row_end, cplx* A, uint64_t lda,
                        uint2* near_list, unsigned int near_cap, unsigned int* near_count, int background_blocks_per_sm,
                        unsigned int* work_counters, FarRelaunch* relaunch, cudaStream_t s);
+// ph.adm != NULL launches the admittance instantiation of the far kernel (its Y = 0 columns keep the bits of the plain one)
 // right-hand-side term of the un-subdivided (row, non-zero-velocity column) pairs; same near/far split as launch_far
 cudaError_t launch_rhs_far(const DeviceMesh& m, const Phys& ph, uint64_t row_begin, uint64_t row_end, cplx* rhs, cudaStream_t s);
 cudaError_t launch_near_list(const DeviceMesh& m, const Phys& ph, uint64_t row_begin, cplx* A, uint64_t lda, cplx* rhs,

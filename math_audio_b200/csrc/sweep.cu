@@ -24,9 +24,17 @@ using namespace bemb;
 // =============================================================================================================
 // sweep
 // =============================================================================================================
+// bemb200_assembly_options with the admittance owned (empty: none)
+struct AssemblyOptionsCopy {
+    int32_t dg_dn_sign = 0, consistent_beta = 0;
+    std::vector<double> admittance;
+    bemb200_assembly_options view() const { return {dg_dn_sign, consistent_beta, admittance.empty() ? nullptr : admittance.data()}; }
+};
+
 struct SweepJob {
     bemb200_physics phys;
     double beta_re, beta_im;
+    AssemblyOptionsCopy opts;  // bemb200_sweep_set_assembly_options current at submit
     std::vector<double> rhs_extra;  // 2 n doubles or empty
     // bemb200_sweep_submit_incident: nrhs > 0 incident right-hand sides, built by the worker into the slot's device buffer
     uint32_t nrhs = 0;
@@ -65,6 +73,7 @@ struct bemb200_sweep {
     uint32_t pc_subdomains = 0;
     std::vector<uint64_t> pc_ptr, pc_idx;
     double pc_setup_ms = 0.0;  // device time of the last preconditioner set-up
+    AssemblyOptionsCopy opts;  // assembly options of every frequency submitted from now on (bemb200_sweep_set_assembly_options)
     // per matrix slot: the incident block of the job owning the slot (nrhs x n complex128, device of ctx_asm, grow-only)
     bemb::cplx* inc[2] = {nullptr, nullptr};
     size_t inc_cap[2] = {0, 0};
@@ -107,7 +116,9 @@ static void sweep_worker(bemb200_sweep* sw) {
             foreground = job == sw->queue.front();
         }
         bemb200_ctx_set_background(sw->ctx_asm, (sw->overlap && !foreground) ? sw->background : 0);
-        int rc = bemb200_assemble_staged(sw->ctx_asm, sw->staged, &job->phys, job->beta_re, job->beta_im, sw->r0, sw->r1, &sw->buf[job->slot]);
+        const bemb200_assembly_options opts = job->opts.view();
+        int rc = bemb200_assemble_staged_opts(sw->ctx_asm, sw->staged, &job->phys, job->beta_re, job->beta_im, &opts, sw->r0, sw->r1,
+                                              &sw->buf[job->slot]);
         if (rc == BEMB200_OK && sw->overlap && !sw->buf_handed[job->slot]) {
             rc = bemb200_matrix_set_context(sw->buf[job->slot], sw->ctx_solve);  // the solver owns the handle from now on
             sw->buf_handed[job->slot] = rc == BEMB200_OK;
@@ -171,6 +182,7 @@ int bemb200_sweep_submit(bemb200_sweep* sw, const bemb200_physics* phys, double 
     job->tolerance = tolerance;
     {
         std::lock_guard<std::mutex> lk(sw->mu);
+        job->opts = sw->opts;
         job->slot = (int)(sw->submitted & 1u);
         sw->submitted += 1;
         sw->queue.push_back(job);
@@ -206,6 +218,7 @@ int bemb200_sweep_submit_incident(bemb200_sweep* sw, const bemb200_physics* phys
     job->tolerance = tolerance;
     {
         std::lock_guard<std::mutex> lk(sw->mu);
+        job->opts = sw->opts;
         job->slot = (int)(sw->submitted & 1u);
         sw->submitted += 1;
         sw->queue.push_back(job);
@@ -367,6 +380,20 @@ int bemb200_sweep_set_block_jacobi(bemb200_sweep* sw, uint32_t num_subdomains, c
         sw->pc_ptr.assign(sub_ptr, sub_ptr + num_subdomains + 1);
         sw->pc_idx.assign(sub_idx, sub_idx + sub_ptr[num_subdomains]);
     }
+    return BEMB200_OK;
+}
+
+int bemb200_sweep_set_assembly_options(bemb200_sweep* sw, const bemb200_assembly_options* opts) {
+    if (!sw) return set_error(nullptr, BEMB200_EINVAL, "NULL argument");
+    if (check_assembly_options(sw->ctx_solve, sw->staged, opts) != BEMB200_OK) return BEMB200_EINVAL;
+    AssemblyOptionsCopy c;
+    if (opts) {
+        c.dg_dn_sign = opts->dg_dn_sign;
+        c.consistent_beta = opts->consistent_beta;
+        if (opts->admittance) c.admittance.assign(opts->admittance, opts->admittance + 2 * sw->n);
+    }
+    std::lock_guard<std::mutex> lk(sw->mu);
+    sw->opts = std::move(c);
     return BEMB200_OK;
 }
 

@@ -46,6 +46,8 @@ class Sweep:
         _capi.check(self._lib.bemb200_sweep_create(device, rank, nranks, idbuf, C.byref(cm), 1 if overlap else 0,
                                                    background_blocks_per_sm, C.byref(self._h)), None)
         self.n = int(self._lib.bemb200_sweep_num_dofs(self._h))
+        self._enum_to_dof = bem.enumeration_to_dof(mesh)
+        self._bc_type = bem.surface_values_in_dof_order(self._enum_to_dof, np.asarray(mesh.bc_type, dtype=np.int32)[np.asarray(mesh.is_eval) == 0])
         self.mesh_nbytes = _capi.mesh_nbytes(mesh)
 
     def submit(self, physics: PhysicsParams, beta: complex, rhs_extra: Optional[np.ndarray], config: "bem.GmresConfig") -> None:
@@ -121,6 +123,16 @@ class Sweep:
         ptr[1:] = np.cumsum([len(p) for p in subdomains])
         idx = np.ascontiguousarray(np.concatenate([np.asarray(p, dtype=np.uint64) for p in subdomains]))
         self._capi.check(self._lib.bemb200_sweep_set_block_jacobi(self._h, len(subdomains), self._capi.ptr(ptr), self._capi.ptr(idx)), None)
+
+    def set_assembly_options(self, options: "Optional[bem.AssemblyOptions]") -> None:
+        """Assemble every frequency submitted from now on with ``options`` (``bem.AssemblyOptions``; None restores the
+        reference's assembly).  The admittance is copied now, so call this before each submit to give every frequency its
+        own Y(f)."""
+        if options is None:
+            self._capi.check(self._lib.bemb200_sweep_set_assembly_options(self._h, None), None)
+            return
+        copts, _y = options.to_c(self._bc_type, self._enum_to_dof)
+        self._capi.check(self._lib.bemb200_sweep_set_assembly_options(self._h, self._C.byref(copts)), None)
 
     @property
     def boosts(self) -> int:

@@ -32,6 +32,9 @@ pub struct bemb200_mesh {
 pub struct bemb200_physics { pub wave_number: f64, pub harmonic_factor: f64, pub tau: f64, pub gamma: f64 }
 /// `int apply(void* user, const double* r, double* z, uint64_t n)`: z = M^-1 r on host memory, 0 = success (`Preconditioner::apply`).
 pub type bemb200_precond_fn = Option<unsafe extern "C" fn(user: *mut c_void, r: *const f64, z: *mut f64, n: u64) -> c_int>;
+/// `bemb200_assembly_options`: admittance boundaries and the sign-consistent formulation (DESIGN.md 4.8).
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct bemb200_assembly_options { pub dg_dn_sign: i32, pub consistent_beta: i32, pub admittance: *const f64 }
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct bemb200_gmres_info { pub iterations: u64, pub restarts: u64, pub residual: f64, pub converged: i32 }
 
@@ -51,6 +54,9 @@ extern "C" {
     pub fn bemb200_assemble_staged(ctx: *mut bemb200_ctx, sm: *const bemb200_staged_mesh, phys: *const bemb200_physics,
                                    beta_re: c_double, beta_im: c_double, row_begin: u64, row_end: u64,
                                    inout: *mut *mut bemb200_matrix) -> c_int;
+    pub fn bemb200_assemble_staged_opts(ctx: *mut bemb200_ctx, sm: *const bemb200_staged_mesh, phys: *const bemb200_physics,
+                                        beta_re: c_double, beta_im: c_double, opts: *const bemb200_assembly_options, row_begin: u64,
+                                        row_end: u64, inout: *mut *mut bemb200_matrix) -> c_int;
     pub fn bemb200_assemble(ctx: *mut bemb200_ctx, mesh: *const bemb200_mesh, phys: *const bemb200_physics,
                             beta_re: c_double, beta_im: c_double, row_begin: u64, row_end: u64,
                             out: *mut *mut bemb200_matrix) -> c_int;
@@ -129,6 +135,7 @@ extern "C" {
                                     nrhs_out: *mut u32, stats: *mut bemb200_assembly_stats) -> c_int;
     pub fn bemb200_sweep_boosts(sw: *const bemb200_sweep) -> u64;
     pub fn bemb200_sweep_set_block_jacobi(sw: *mut bemb200_sweep, num_subdomains: u32, sub_ptr: *const u64, sub_idx: *const u64) -> c_int;
+    pub fn bemb200_sweep_set_assembly_options(sw: *mut bemb200_sweep, opts: *const bemb200_assembly_options) -> c_int;
     pub fn bemb200_sweep_destroy(sw: *mut bemb200_sweep);
     // one process, several devices
     pub fn bemb200_multi_create(devices: *const c_int, n: c_int, out: *mut *mut bemb200_multi) -> c_int;
