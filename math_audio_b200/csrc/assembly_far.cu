@@ -31,7 +31,6 @@
 // near-field kernel, which re-takes the decision bit-faithfully and overwrites the entry.
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 
 #include "internal.h"
 
@@ -56,11 +55,14 @@ __device__ double2 d_sincos_tab[SINCOS_TAB];  // (cos, sin)(i*pi/1024), filled b
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+// resident blocks per SM the far kernel is compiled for (registers <= 128 per thread)
+constexpr int FAR_MINB = 4;
+
 // ADM: the instantiation for assemblies with admittance columns (DESIGN.md 4.8).  A tile that holds one accumulates, in the
 // same quadrature loop, T_ij = sum_q zg_q (gamma tau + beta (m rho^2 - i k m rho)) = gamma tau G_ij + beta H^T_ij and stores
 // A_ij - Y_j T_ij; its Y = 0 columns, and every column of the other tiles, keep the instruction sequence of ADM = false.
-template <int NQ, bool BIMAG, int MINB, bool ADM>
-__global__ void __launch_bounds__(TILE, MINB)
+template <int NQ, bool BIMAG, bool ADM>
+__global__ void __launch_bounds__(TILE, FAR_MINB)
 far_kernel(const double* __restrict__ far_k, const double* __restrict__ far_c, const uint8_t* __restrict__ col_class,
            const double* __restrict__ srcdat, uint32_t n, uint64_t row_begin, uint64_t row_end, uint32_t rows_per_block,
            uint32_t nchunks, uint32_t total_items, uint32_t items_per_block,
@@ -403,20 +405,15 @@ cudaError_t upload_tables() {
     return cudaSuccess;
 }
 
-int env_int(const char* name, int dflt) {
-    const char* v = std::getenv(name);
-    return v ? std::atoi(v) : dflt;
-}
-
-template <int NQ, bool BIMAG, int MINB, bool ADM>
+template <int NQ, bool BIMAG, bool ADM>
 cudaError_t launch_far_v(const DeviceMesh& m, const Phys& ph, uint64_t row_begin, uint64_t row_end, cplx* A, uint64_t lda,
                          uint2* near_list, unsigned int near_cap, unsigned int* near_count, int background_blocks_per_sm,
                          unsigned int* work_counter, FarRelaunch* relaunch, cudaStream_t s) {
     const uint64_t nrows = row_end - row_begin;
-    // enough work items to fill 148 SMs x MINB resident blocks several times over, but row chunks
+    // enough work items to fill 148 SMs x FAR_MINB resident blocks several times over, but row chunks
     // long enough to amortise the per-block set-up
     uint32_t rpb = 128;
-    while (rpb > 8 && (uint64_t)m.ntiles * ((nrows + rpb - 1) / rpb) < 148ull * MINB * 4ull) rpb >>= 1;
+    while (rpb > 8 && (uint64_t)m.ntiles * ((nrows + rpb - 1) / rpb) < 148ull * FAR_MINB * 4ull) rpb >>= 1;
     const uint32_t nchunks = (uint32_t)((nrows + rpb - 1) / rpb);
     const uint32_t total = m.ntiles * nchunks;
     uint32_t grid = total, ipb = 1;
@@ -442,20 +439,20 @@ cudaError_t launch_far_v(const DeviceMesh& m, const Phys& ph, uint64_t row_begin
         cudaGetDevice(&dev);
         if (dev < 0 || dev >= 64) dev = 63;
         if (!attr_done[dev].load()) {
-            cudaError_t ae = cudaFuncSetAttribute(far_kernel<NQ, BIMAG, MINB, ADM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TAB_BYTES);
+            cudaError_t ae = cudaFuncSetAttribute(far_kernel<NQ, BIMAG, ADM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TAB_BYTES);
             if (ae != cudaSuccess) return ae;
             attr_done[dev].store(1);
         }
     }
     auto launch = [=](cudaStream_t st, unsigned int g, unsigned int* ctr) -> cudaError_t {
-        far_kernel<NQ, BIMAG, MINB, ADM><<<g, TILE, TAB_BYTES, st>>>(far_k, far_c, col_class, src, n, row_begin, row_end, rpb, nchunks, total,
-                                                            ipb, wavruim, cis, k2, cH, bre, bim, A, lda, near_list, near_cap, near_count, ctr,
-                                                            adm, gamtau);
+        far_kernel<NQ, BIMAG, ADM><<<g, TILE, TAB_BYTES, st>>>(far_k, far_c, col_class, src, n, row_begin, row_end, rpb, nchunks, total,
+                                                       ipb, wavruim, cis, k2, cH, bre, bim, A, lda, near_list, near_cap, near_count, ctr,
+                                                       adm, gamtau);
         return cudaGetLastError();
     };
     if (counter && relaunch) {
         // helper launch for bemb200_matrix_boost_assembly: a full-occupancy grid pulling from the same counter
-        const unsigned int hg = total < 148u * 4u ? total : 148u * 4u;
+        const unsigned int hg = total < 148u * FAR_MINB ? total : 148u * FAR_MINB;
         relaunch->push_back([=](cudaStream_t st) { return launch(st, hg, counter); });
     }
     return launch(s, grid, counter);
@@ -466,24 +463,15 @@ cudaError_t launch_far_t(const DeviceMesh& m, const Phys& ph, uint64_t row_begin
                          uint2* near_list, unsigned int near_cap, unsigned int* near_count, int bg, unsigned int* work_counter,
                          FarRelaunch* relaunch, cudaStream_t s) {
     const bool bimag = (ph.beta.re == 0.0);
-    static const int minb = env_int("BEMB200_FAR_MINB", 4);  // read once, not on every launch
-    if (ph.adm) {  // admittance columns: one instantiation per beta form, at the default occupancy
-        if (bimag) return launch_far_v<NQ, true, 4, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
-                                                          relaunch, s);
-        return launch_far_v<NQ, false, 4, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
-                                                relaunch, s);
+    if (ph.adm) {  // admittance columns: one instantiation per beta form
+        if (bimag) return launch_far_v<NQ, true, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
+                                                       relaunch, s);
+        return launch_far_v<NQ, false, true>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
+                                             relaunch, s);
     }
-#define FAR_DISPATCH(B, M) \
-    return launch_far_v<NQ, B, M, false>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter, relaunch, s)
-    if (bimag) {
-        if (minb == 2) FAR_DISPATCH(true, 2);
-        if (minb == 3) FAR_DISPATCH(true, 3);
-        if (minb == 5) FAR_DISPATCH(true, 5);
-        if (minb == 6) FAR_DISPATCH(true, 6);
-        FAR_DISPATCH(true, 4);
-    }
-    FAR_DISPATCH(false, 4);
-#undef FAR_DISPATCH
+    if (bimag) return launch_far_v<NQ, true, false>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter,
+                                                    relaunch, s);
+    return launch_far_v<NQ, false, false>(m, ph, row_begin, row_end, A, lda, near_list, near_cap, near_count, bg, work_counter, relaunch, s);
 }
 
 }  // namespace

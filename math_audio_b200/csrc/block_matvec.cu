@@ -262,9 +262,8 @@ cudaError_t launch_streamk_t(const cplx* A, uint64_t lda, uint64_t nrows, uint64
 
 }  // namespace
 
-// DMMA stream-K block matvec; same contract as launch_zgemm_block (X interleaved [k][S], Y interleaved [row][S])
-cudaError_t launch_zgemm_block_streamk(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* X, cplx* Y,
-                                       int nrhs, cudaStream_t s) {
+cudaError_t launch_zgemm_block(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* X, cplx* Y, int nrhs,
+                               cudaStream_t s) {
     if (nrows == 0) return cudaSuccess;
     if (ncols == 0) return cudaMemsetAsync(Y, 0, nrows * (size_t)nrhs * sizeof(cplx), s);
     switch (nrhs) {

@@ -11,7 +11,6 @@
 // vectors, so all ranks hold bit-identical Krylov bases and Hessenberg columns and take the
 // same convergence decisions without any all-reduce.
 #include <chrono>
-#include <cstdio>
 #include <cstdlib>
 #include <cmath>
 #include <cstring>
@@ -272,11 +271,6 @@ static void accumulate_matvec_time(bemb200_matrix* m) {
     else cudaGetLastError();
 }
 
-static const bool g_speculate = []() {
-    const char* v = std::getenv("BEMB200_GMRES_SPECULATE");
-    return v ? (std::atoi(v) != 0) : true;
-}();
-
 static int norm_of(bemb200_matrix* m, const cplx* b, const cplx* ax, cplx* r, double* out, const cplx* pinv = nullptr) {
     bemb200_ctx* ctx = m->ctx;
     GmresWorkspace* ws = m->ws;
@@ -372,6 +366,17 @@ static int update_x(bemb200_matrix* m, cplx* x, const std::vector<cplx>& y) {
 // (perfect load balance for free) outweighs the saved launches, from two ranks on the sharded Gram-Schmidt and the single
 // exchange per iteration win.
 static const int g_fused_mode = []() { const char* v = std::getenv("BEMB200_GMRES_FUSED"); return v ? (std::atoi(v) != 0 ? 1 : 0) : -1; }();
+
+// BEMB200_PEER_TIMEOUT_MS (default 4000): bound of every device-side wait for data of another rank or CTA
+static unsigned long long peer_timeout_ns() {
+    static const unsigned long long ns = []() {
+        const char* v = std::getenv("BEMB200_PEER_TIMEOUT_MS");
+        const long long ms = v ? std::atoll(v) : 4000;
+        return (unsigned long long)(ms > 0 ? ms : 4000) * 1000000ull;
+    }();
+    return ns;
+}
+
 static double g_fused_total_ms = 0.0, g_fused_matvec_ms = 0.0, g_fused_round_ms = 0.0;
 static unsigned long long g_fused_rounds = 0;
 
@@ -443,10 +448,6 @@ static int ensure_fused_exchange(bemb200_ctx* ctx, uint64_t npad, bool* ok) {
     }
     FusedLocal& fx = ctx->fx;
     int grid = ctx->fused_grid;
-    if (grid <= 0) {
-        static const int env_grid = []() { const char* v = std::getenv("BEMB200_FUSED_GRID"); return v ? std::atoi(v) : 0; }();
-        grid = env_grid;
-    }
     if (grid <= 0) {
         int sms = 0;
         BEMB_CUDA(ctx, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
@@ -529,12 +530,7 @@ static int gmres_fused_solve(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t
     p.tol = tol;
     p.ex0 = (uint32_t)px.epoch;
     p.er0 = fx.er;
-    static const unsigned long long timeout_ns = []() {
-        const char* v = std::getenv("BEMB200_PEER_TIMEOUT_MS");
-        const long long ms = v ? std::atoll(v) : 4000;
-        return (unsigned long long)(ms > 0 ? ms : 4000) * 1000000ull;
-    }();
-    p.timeout_ns = timeout_ns;
+    p.timeout_ns = peer_timeout_ns();
     p.result = static_cast<FusedResult*>(fx.result_d);
     const uint32_t G = (uint32_t)fx.grid;
     p.S = (p.nloc + G - 1) / G;
@@ -542,17 +538,16 @@ static int gmres_fused_solve(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t
     // Row ownership.  SMs do not stream from HBM equally fast (the SMs of fuller GPCs share their path to L2: 86 ... 103 ms per
     // 100 matvecs at 20 480 unknowns), and the slowest CTA sets the pace of every iteration.  The first sizeable solve of a context
     // runs with equal shares and measures rows/ns per CTA (and the SM it sat on); later solves split the slab proportionally.
-    // One refinement, then the table is frozen (same inputs -> same bits from then on); BEMB200_FUSED_BALANCE=0 keeps equal shares.
-    static const int balance = []() { const char* v = std::getenv("BEMB200_FUSED_BALANCE"); return v ? std::atoi(v) : 1; }();
+    // One refinement, then the table is frozen (same inputs -> same bits from then on).
     p.row_off = nullptr;
     p.unit_off = nullptr;
     p.units_per_row = 0;
     p.frag = fx.frag;
     std::vector<uint32_t> off;
-    const bool have_speed = balance && fx.speed.size() == G;
-    if (balance && p.nloc >= 4 * G) {
+    const bool have_speed = fx.speed.size() == G;
+    if (p.nloc >= 4 * G) {
         // CTA boundaries in units of (row, segment): shares proportional to the measured speeds (equal before the calibration)
-        const uint32_t nsegu = (p.n + fused_segment_width(polite) - 1) / fused_segment_width(polite);
+        const uint32_t nsegu = (p.n + FUSED_SEGMENT_WIDTH - 1) / FUSED_SEGMENT_WIDTH;
         const uint64_t total_units = (uint64_t)p.nloc * nsegu;
         double tot = 0.0;
         for (uint32_t c = 0; c < G; ++c) tot += have_speed ? fx.speed[c] : 1.0;
@@ -599,7 +594,6 @@ static int gmres_fused_solve(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t
     p.rblk = fused_pick_rblk(p.S);
     const size_t smem = fused_smem_bytes(p.S, p.rblk, restart);
     if (smem > 200 * 1024) return BEMB200_OK;
-    static const bool want_trace = std::getenv("BEMB200_FUSED_TRACE") != nullptr;
     p.trace = fx.trace_d;
     FusedResult* res = static_cast<FusedResult*>(fx.result_h);
     std::memset(res, 0, sizeof(FusedResult));
@@ -622,7 +616,7 @@ static int gmres_fused_solve(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t
         bool same_map = fx.smid.size() == G;
         for (uint32_t c = 0; c < G && same_map; ++c) same_map = fx.smid[c] == (unsigned)tr[4 * c + 3];
         const bool sizeable = p.nloc >= 16 * G && res->matvecs >= 10;
-        if (balance && sizeable && (fx.calib_runs < 2 || !same_map)) {
+        if (sizeable && (fx.calib_runs < 2 || !same_map)) {
             if (!same_map) fx.calib_runs = 0;
             std::vector<double> sp(G, 0.0);
             bool good = true;
@@ -636,27 +630,6 @@ static int gmres_fused_solve(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t
                 for (uint32_t c = 0; c < G; ++c) fx.smid[c] = (unsigned)tr[4 * c + 3];
                 fx.calib_runs += 1;
             }
-        }
-        if (want_trace) {
-            double mn = 1e30, mx = 0, av = 0, wmn = 1e30, wmx = 0;
-            for (uint32_t c = 0; c < G; ++c) {
-                const double t = (double)tr[4 * c] * 1e-6, w = (double)tr[4 * c + 1] * 1e-6;
-                if (t < mn) mn = t;
-                if (t > mx) mx = t;
-                av += t / G;
-                if (w < wmn) wmn = w;
-                if (w > wmx) wmx = w;
-            }
-            std::fprintf(stderr, "[fused trace rank %d] matvec ms per CTA: min %.3f max %.3f avg %.3f; round wait ms min %.3f max %.3f; total %.3f ms, %llu matvecs, "
-                         "weighted %d units %d calib_runs %d S %u\n", ctx->rank, mn, mx, av, wmn, wmx, (double)res->t_total_ns * 1e-6, res->matvecs,
-                         (p.row_off || (p.unit_off && have_speed)) ? 1 : 0, p.unit_off ? 1 : 0, fx.calib_runs, p.S);
-            if (std::getenv("BEMB200_FUSED_TRACE_FULL"))
-                for (uint32_t c = 0; c < G; c += 8) {
-                    std::fprintf(stderr, "   cta %3u:", c);
-                    for (uint32_t e = c; e < c + 8 && e < G; ++e)
-                        std::fprintf(stderr, " %7.3f/%6.3f/%llu@%llu", (double)tr[4 * e] * 1e-6, (double)tr[4 * e + 1] * 1e-6, tr[4 * e + 2], tr[4 * e + 3]);
-                    std::fprintf(stderr, "\n");
-                }
         }
     }
     if (res->error || !res->done) {
@@ -738,12 +711,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
         if (ctx->px.err_h) *ctx->px.err_h = 0;
     }
     const bool peer_fused = !P.own_step() && allow_grid && ctx->nranks > 1 && ctx->px.ok && ctx->px.npad >= ws->npad && ws->npad == ws->chunk * (uint64_t)ctx->nranks &&
-                            mgs_peer_wait_capable(n, restart, allow_grid);
-    static const unsigned long long peer_timeout_ns = []() {
-        const char* v = std::getenv("BEMB200_PEER_TIMEOUT_MS");
-        const long long ms = v ? std::atoll(v) : 4000;
-        return (unsigned long long)(ms > 0 ? ms : 4000) * 1000000ull;
-    }();
+                            mgs_peer_wait_capable(n, restart);
     struct PeerErrCheck {  // a consumer kernel that gave up waiting for a peer poisons the solve: report it
         bemb200_ctx* c; bool on;
         int check() const { return (on && c->px.err_h && *c->px.err_h) ? 1 : 0; }
@@ -787,7 +755,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
                 pw.ll = px_work(px, ctx->rank, epoch);
                 pw.epoch = (uint32_t)epoch;
                 pw.err = px.err_h;
-                pw.timeout_ns = peer_timeout_ns;
+                pw.timeout_ns = peer_timeout_ns();
             } else {
                 cplx* yloc = ws->w + (ctx->nranks > 1 ? (uint64_t)ctx->rank * ws->chunk : m->r0);
                 cplx* av = P.schwarz ? P.schwarz->tmp : yloc;  // Schwarz: A v_j into scratch, M^-1 writes the rank's rows of w
@@ -803,7 +771,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
             BEMB_CUDA(ctx, launch_mgs(ws->V, ws->npad, const_cast<cplx*>(wvec), j, n, hd, ws->V + (uint64_t)(j + 1) * ws->npad, P.pinv,
                                       direct_scale, ws->lmat_d, (int)ws->restart + 1,
                                       ws->lmat_d + (size_t)(ws->restart + 1) * (ws->restart + 1),
-                                      ws->hcol_h + (size_t)j * ws->ldh_slot, &wrote_host, allow_grid, pw, ctx->nranks > 1, s));
+                                      ws->hcol_h + (size_t)j * ws->ldh_slot, &wrote_host, pw, ctx->nranks > 1, s));
             if (!wrote_host)
                 BEMB_CUDA(ctx, cudaMemcpyAsync(ws->hcol_h + (size_t)j * ws->ldh_slot, hd, (j + 2) * sizeof(cplx),
                                                cudaMemcpyDeviceToHost, s));
@@ -819,7 +787,7 @@ static int gmres_core(bemb200_matrix* m, const cplx* b, cplx* x, uint32_t max_it
                 if (rc != BEMB200_OK) return rc;
             }
             // (never with a callback: the caller's apply runs exactly as often as in the reference)
-            if (g_speculate && !P.user && j + 1 < mm && !ws->launched[j + 1]) {
+            if (!P.user && j + 1 < mm && !ws->launched[j + 1]) {
                 rc = enqueue_iteration(j + 1);
                 if (rc != BEMB200_OK) return rc;
             }

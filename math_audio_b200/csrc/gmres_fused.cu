@@ -28,7 +28,6 @@
 // than the reference's count, the reported iteration/restart numbers are the reference's.
 #include <cooperative_groups.h>
 #include <atomic>
-#include <cstdlib>
 #include <cstring>
 
 #include "api_internal.h"
@@ -214,6 +213,7 @@ __device__ __forceinline__ void matvec_rows(const FusedParams& p, const Smem& sm
     constexpr int WCOLS = 32 * CPL;   // columns per warp and segment
     constexpr int SEGW = NW * WCOLS;  // columns per segment
     static_assert(RB == 2 || RB == 4, "rows per step");
+    static_assert(SEGW == FUSED_SEGMENT_WIDTH, "the host sizes the row-balancing units by FUSED_SEGMENT_WIDTH");
     const int tid = threadIdx.x, lane = tid & 31, wq = tid >> 5;
     const uint4* xin = p.xbuf[p.rank] + (size_t)(ex & 1u) * 2 * p.npad;
     const uint32_t n = p.n;
@@ -890,7 +890,6 @@ __device__ __forceinline__ void gmres_body(const FusedParams& p) {
 }
 
 __global__ void __launch_bounds__(FUSED_THREADS, 1) gmres_fused_kernel(const __grid_constant__ FusedParams p) { gmres_body<4, 4>(p); }
-__global__ void __launch_bounds__(FUSED_THREADS, 1) gmres_fused_kernel_w(const __grid_constant__ FusedParams p) { gmres_body<2, 8>(p); }
 // "polite" build: at most 96 registers per thread, so that a background assembly block (128 threads x 128 registers) fits
 // beside a solver CTA on every SM (frequency sweeps: assembly of f + 1 underneath the solve of f)
 __global__ void __maxnreg__(96) gmres_fused_kernel_polite(const __grid_constant__ FusedParams p) { gmres_body<2, 4>(p); }
@@ -914,20 +913,13 @@ uint32_t fused_pick_rblk(uint32_t S) {
     return r ? r : 1;
 }
 
-uint32_t fused_segment_width(bool polite) {
-    static const int variant = []() { const char* v = std::getenv("BEMB200_FUSED_VARIANT"); return v ? std::atoi(v) : 0; }();
-    return (uint32_t)(NW * 32 * ((!polite && variant == 1) ? 8 : 4));
-}
-
 cudaError_t launch_gmres_fused(const FusedParams& p, int grid, size_t smem, bool polite, cudaStream_t s) {
     static std::atomic<unsigned long long> attr_done[64];
-    static const int variant = []() { const char* v = std::getenv("BEMB200_FUSED_VARIANT"); return v ? std::atoi(v) : 0; }();
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64) dev = 63;
     if (attr_done[dev].load() < smem) {
         cudaError_t e = cudaFuncSetAttribute(gmres_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gmres_fused_kernel_w, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(gmres_fused_kernel_polite, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         attr_done[dev].store(smem);
@@ -943,7 +935,6 @@ cudaError_t launch_gmres_fused(const FusedParams& p, int grid, size_t smem, bool
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     if (polite) return cudaLaunchKernelEx(&cfg, gmres_fused_kernel_polite, p);
-    if (variant == 1) return cudaLaunchKernelEx(&cfg, gmres_fused_kernel_w, p);
     return cudaLaunchKernelEx(&cfg, gmres_fused_kernel, p);
 }
 

@@ -7,6 +7,7 @@ namespace bemb {
 constexpr int FUSED_THREADS = 512;
 constexpr int FUSED_KMAX = 160;        // complex values per reduction round / broadcast (2 (restart + 1) + 2 <= 130, padded)
 constexpr int FUSED_MAX_RESTART = 63;  // larger restarts use the per-iteration kernels of linalg.cu
+constexpr uint32_t FUSED_SEGMENT_WIDTH = FUSED_THREADS * 4;  // matrix columns per segment of the matvec (4 per thread, both builds)
 
 struct FusedResult {
     unsigned long long iterations, restarts, matvecs;
@@ -52,7 +53,6 @@ struct FusedParams {
 
 size_t fused_smem_bytes(uint32_t S, uint32_t rblk, uint32_t restart);
 uint32_t fused_pick_rblk(uint32_t S);
-uint32_t fused_segment_width(bool polite);  // matrix columns per segment of the kernel variant in use
 // polite: the 96-register build that leaves room for a background assembly block on every SM
 cudaError_t launch_gmres_fused(const FusedParams& p, int grid, size_t smem, bool polite, cudaStream_t s);
 

@@ -12,9 +12,6 @@
 //   residual / scale / update kernels for gmres.rs:143-172,238-262
 #include <cooperative_groups.h>
 #include <atomic>
-#include <cstdlib>
-
-#include <string>
 
 #include "linalg.h"
 
@@ -948,106 +945,6 @@ __global__ void cgs_p_kernel(const cplx* __restrict__ r, const cplx* __restrict_
     p[k] = uu + qp * beta;
 }
 
-// ------------------------------------------------------------------------------------------
-// K6: block matvec Y = A X for S = 8*NT right-hand sides (multi-RHS scattering, BASELINE config 5).
-// A is read ONCE for all S columns, so the op is a genuine dense contraction (8 N^2 S flops on
-// 16 N^2 bytes): FP64 tensor cores, mma.sync.m8n8k4.f64 (tcgen05 has no f64 kind).  Complex
-// product = 4 real MMAs per (k-step, n-tile).  X is [ncols][S] (RHS-interleaved), Y is [nrows][S].
-// Block = 8 warps x 8 rows; the A fragment layout (lane -> row lane/4, k lane%4) is loaded
-// straight from global (each 128-byte line is consumed by two consecutive k-steps), the X chunk
-// of 32 k's is staged in shared memory with cp.async, double buffered.
-// ------------------------------------------------------------------------------------------
-constexpr int BM_WARPS = 8;
-constexpr int BM_ROWS = BM_WARPS * 8;
-constexpr int BM_KC = 32;
-
-__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(d0), "+d"(d1)
-                 : "d"(a), "d"(b));
-}
-
-template <int NT>
-__global__ void __launch_bounds__(BM_WARPS * 32)
-zgemm_block_kernel(const cplx* __restrict__ A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* __restrict__ X,
-                   cplx* __restrict__ Y) {
-    constexpr int S = 8 * NT;
-    constexpr int XLD = S + 1;  // padded row stride (in complex) against bank conflicts
-    __shared__ __align__(16) cplx Xs[2][BM_KC * XLD];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int g = lane >> 2, kq = lane & 3;
-    const uint64_t r_out = (uint64_t)blockIdx.x * BM_ROWS + warp * 8 + g;
-    const uint64_t r = r_out < nrows ? r_out : nrows - 1;
-    const cplx* arow = A + r * lda;
-    const uint64_t nchunks = (ncols + BM_KC - 1) / BM_KC;
-
-    double acc_re[NT][2], acc_im[NT][2];
-#pragma unroll
-    for (int t = 0; t < NT; ++t) { acc_re[t][0] = acc_re[t][1] = acc_im[t][0] = acc_im[t][1] = 0.0; }
-
-    auto load_a = [&](uint64_t c, double2* dst) {
-#pragma unroll
-        for (int i = 0; i < BM_KC / 4; ++i) {
-            const uint64_t col = c * BM_KC + 4 * i + kq;
-            dst[i] = col < ncols ? __ldg(reinterpret_cast<const double2*>(arow + col)) : make_double2(0.0, 0.0);
-        }
-    };
-    auto stage_x = [&](uint64_t c, int buf) {
-        // BM_KC x S complex values, coalesced 16-byte cp.async
-        for (int e = tid; e < BM_KC * S; e += BM_WARPS * 32) {
-            const int kk = e / S, n = e - kk * S;
-            const uint64_t k = c * BM_KC + kk;
-            cplx* dst = &Xs[buf][kk * XLD + n];
-            if (k < ncols) {
-                const uint32_t sa = (uint32_t)__cvta_generic_to_shared(dst);
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(X + k * S + n) : "memory");
-            } else {
-                *dst = C(0, 0);
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-
-    double2 a_cur[BM_KC / 4], a_nxt[BM_KC / 4];
-    load_a(0, a_cur);
-    stage_x(0, 0);
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncthreads();
-    for (uint64_t c = 0; c < nchunks; ++c) {
-        const int buf = (int)(c & 1);
-        if (c + 1 < nchunks) {
-            load_a(c + 1, a_nxt);
-            stage_x(c + 1, buf ^ 1);
-        }
-#pragma unroll
-        for (int i = 0; i < BM_KC / 4; ++i) {
-            const double are = a_cur[i].x, aim = a_cur[i].y, naim = -aim;
-            const cplx* xb = &Xs[buf][(4 * i + kq) * XLD + g];
-#pragma unroll
-            for (int t = 0; t < NT; ++t) {
-                const cplx b = xb[t * 8];
-                dmma884(acc_re[t][0], acc_re[t][1], are, b.re);
-                dmma884(acc_re[t][0], acc_re[t][1], naim, b.im);
-                dmma884(acc_im[t][0], acc_im[t][1], are, b.im);
-                dmma884(acc_im[t][0], acc_im[t][1], aim, b.re);
-            }
-        }
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        __syncthreads();
-#pragma unroll
-        for (int i = 0; i < BM_KC / 4; ++i) a_cur[i] = a_nxt[i];
-    }
-    if (r_out < nrows) {
-        cplx* yrow = Y + r_out * S;
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-            // D fragment: row g, columns 2*kq, 2*kq+1 of n-tile t
-            double4 v = make_double4(acc_re[t][0], acc_im[t][0], acc_re[t][1], acc_im[t][1]);
-            *reinterpret_cast<double4*>(yrow + t * 8 + 2 * kq) = v;
-        }
-    }
-}
-
 // ---- batched (one cluster per right-hand side) MGS step; same algebra as
 // mgs_cluster_reg_kernel.  RHS index = blockIdx.y.  w is read from the block-matvec output
 // Yblk[k][S]; v_{j+1} is written both to the RHS's own contiguous Krylov basis and to the
@@ -1364,23 +1261,12 @@ cudaError_t launch_cluster(Kern kern, int cluster, int threads, size_t smem, cud
 static cudaError_t launch_zgemv_impl(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* x, cplx* y,
                                      const PeerOut* po, cudaStream_t s) {
     if (nrows == 0 && !po) return cudaSuccess;
-    static const int variant = []() { const char* v = std::getenv("BEMB200_GEMV_VARIANT"); return v ? std::atoi(v) : 24; }();
-    const int rb = variant / 10, u = variant % 10;
-    uint64_t blocks = (nrows + rb - 1) / rb;
+    uint64_t blocks = (nrows + 1) / 2;  // 2 rows per block
     const uint64_t maxb = 148ull * 8ull * 8ull;
     if (blocks > maxb) blocks = maxb;
     if (blocks == 0) blocks = 1;  // an empty slab still has to publish its epoch
-    if (po) {
-        zgemv_kernel<2, 4, true><<<(unsigned)((nrows + 1) / 2 > maxb ? maxb : (nrows + 1) / 2 ? (nrows + 1) / 2 : 1), GEMV_THREADS, 0, s>>>(
-            A, lda, nrows, ncols, x, y, *po);
-        return cudaGetLastError();
-    }
-    const PeerOut none{};
-#define GEMV_CASE(R, U) \
-    if (rb == R && u == U) { zgemv_kernel<R, U, false><<<(unsigned)blocks, GEMV_THREADS, 0, s>>>(A, lda, nrows, ncols, x, y, none); return cudaGetLastError(); }
-    GEMV_CASE(4, 2) GEMV_CASE(2, 2)
-#undef GEMV_CASE
-    zgemv_kernel<2, 4, false><<<(unsigned)blocks, GEMV_THREADS, 0, s>>>(A, lda, nrows, ncols, x, y, none);
+    if (po) zgemv_kernel<2, 4, true><<<(unsigned)blocks, GEMV_THREADS, 0, s>>>(A, lda, nrows, ncols, x, y, *po);
+    else zgemv_kernel<2, 4, false><<<(unsigned)blocks, GEMV_THREADS, 0, s>>>(A, lda, nrows, ncols, x, y, PeerOut{});
     return cudaGetLastError();
 }
 
@@ -1490,31 +1376,26 @@ static cudaError_t launch_mgs_grid(int G, const cplx* V, uint64_t ldv, const cpl
 
 size_t mgs_scratch_elems() { return (size_t)GR_MAX_CTAS * 2 * LS_MAXV + GR_MAX_CTAS; }
 
-static const int g_mgs_mode_env = []() {
-    const char* v = std::getenv("BEMB200_MGS_MODE");
-    return v ? std::atoi(v) : 3;
-}();
-static PerDeviceInt g_mgs_mode(g_mgs_mode_env);  // 3: whole-GPU cooperative low-sync kernel, 0: low-sync register kernel (16-CTA cluster) when the slice fits, 2: one-vector register kernel, 1: generic kernel only
+// 3: whole-GPU cooperative low-sync kernel; 0: the cluster kernels of launch_mgs_cluster_path, for good once this device
+// could not place the cooperative grid
+static PerDeviceInt g_mgs_mode(3);
 
-bool mgs_peer_wait_capable(uint64_t n, uint32_t restart, bool allow_grid) {
+bool mgs_peer_wait_capable(uint64_t n, uint32_t restart) {
     if (restart + 1 > (uint32_t)LS_MAXV) return false;
-    const int mode = g_mgs_mode.get();
-    if (mode != 3 && mode != 0) return false;
     if (n <= 16ull * LS_THREADS * 8ull) return true;  // cluster low-sync kernel
-    return mode == 3 && allow_grid && n <= (uint64_t)GR_MAX_CTAS * 1024ull;
+    return g_mgs_mode.get() == 3 && n <= (uint64_t)GR_MAX_CTAS * 1024ull;
 }
 
 // `strict`: the caller is one rank of a row-sharded solve.  Every rank must run the SAME Arnoldi kernel
 // (convergence decisions are not all-reduced; they agree because the arithmetic is identical), so a
 // kernel that cannot be placed on this device is an error there, never a silent per-rank fallback.
-static cudaError_t launch_mgs_cluster_path(int mode_in, const cplx* V, uint64_t ldv, cplx* w, int j, uint64_t n, cplx* hcol,
+static cudaError_t launch_mgs_cluster_path(const cplx* V, uint64_t ldv, cplx* w, int j, uint64_t n, cplx* hcol,
                                            cplx* vnext, const cplx* pinv, int direct_scale, cplx* Lmat, int ldl, cplx* hcol_host,
                                            bool* wrote_host, const PeerWait& pw, bool strict, cudaStream_t s) {
     *wrote_host = false;
     // 0: low-sync register kernel (16-CTA cluster) when the slice fits, 2: one-vector register kernel, 1: generic kernel;
     // a kernel this device cannot place demotes the mode of THIS device for good
-    static PerDeviceInt cluster_mode(-1);
-    if (cluster_mode.get() < 0) cluster_mode.set(mode_in);
+    static PerDeviceInt cluster_mode(0);
     int mode = cluster_mode.get();
     if (mode == 0 && Lmat && j + 1 <= LS_MAXV && n <= 16ull * LS_THREADS * 8ull) {
         const int cl = n >= 2048 ? 16 : (n >= 512 ? 4 : 1);
@@ -1571,17 +1452,14 @@ static cudaError_t launch_mgs_cluster_path(int mode_in, const cplx* V, uint64_t 
 }
 
 cudaError_t launch_mgs(const cplx* V, uint64_t ldv, cplx* w, int j, uint64_t n, cplx* hcol, cplx* vnext, const cplx* pinv,
-                       int direct_scale, cplx* Lmat, int ldl, cplx* scratch, cplx* hcol_host, bool* wrote_host, bool allow_grid,
+                       int direct_scale, cplx* Lmat, int ldl, cplx* scratch, cplx* hcol_host, bool* wrote_host,
                        const PeerWait& pw, bool strict, cudaStream_t s) {
     *wrote_host = false;
-    // mode 3 (default): whole-GPU cooperative kernel; the slice per CTA depends on n only
-    // The whole-GPU cooperative kernel also beside a background assembly (BEMB200_MGS_FORCE_GRID=0 restores the 16-CTA cluster
-    // kernel there): with the counter-driven far kernel at two persistent blocks per SM it measured 100.4 against 104.3 ms per
-    // frequency for cluster kernel + one block per SM on the same box (profiles/r02r_*.json); the cluster kernel cannot be
-    // placed while two far blocks sit on every SM, the cooperative grid (one small CTA per SM) can.
-    static const bool force_grid = []() { const char* v = std::getenv("BEMB200_MGS_FORCE_GRID"); return v ? std::atoi(v) != 0 : true; }();
-    const int mode = g_mgs_mode.get();
-    if (mode == 3 && (allow_grid || force_grid) && Lmat && scratch && j + 1 <= LS_MAXV && n >= 4096 && n <= (uint64_t)GR_MAX_CTAS * 1024ull) {
+    // mode 3: whole-GPU cooperative kernel; the slice per CTA depends on n only.
+    // It runs beside a background assembly too: with the counter-driven far kernel at two persistent blocks per SM it measured
+    // 100.4 against 104.3 ms per frequency for cluster kernel + one block per SM on the same box (profiles/r02r_*.json); the
+    // cluster kernel cannot be placed while two far blocks sit on every SM, the cooperative grid (one small CTA per SM) can.
+    if (g_mgs_mode.get() == 3 && Lmat && scratch && j + 1 <= LS_MAXV && n >= 4096 && n <= (uint64_t)GR_MAX_CTAS * 1024ull) {
         const int G = GR_MAX_CTAS;  // fixed (not the SM count of the device): the summation order must not depend on the rank's GPU
         const uint64_t S = (n + G - 1) / G;
         cudaError_t e;
@@ -1596,10 +1474,8 @@ cudaError_t launch_mgs(const cplx* V, uint64_t ldv, cplx* w, int j, uint64_t n, 
         cudaGetLastError();  // cooperative launch not placeable on this device: cluster kernels from now on
         g_mgs_mode.set(0);
     }
-    // small or very long vectors, or BEMB200_MGS_MODE in {0,1,2}: the cluster kernels
-    const int m2 = g_mgs_mode.get();
-    return launch_mgs_cluster_path(m2 == 3 ? 0 : m2, V, ldv, w, j, n, hcol, vnext, pinv, direct_scale, Lmat, ldl,
-                                   hcol_host, wrote_host, pw, strict, s);
+    // small or very long vectors, or a device that cannot place the cooperative grid: the cluster kernels
+    return launch_mgs_cluster_path(V, ldv, w, j, n, hcol, vnext, pinv, direct_scale, Lmat, ldl, hcol_host, wrote_host, pw, strict, s);
 }
 
 cudaError_t launch_residual(const cplx* b, const cplx* ax, cplx* r, uint64_t n, double* out, const cplx* pinv, cudaStream_t s) {
@@ -1657,22 +1533,6 @@ cudaError_t launch_cgs_update(cplx* x, const cplx* uq, const cplx* w, cplx* r, c
 }
 cudaError_t launch_cgs_p(const cplx* r, const cplx* q, cplx beta, cplx* u, cplx* p, uint64_t n, cudaStream_t s) {
     cgs_p_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(r, q, beta, u, p, n);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_zgemm_block(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* X, cplx* Y, int nrhs,
-                               cudaStream_t s) {
-    if (nrows == 0) return cudaSuccess;
-    static const bool use_dmma = []() { const char* v = std::getenv("BEMB200_BLOCK_MATVEC"); return v && std::string(v) == "legacy"; }();
-    if (!use_dmma) return launch_zgemm_block_streamk(A, lda, nrows, ncols, X, Y, nrhs, s);
-    const unsigned blocks = (unsigned)((nrows + BM_ROWS - 1) / BM_ROWS);
-    switch (nrhs) {
-        case 8: zgemm_block_kernel<1><<<blocks, BM_WARPS * 32, 0, s>>>(A, lda, nrows, ncols, X, Y); break;
-        case 16: zgemm_block_kernel<2><<<blocks, BM_WARPS * 32, 0, s>>>(A, lda, nrows, ncols, X, Y); break;
-        case 24: zgemm_block_kernel<3><<<blocks, BM_WARPS * 32, 0, s>>>(A, lda, nrows, ncols, X, Y); break;
-        case 32: zgemm_block_kernel<4><<<blocks, BM_WARPS * 32, 0, s>>>(A, lda, nrows, ncols, X, Y); break;
-        default: return cudaErrorInvalidValue;
-    }
     return cudaGetLastError();
 }
 

@@ -21,12 +21,12 @@ struct PeerWait {
 };
 cudaError_t launch_zgemv_peer(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* x, const PeerOut& po,
                               cudaStream_t s);
-bool mgs_peer_wait_capable(uint64_t n, uint32_t restart, bool allow_grid);
+bool mgs_peer_wait_capable(uint64_t n, uint32_t restart);
 cudaError_t launch_zgemv(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* x, cplx* y, cudaStream_t s);
 cudaError_t launch_zgemv_t(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* x, cplx* y, cudaStream_t s);
 // Lmat (may be NULL): (ldl x ldl) scratch for the Gram triangle of the current restart cycle (low-sync kernel)
 cudaError_t launch_mgs(const cplx* V, uint64_t ldv, cplx* w, int j, uint64_t n, cplx* hcol, cplx* vnext, const cplx* pinv,
-                       int direct_scale, cplx* Lmat, int ldl, cplx* scratch, cplx* hcol_host, bool* wrote_host, bool allow_grid,
+                       int direct_scale, cplx* Lmat, int ldl, cplx* scratch, cplx* hcol_host, bool* wrote_host,
                        const PeerWait& pw, bool strict, cudaStream_t s);  // strict: one rank of a row-sharded solve, no per-rank kernel fallback  // hcol_host: mapped pinned copy of the column (written by the kernel when *wrote_host)
 size_t mgs_scratch_elems();  // cplx elements of scratch launch_mgs needs after the ldl*ldl Gram triangle
 cudaError_t launch_residual(const cplx* b, const cplx* ax, cplx* r, uint64_t n, double* out, const cplx* pinv, cudaStream_t s);
@@ -43,12 +43,10 @@ cudaError_t launch_cgs_q(const cplx* u, const cplx* v, cplx alpha, cplx* q, cplx
 cudaError_t launch_cgs_update(cplx* x, const cplx* uq, const cplx* w, cplx* r, const cplx* r0, cplx alpha, uint64_t n, cplx* out,
                               cudaStream_t s);
 cudaError_t launch_cgs_p(const cplx* r, const cplx* q, cplx beta, cplx* u, cplx* p, uint64_t n, cudaStream_t s);
+// block_matvec.cu: Y = A X for nrhs = 8, 16, 24 or 32 right-hand sides (X interleaved [k][S], Y interleaved [row][S]);
+// DMMA.8x8x4 kernel with shared-memory staging and a stream-K decomposition
 cudaError_t launch_zgemm_block(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* X, cplx* Y, int nrhs,
                                cudaStream_t s);
-// block_matvec.cu: DMMA.8x8x4 kernel with shared-memory staging and a stream-K decomposition (the default behind
-// launch_zgemm_block; BEMB200_BLOCK_MATVEC=legacy selects the round-1 kernel of linalg.cu)
-cudaError_t launch_zgemm_block_streamk(const cplx* A, uint64_t lda, uint64_t nrows, uint64_t ncols, const cplx* X, cplx* Y, int nrhs,
-                                       cudaStream_t s);
 cudaError_t launch_mgs_batched(int nrhs, const cplx* Vall, uint64_t ldv, uint64_t vstride, const cplx* Yblk, int j, uint64_t n,
                                cplx* hcol_all, uint64_t hstride, cplx* Xblk, const unsigned char* active, cudaStream_t s);
 cudaError_t launch_block_residual(const cplx* B, const cplx* AX, cplx* R, uint64_t n, int nrhs, double* out, cudaStream_t s);
