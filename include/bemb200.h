@@ -343,6 +343,17 @@ int bemb200_compute_rcs_batch(const bemb200_staged_mesh* sm, const bemb200_physi
 int bemb200_scattered_field_batch(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
                                   const double* surface_pressure, const double* surface_velocity, int on_device,
                                   uint64_t n_eval, const double* eval_pts, double* out);
+/* Complex far-field amplitude F(d) of nsol (1..4096) surface solutions in n_dirs (>= 1) unit directions dirs[3*n_dirs]
+ * (finite, | |d| - 1 | <= 1e-9), defined by p_scat(R d) = F(d) exp(i s k R) / R + O(1/R^2) with s = harmonic_factor:
+ *   F(d) = 1/(4 pi) sum_j [-i s k (d.n_j) p_j - v_j] int_{E_j} exp(-i s k d.y) dS_y
+ * from the representation of bemb200_scattered_field (v = dp/dn), over the whole element: Tri3 with the field kernel's
+ * 7-point rule, Quad4 with 3 x 3 Gauss-Legendre on the bilinear map (its Jacobian, and its normal at each point).
+ * surface_pressure / surface_velocity (may be NULL: v = 0): [nsol * num_dofs] complex128 in DOF order, host (on_device = 0)
+ * or device memory of the staged mesh's device (on_device = 1).  out [nsol * n_dirs] complex128 (host), solution-major.
+ * Row s has the bits of the nsol = 1 call on solution s, for host and device input alike.  Bad arguments return
+ * BEMB200_EINVAL before the staged mesh or a device is touched. */
+int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                      const double* surface_velocity, int on_device, uint32_t n_dirs, const double* dirs, double* out);
 
 /* ---- room-acoustics dense path (SURVEY 8f rank 3): math-bem/src/room_acoustics/solver.rs -------
  * Point collocation on a RoomMesh (math-xem-common/src/types.rs:185-192): nodes [n_nodes*3],

@@ -815,6 +815,23 @@ inline std::vector<double> compute_rcs(const StagedMesh& mesh, const std::vector
           mesh.context().handle());
     return out;
 }
+// Complex far-field amplitude F(d) with the surface-velocity term (bemb200_far_field) for n x 3 unit directions;
+// surface_velocity (v = dp/dn) may be empty (rigid).  p_scat(R d) = F(d) exp(i s k R) / R + O(1/R^2).
+inline std::vector<Complex64> compute_far_field(const StagedMesh& mesh, const std::vector<Complex64>& surface_pressure,
+                                                const std::vector<Complex64>& surface_velocity, const std::vector<double>& directions,
+                                                const PhysicsParams& physics) {
+    if (directions.empty() || directions.size() % 3 != 0) throw std::invalid_argument("compute_far_field: directions must be n x 3, n >= 1");
+    if (surface_pressure.size() != mesh.num_dofs() || (!surface_velocity.empty() && surface_velocity.size() != mesh.num_dofs()))
+        throw std::invalid_argument("compute_far_field: surface vectors must have num_dofs entries");
+    const bemb200_physics phys = physics_abi(physics);
+    std::vector<Complex64> out(directions.size() / 3);
+    const std::vector<Complex64> ps = mesh.in_dof_order(surface_pressure), vs = mesh.in_dof_order(surface_velocity);
+    check(bemb200_far_field(mesh.handle(), &phys, 1, reinterpret_cast<const double*>(ps.data()),
+                            vs.empty() ? nullptr : reinterpret_cast<const double*>(vs.data()), 0, static_cast<uint32_t>(out.size()),
+                            directions.data(), reinterpret_cast<double*>(out.data())),
+          mesh.context().handle());
+    return out;
+}
 
 struct LuError : std::runtime_error {  // lu.rs:15-21
     enum Kind { SingularMatrix, DimensionMismatch } kind;

@@ -738,6 +738,39 @@ def compute_rcs(surface_pressure: np.ndarray, staged: StagedMesh, direction, phy
     return float(out[0]) if single else out
 
 
+def compute_far_field(directions, staged: StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                      nsol: Optional[int] = None) -> np.ndarray:
+    """Complex far-field amplitude F in the (M, 3) unit ``directions`` (DESIGN.md 4.9): p_scat(R d) = F(d) exp(i s k R) / R +
+    O(1/R^2), s = harmonic_factor, from the representation ``compute_scattered_field`` evaluates, with the surface-velocity
+    term and over the whole element (Quad4: its bilinear map).  ``surface_velocity`` is v = dp/dn (None: rigid, v = 0).
+
+    Surface values as ``compute_scattered_field`` takes them: a 1-D ``surface_pressure`` (num_dofs,) returns (M,) complex; an
+    (nsol, num_dofs) array, or a device pointer (int) to nsol DOF-ordered vectors with ``nsol``, returns (nsol, M), row s
+    with the bits of the single call on solution s.  ``surface_velocity`` is given the same way, or None."""
+    single = not isinstance(surface_pressure, (int, np.integer)) and np.ndim(surface_pressure) == 1
+    if single:
+        surface_pressure = np.reshape(surface_pressure, (1, -1))
+        if surface_velocity is not None:
+            if isinstance(surface_velocity, (int, np.integer)) or np.ndim(surface_velocity) != 1:
+                raise ValueError("a 1-D surface_pressure needs a 1-D surface_velocity (or None)")
+            surface_velocity = np.reshape(surface_velocity, (1, -1))
+    ps, nsol, on_dev = _solutions_arg(surface_pressure, staged, nsol, "surface_pressure")
+    vs, _, v_dev = _solutions_arg(surface_velocity, staged, nsol, "surface_velocity", allow_none=True)
+    if vs is not None and v_dev != on_dev:
+        raise ValueError("surface_pressure and surface_velocity must both be host arrays or both device pointers")
+    d = np.ascontiguousarray(directions, dtype=np.float64)
+    if d.ndim != 2 or d.shape[1] != 3 or d.shape[0] == 0:
+        raise ValueError("directions must be an (M, 3) array with M >= 1")
+    if not np.all(np.isfinite(d)) or np.any(np.abs(np.sqrt((d * d).sum(axis=1)) - 1.0) > 1e-9):
+        raise ValueError("directions must be finite unit vectors (| |d| - 1 | <= 1e-9)")
+    out = np.empty((nsol, d.shape[0]), dtype=np.complex128)
+    ph = _cphys(physics)
+    vptr = None if vs is None else (vs if on_dev else _capi.ptr(vs))
+    _capi.check(_capi.lib().bemb200_far_field(staged._h, C.byref(ph), nsol, ps if on_dev else _capi.ptr(ps), vptr, 1 if on_dev else 0,
+                                              d.shape[0], _capi.ptr(d), _capi.ptr(out)), staged.ctx._h)
+    return out[0] if single else out
+
+
 class IdentityPreconditioner:
     """traits.rs:377-385."""
 

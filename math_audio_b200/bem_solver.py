@@ -22,7 +22,7 @@ import numpy as np
 
 from . import bem
 from .incident import IncidentField
-from .postprocess import FieldPoint, compute_total_field
+from .postprocess import FieldPoint, compute_far_field, compute_total_field, surface_power
 from .mesh import BC_PRESSURE, BC_VELOCITY, Mesh, generate_icosphere_mesh, generate_sphere_mesh
 from .types import PhysicsParams
 
@@ -57,6 +57,7 @@ class BemProblem:
     bc_type: BoundaryConditionType = BoundaryConditionType.Rigid
     use_burton_miller: bool = True
     admittance: Optional[np.ndarray] = None  # Y per element (or one for all), see with_admittance
+    surface_velocity: Optional[np.ndarray] = None  # prescribed dp/dn per element (or one for all), see with_surface_velocity
 
     @staticmethod
     def rigid_sphere_scattering(radius: float, frequency: float, speed_of_sound: float, density: float) -> "BemProblem":
@@ -89,6 +90,15 @@ class BemProblem:
         self.admittance = admittance
         return self
 
+    def with_surface_velocity(self, v_bar) -> "BemProblem":
+        """A prescribed surface velocity v_bar = dp/dn (outward normal, as ``Velocity`` values), one complex value for all
+        elements or one per element in enumeration order, constant over each element.  With ``with_admittance`` the surface
+        satisfies v = v_bar + Y p.  With an empty ``IncidentField()`` this poses a radiation problem.  Above ka = 0.5 pair it
+        with ``BemSolver.with_sign_consistent_formulation(True)``: the reference's formulation does not converge to the
+        physical solution there (DESIGN.md 4.8)."""
+        self.surface_velocity = v_bar
+        return self
+
     def with_burton_miller(self, use_bm: bool) -> "BemProblem":
         self.use_burton_miller = use_bm
         return self
@@ -108,14 +118,40 @@ class BemSolution:
     physics: PhysicsParams
     staged: Optional[bem.StagedMesh] = field(default=None, repr=False)
     admittance: Optional[np.ndarray] = None  # the problem's admittance: the surface velocity is Y p
+    v_bar: Optional[np.ndarray] = None       # the problem's prescribed surface velocity
 
-    def evaluate_pressure_field(self, points) -> List[FieldPoint]:
-        """compute_total_field (pressure.rs:273-309): incident + scattered (device field kernel).  With an admittance the
-        scattered field takes the surface velocity v = Y p."""
+    @property
+    def surface_velocity(self) -> np.ndarray:
+        """v = dp/dn = v_bar + Y p on the boundary elements (enumeration order); zero for a rigid body."""
+        n = len(self.surface_pressure)
+        v_bar = None if self.v_bar is None else np.broadcast_to(np.asarray(self.v_bar, dtype=np.complex128), (n,))
+        if self.admittance is None:
+            return np.zeros(n, dtype=np.complex128) if v_bar is None else np.array(v_bar)
+        return bem.surface_velocity(self.mesh, self.admittance, self.surface_pressure, v_bar)
+
+    def _velocity_or_none(self) -> Optional[np.ndarray]:
+        return None if self.admittance is None and self.v_bar is None else self.surface_velocity
+
+    def _staged(self) -> bem.StagedMesh:
         if self.staged is None:
             self.staged = bem.StagedMesh(self.mesh)
-        v = None if self.admittance is None else bem.surface_velocity(self.mesh, self.admittance, self.surface_pressure)
-        return compute_total_field(points, self.staged, self.surface_pressure, v, self.incident_field, self.physics)
+        return self.staged
+
+    def evaluate_pressure_field(self, points) -> List[FieldPoint]:
+        """compute_total_field (pressure.rs:273-309): incident + scattered (device field kernel).  With an admittance or a
+        prescribed velocity the scattered field takes the surface velocity v = v_bar + Y p."""
+        return compute_total_field(points, self._staged(), self.surface_pressure, self._velocity_or_none(), self.incident_field,
+                                   self.physics)
+
+    def far_field(self, directions) -> np.ndarray:
+        """Complex far-field amplitude F of the scattered / radiated field in the (M, 3) unit ``directions``:
+        p_scat(R d) = F(d) exp(i s k R) / R + O(1/R^2) (device; DESIGN.md 4.9)."""
+        return compute_far_field(directions, self._staged(), self.surface_pressure, self._velocity_or_none(), self.physics)
+
+    def radiated_power(self) -> float:
+        """Power through the surface, W = -(s / (2 omega rho)) sum_j A_j Im(p_j conj(v_j)): radiated power of a source,
+        minus the absorbed power of an absorbing body (host, O(N); DESIGN.md 4.9)."""
+        return surface_power(self.mesh, self.surface_pressure, self.surface_velocity, self.physics)
 
     def evaluate_pressure(self, point) -> complex:
         return self.evaluate_pressure_field(np.asarray(point, dtype=np.float64).reshape(1, 3))[0].p_total
@@ -184,6 +220,17 @@ class BemSolver:
         else:
             mesh.bc_type[:] = BC_VELOCITY      # Velocity(vec![0]) / VelocityWithAdmittance{velocity: vec![0], ..} (tbem.rs:236-238)
         mesh.dof[:] = np.arange(n, dtype=np.uint32)  # elem.dof_addresses = vec![i]
+        if problem.surface_velocity is not None:
+            if problem.bc_type == BoundaryConditionType.Soft:
+                raise BemError("InvalidMesh: a prescribed surface velocity needs a velocity boundary condition, not Soft")
+            v = np.asarray(problem.surface_velocity, dtype=np.complex128)
+            if v.ndim > 1 or (v.ndim == 1 and v.shape != (n,)):
+                raise BemError(f"InvalidMesh: surface velocity has {v.size} entries, the mesh has {n} elements")
+            v = np.broadcast_to(v, (n,))
+            # constant over the element: one value per node (a single value would weight the first node's shape function only)
+            mesh.bc_len[:] = mesh.etype
+            for i in range(4):
+                mesh.bc_val[:, i] = np.where(i < mesh.etype, v, 0.0)
         return mesh
 
     # -- bem_solver.rs:273-317 ------------------------------------------------------------------
@@ -209,7 +256,7 @@ class BemSolver:
         x = self.solve_dense_system(system, rhs, stats)
         if self.verbose:
             print(f"Solution complete. Max surface pressure: {np.abs(x).max():.6f}")
-        return BemSolution(x, mesh, problem.incident_field, problem.physics, staged, problem.admittance)
+        return BemSolution(x, mesh, problem.incident_field, problem.physics, staged, problem.admittance, problem.surface_velocity)
 
     # -- bem_solver.rs:435-463 ------------------------------------------------------------------
     def solve_dense_system(self, system, rhs: np.ndarray, stats: Optional[dict] = None) -> np.ndarray:

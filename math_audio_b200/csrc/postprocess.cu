@@ -2,6 +2,8 @@
 //   incident_rhs_kernel      IncidentField::compute_rhs_with_beta   math-bem/src/core/incident.rs:93-342
 //   scattered_field_kernel   compute_scattered_field                 math-bem/src/core/postprocess/pressure.rs:81-259
 //   rcs_kernel               compute_rcs                             math-bem/src/core/postprocess/pressure.rs:438-478
+//   far_field_kernel         the complex far-field amplitude with the surface-velocity term (DESIGN.md section 4.9; no
+//                            reference counterpart)
 // All work on the staged (DOF-ordered) mesh so that a frequency sweep never leaves the device.
 //
 // The *_batch kernels serve several right-hand sides / solutions of one mesh (plane waves from many directions, DESIGN.md
@@ -9,6 +11,8 @@
 // field -- is evaluated once and applied to every solution of a chunk.  Per solution they repeat the single kernels'
 // expressions, thread-to-element mapping and reduction order, so row s of a batch has the bits of the single call on
 // solution s (this unit is compiled with -fmad=false: no contraction can differ between the two).
+#include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include "api_internal.h"
@@ -306,6 +310,138 @@ rcs_batch_kernel(const double* __restrict__ src, const double* __restrict__ area
     if ((int)threadIdx.x < cnt) out[(uint64_t)(s0 + threadIdx.x) * n_dirs + blockIdx.x] = 4.0 * 3.14159265358979323846 * (t.re * t.re + t.im * t.im);
 }
 
+// ---- far-field amplitude (DESIGN.md section 4.9) -------------------------------------------------------------------------
+// F(d) = 1/(4 pi) sum_j [-i w (d.n) p_j - v_j] int_{E_j} exp(-i w d.y) dS_y with w = harmonic_factor * k: the R -> infinity
+// limit of R exp(-i w R) p_scat(R d) of the field kernel's representation, over the whole element (Quad4: bilinear map,
+// 3 x 3 Gauss-Legendre; Tri3: the field kernel's 7-point rule).  The geometry-only sums a_j(d) = sum_q w_q J_q exp(-i w d.y_q)
+// and b_j(d) = sum_q w_q J_q (d.n_q) exp(-i w d.y_q) are formed once per (direction, element) for a chunk of solutions;
+// each solution then adds p_j (-i w b_j) - v_j a_j.
+constexpr int FF_DIRS = 8;   // directions per block: warp w serves direction FF_DIRS * blockIdx.x + w
+constexpr int FF_TILE = 32;  // elements per shared-memory tile: lane e of every warp serves element e of the tile
+constexpr int FF_NQ = 9;     // quadrature points per element: 7 (Tri3) or 3 x 3 (Quad4)
+
+// Quadrature point q of the element with gathered coordinates c and type et: position y, weight x Jacobian wj and weight x
+// the unnormalised normal of the map, wn = wj n (Tri3: e1 x e2 of the field kernel; Quad4: dy/dxi x dy/deta at the point).
+__device__ __forceinline__ void far_field_point(const double* c, int et, int q, double y[3], double& wj, double wn[3]) {
+    double nv[3], w;
+    if (et == 3) {
+        const double xi = d_tr7[q][0], eta = d_tr7[q][1], l0 = 1.0 - xi - eta;
+        w = d_tr7[q][2] * 0.5;
+        const double e1[3] = {c[3] - c[0], c[4] - c[1], c[5] - c[2]};
+        const double e2[3] = {c[6] - c[0], c[7] - c[1], c[8] - c[2]};
+        nv[0] = e1[1] * e2[2] - e1[2] * e2[1];
+        nv[1] = e1[2] * e2[0] - e1[0] * e2[2];
+        nv[2] = e1[0] * e2[1] - e1[1] * e2[0];
+        for (int k = 0; k < 3; ++k) y[k] = l0 * c[k] + xi * c[3 + k] + eta * c[6 + k];
+    } else {  // nodes at (xi, eta) = (-1,-1), (1,-1), (1,1), (-1,1)
+        const double xi = BEMQ_GL3_X[q / 3], eta = BEMQ_GL3_X[q % 3];
+        w = BEMQ_GL3_W[q / 3] * BEMQ_GL3_W[q % 3];
+        const double n0 = 0.25 * (1.0 - xi) * (1.0 - eta), n1 = 0.25 * (1.0 + xi) * (1.0 - eta);
+        const double n2 = 0.25 * (1.0 + xi) * (1.0 + eta), n3 = 0.25 * (1.0 - xi) * (1.0 + eta);
+        double dxi[3], deta[3];
+        for (int k = 0; k < 3; ++k) {
+            y[k] = n0 * c[k] + n1 * c[3 + k] + n2 * c[6 + k] + n3 * c[9 + k];
+            dxi[k] = 0.25 * ((1.0 - eta) * (c[3 + k] - c[k]) + (1.0 + eta) * (c[6 + k] - c[9 + k]));
+            deta[k] = 0.25 * ((1.0 - xi) * (c[9 + k] - c[k]) + (1.0 + xi) * (c[6 + k] - c[3 + k]));
+        }
+        nv[0] = dxi[1] * deta[2] - dxi[2] * deta[1];
+        nv[1] = dxi[2] * deta[0] - dxi[0] * deta[2];
+        nv[2] = dxi[0] * deta[1] - dxi[1] * deta[0];
+    }
+    wj = sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]) * w;
+    for (int k = 0; k < 3; ++k) wn[k] = nv[k] * w;
+}
+
+// Partial far field of elements [per_split * blockIdx.z, +per_split) for solutions [SOL_CHUNK * blockIdx.y, +SOL_CHUNK) and
+// directions [FF_DIRS * blockIdx.x, +FF_DIRS): part[z][s][d], without the 1/(4 pi).  The block stages the quadrature points of a
+// tile of FF_TILE elements and the chunk's surface values in shared memory; lane e of warp w forms a_j, b_j of (direction w,
+// element e).  The lane sums are reduced by a fixed butterfly, so a solution's bits depend neither on nsol nor on its chunk.
+__global__ void __launch_bounds__(256)
+far_field_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, uint32_t n, uint32_t per_split,
+                 const double* __restrict__ dirs, uint32_t n_dirs, uint32_t nsol, const cplx* __restrict__ ps,
+                 const cplx* __restrict__ vs, double wavruim, cplx* __restrict__ part) {
+    __shared__ double sy[3][FF_NQ * FF_TILE], swj[FF_NQ * FF_TILE], swn[3][FF_NQ * FF_TILE];
+    __shared__ cplx sp[SOL_CHUNK][FF_TILE], sv[SOL_CHUNK][FF_TILE];
+    __shared__ int snq[FF_TILE];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t dir = blockIdx.x * FF_DIRS + warp;
+    const bool dir_ok = dir < n_dirs;
+    const double d0 = dir_ok ? dirs[3ull * dir] : 0.0, d1 = dir_ok ? dirs[3ull * dir + 1] : 0.0, d2 = dir_ok ? dirs[3ull * dir + 2] : 0.0;
+    const uint32_t s0 = blockIdx.y * SOL_CHUNK;
+    const int cnt = (int)min((uint32_t)SOL_CHUNK, nsol - s0);
+    const uint32_t j_begin = blockIdx.z * per_split, j_end = min(n, j_begin + per_split);
+    cplx acc[SOL_CHUNK];
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) acc[c] = C(0, 0);
+    for (uint32_t t0 = j_begin; t0 < j_end; t0 += FF_TILE) {
+        for (int i = threadIdx.x; i < FF_NQ * FF_TILE; i += blockDim.x) {
+            const int q = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            double y[3] = {0.0, 0.0, 0.0}, wj = 0.0, wn[3] = {0.0, 0.0, 0.0};
+            const int et = j < j_end ? etype[j] : 3;
+            if (j < j_end && (et == 4 || q < 7)) far_field_point(coords + 12ull * j, et, q, y, wj, wn);
+            if (q == 0) snq[e] = et == 4 ? 9 : 7;
+            for (int k = 0; k < 3; ++k) { sy[k][i] = y[k]; swn[k][i] = wn[k]; }
+            swj[i] = wj;
+        }
+        for (int i = threadIdx.x; i < SOL_CHUNK * FF_TILE; i += blockDim.x) {
+            const int c = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            const bool ok = c < cnt && j < j_end;
+            const uint64_t at = (uint64_t)(s0 + c) * n + j;
+            sp[c][e] = ok ? ps[at] : C(0, 0);
+            sv[c][e] = (ok && vs) ? vs[at] : C(0, 0);
+        }
+        __syncthreads();
+        if (dir_ok && t0 + lane < j_end) {
+            double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+            const int nq = snq[lane];
+            for (int q = 0; q < nq; ++q) {
+                const int at = q * FF_TILE + lane;
+                double sn, cs;
+                sincos(-wavruim * (d0 * sy[0][at] + d1 * sy[1][at] + d2 * sy[2][at]), &sn, &cs);
+                const double wj = swj[at], dn = d0 * swn[0][at] + d1 * swn[1][at] + d2 * swn[2][at];
+                ar += wj * cs;
+                ai += wj * sn;
+                br += dn * cs;
+                bi += dn * sn;
+            }
+            const cplx a = C(ar, ai), mikb = C(wavruim * bi, -(wavruim * br));  // -i w b
+#pragma unroll
+            for (int c = 0; c < SOL_CHUNK; ++c) {
+                if (c < cnt) {
+                    acc[c] += sp[c][lane] * mikb;
+                    if (vs) acc[c] -= sv[c][lane] * a;
+                }
+            }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) {
+#pragma unroll
+        for (int m = 16; m >= 1; m >>= 1) {
+            acc[c].re += __shfl_xor_sync(0xffffffffu, acc[c].re, m);
+            acc[c].im += __shfl_xor_sync(0xffffffffu, acc[c].im, m);
+        }
+    }
+    if (lane == 0 && dir_ok) {
+        const uint64_t base = (uint64_t)blockIdx.z * nsol;
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c)
+            if (c < cnt) part[(base + s0 + c) * n_dirs + dir] = acc[c];
+    }
+}
+
+// out[s][d] = (sum over the element splits z in order of part[z][s][d]) / (4 pi)
+__global__ void far_field_reduce_kernel(const cplx* __restrict__ part, uint32_t nsplit, uint64_t total, cplx* __restrict__ out) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    cplx t = part[i];
+    for (uint32_t z = 1; z < nsplit; ++z) t += part[z * total + i];
+    out[i] = t / (4.0 * PI);
+}
+
 // b[s] = sys + inc[s] for the nrhs columns of a block (in place: out may be inc), the one IEEE add of bemb200_sweep_next
 __global__ void add_system_rhs_kernel(const cplx* __restrict__ sys, const cplx* inc, uint64_t n, uint64_t total, cplx* out) {
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x)
@@ -584,5 +720,61 @@ extern "C" int bemb200_scattered_field_batch(const bemb200_staged_mesh* sm, cons
     if (tmp_p) cudaFreeAsync(tmp_p, s);
     if (tmp_v) cudaFreeAsync(tmp_v, s);
     if (e != cudaSuccess) return cuda_fail(ctx, e, "scattered_field_batch");
+    return BEMB200_OK;
+}
+
+extern "C" int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                                 const double* surface_velocity, int on_device, uint32_t n_dirs, const double* dirs, double* out) {
+    // every argument is checked before a device is touched (the staged mesh last, so each check answers for itself)
+    bemb200_ctx* ctx = sm ? sm->ctx : nullptr;
+    if (!phys || !surface_pressure || !dirs || !out) return set_error(ctx, BEMB200_EINVAL, "NULL argument");
+    if (nsol == 0 || nsol > 4096) return set_error(ctx, BEMB200_EINVAL, "need 1..4096 solutions");
+    if (on_device != 0 && on_device != 1) return set_error(ctx, BEMB200_EINVAL, "on_device must be 0 (host arrays) or 1 (device arrays)");
+    if (n_dirs == 0 || n_dirs > 0x7fffffffu) return set_error(ctx, BEMB200_EINVAL, "need 1..2^31-1 directions");
+    for (uint32_t d = 0; d < n_dirs; ++d) {
+        const double x = dirs[3ull * d], y = dirs[3ull * d + 1], z = dirs[3ull * d + 2];
+        const double len = std::sqrt(x * x + y * y + z * z);
+        if (!std::isfinite(x) || !std::isfinite(y) || !std::isfinite(z) || !(std::fabs(len - 1.0) <= 1e-9))
+            return set_error(ctx, BEMB200_EINVAL, "direction " + std::to_string(d) + " is not a finite unit vector (|d| - 1 within 1e-9)");
+    }
+    if (!sm) return set_error(nullptr, BEMB200_EINVAL, "NULL staged mesh");
+    if (on_device && (!device_ptr_on(ctx->device, surface_pressure) || (surface_velocity && !device_ptr_on(ctx->device, surface_velocity))))
+        return set_error(ctx, BEMB200_EINVAL, "surface values are not device memory of the staged mesh's device");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const uint32_t n = sm->dm.n;
+    // Split the elements (at most 32 ways) so that about 1184 blocks (four waves of two 256-thread blocks per SM of a B200)
+    // serve one chunk of solutions when there are few directions.  The split depends on n_dirs and n only, so a solution's bits do not depend on nsol.
+    const uint32_t dir_blocks = (n_dirs + FF_DIRS - 1) / FF_DIRS, tiles = (n + FF_TILE - 1) / FF_TILE;
+    uint32_t nsplit = (1184u + dir_blocks - 1) / dir_blocks;
+    nsplit = std::max(1u, std::min({nsplit, 32u, tiles}));
+    const uint32_t per_split = (tiles + nsplit - 1) / nsplit * FF_TILE;
+    nsplit = (n + per_split - 1) / per_split;
+    const size_t nout = (size_t)nsol * n_dirs;
+    double* ddirs = nullptr;
+    cplx *part = nullptr, *dout = nullptr, *tmp_p = nullptr, *tmp_v = nullptr;
+    const cplx *dps = nullptr, *dvs = nullptr;
+    cudaStream_t s = ctx->stream;
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&ddirs, (size_t)n_dirs * 3 * sizeof(double), s));
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&part, nout * nsplit * sizeof(cplx), s));
+    BEMB_CUDA(ctx, cudaMallocAsync((void**)&dout, nout * sizeof(cplx), s));
+    cudaError_t e = solutions_on_device(surface_pressure, on_device, (size_t)nsol * n, s, &tmp_p, &dps);
+    if (e == cudaSuccess && surface_velocity) e = solutions_on_device(surface_velocity, on_device, (size_t)nsol * n, s, &tmp_v, &dvs);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ddirs, dirs, (size_t)n_dirs * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) {
+        far_field_kernel<<<dim3(dir_blocks, (nsol + SOL_CHUNK - 1) / SOL_CHUNK, nsplit), 256, 0, s>>>(
+            sm->dm.coords, sm->dm.etype, n, per_split, ddirs, n_dirs, nsol, dps, dvs, phys->wave_number * phys->harmonic_factor, part);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) {
+        far_field_reduce_kernel<<<(unsigned)((nout + 255) / 256), 256, 0, s>>>(part, nsplit, nout, dout);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaFreeAsync(ddirs, s); cudaFreeAsync(part, s); cudaFreeAsync(dout, s);
+    if (tmp_p) cudaFreeAsync(tmp_p, s);
+    if (tmp_v) cudaFreeAsync(tmp_v, s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "far_field");
     return BEMB200_OK;
 }

@@ -1,7 +1,11 @@
 """Host-side mirror of ``math-bem/src/core/postprocess/pressure.rs``: evaluation-point generators
 (:311-424), ``FieldPoint`` (:24-56), ``compute_scattered_field`` (:81-137), ``compute_total_field``
 (:273-309) and ``compute_rcs`` (:438-478).  The O(M N) sums run on the device
-(``csrc/postprocess.cu`` behind ``bemb200_scattered_field`` / ``bemb200_compute_rcs``)."""
+(``csrc/postprocess.cu`` behind ``bemb200_scattered_field`` / ``bemb200_compute_rcs``).
+
+Beyond the reference: the complex far-field amplitude with the surface-velocity term (``compute_far_field``, device) and the
+host-side quantities built on it -- ``sphere_quadrature``, ``far_field_power``, ``surface_power`` and ``directivity_index``
+(DESIGN.md 4.9)."""
 from __future__ import annotations
 
 import math
@@ -94,3 +98,57 @@ def compute_total_field(eval_points, staged: bem.StagedMesh, surface_pressure, s
 def compute_rcs(surface_pressure, staged: bem.StagedMesh, direction, physics: PhysicsParams):
     """pressure.rs:438-478 (device)."""
     return bem.compute_rcs(surface_pressure, staged, direction, physics)
+
+
+def compute_far_field(directions, staged: bem.StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                      nsol: Optional[int] = None) -> np.ndarray:
+    """Complex far-field amplitude F, p_scat(R d) = F(d) exp(i s k R) / R + O(1/R^2) (device; ``bem.compute_far_field``)."""
+    return bem.compute_far_field(directions, staged, surface_pressure, surface_velocity, physics, nsol)
+
+
+def sphere_quadrature(n_theta: int, n_phi: int):
+    """(directions (n_theta * n_phi, 3), solid-angle weights) of a product rule on the unit sphere: Gauss-Legendre in
+    cos(theta), uniform in phi (phi_j = 2 pi j / n_phi).  The weights sum to 4 pi; spherical harmonics of degree
+    < min(2 n_theta, n_phi) are integrated exactly."""
+    if int(n_theta) < 1 or int(n_phi) < 1:
+        raise ValueError("n_theta and n_phi must be >= 1")
+    x, w = np.polynomial.legendre.leggauss(int(n_theta))
+    phi = 2.0 * math.pi * np.arange(int(n_phi)) / int(n_phi)
+    st = np.sqrt(1.0 - x * x)
+    dirs = np.stack([np.outer(st, np.cos(phi)), np.outer(st, np.sin(phi)), np.outer(x, np.ones_like(phi))], axis=-1).reshape(-1, 3)
+    return dirs, np.repeat(w * (2.0 * math.pi / int(n_phi)), int(n_phi))
+
+
+def far_field_power(F, weights, physics: PhysicsParams):
+    """Radiated (or scattered) power W = 1/(2 rho c) sum_q w_q |F(d_q)|^2 of far-field amplitudes F ((M,) or (nsol, M)) over
+    a sphere quadrature; a float, or one per solution."""
+    F = np.asarray(F)
+    w = np.asarray(weights, dtype=np.float64)
+    if F.shape[-1] != w.shape[0] or w.ndim != 1:
+        raise ValueError("F must have one entry per quadrature weight (last axis)")
+    out = (np.abs(F) ** 2) @ w / (2.0 * physics.density * physics.speed_of_sound)
+    return float(out) if np.ndim(out) == 0 else out
+
+
+def surface_power(mesh, p, v, physics: PhysicsParams) -> float:
+    """Power through the surface W = -(s / (2 omega rho)) sum_j A_j Im(p_j conj(v_j)) (s = harmonic_factor, v = dp/dn on
+    the outward normal, A_j = Element.area), for surface vectors in enumeration order (entry j <-> the j-th non-evaluation
+    element).  Positive when the surface radiates, negative when it absorbs."""
+    rows = np.asarray(mesh.is_eval) == 0
+    area = np.asarray(mesh.area, dtype=np.float64)[rows]
+    p = np.asarray(p, dtype=np.complex128)
+    v = np.asarray(v, dtype=np.complex128)
+    if p.shape != area.shape or v.shape != area.shape:
+        raise ValueError("p and v must have one entry per boundary element")
+    return float(-physics.harmonic_factor / (2.0 * physics.omega * physics.density) * float(np.sum(area * np.imag(p * np.conj(v)))))
+
+
+def directivity_index(F, weights, on_axis: int) -> float:
+    """DI = 10 log10(4 pi |F(d_on_axis)|^2 / sum_q w_q |F(d_q)|^2) in dB, ``on_axis`` the index of the on-axis direction
+    among the quadrature directions of ``F`` (M,)."""
+    F = np.asarray(F)
+    w = np.asarray(weights, dtype=np.float64)
+    if F.ndim != 1 or w.shape != F.shape:
+        raise ValueError("F and weights must be (M,) arrays of the same length")
+    total = float(np.abs(F) ** 2 @ w)
+    return 10.0 * math.log10(4.0 * math.pi * abs(F[int(on_axis)]) ** 2 / total)
