@@ -354,6 +354,22 @@ int bemb200_scattered_field_batch(const bemb200_staged_mesh* sm, const bemb200_p
  * BEMB200_EINVAL before the staged mesh or a device is touched. */
 int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
                       const double* surface_velocity, int on_device, uint32_t n_dirs, const double* dirs, double* out);
+/* Accurate scattered (or radiated) pressure of nsol (1..4096) surface solutions at n_eval (1..2^31-1) points
+ * eval_pts[3*n_eval] (finite), from the representation of bemb200_scattered_field over the whole element:
+ *   p_sc(x) = sum_j p_j int_{E_j} dG/dn_y dS - v_j int_{E_j} G dS,  G = exp(i s k r) / (4 pi r),  v = dp/dn
+ * Tri3: the flat triangle; Quad4: the bilinear element (its Jacobian and its normal at each point), so far_field is the
+ * R -> infinity limit of this field on both element types.  Pairs with |x - c_j| >= 4 rho_j (c_j node mean, rho_j largest
+ * centroid-to-node distance) take the far-field rules (Tri3 7 points, Quad4 3 x 3 Gauss); nearer pairs are subdivided in the
+ * element's parameter domain until every piece is at least 3 sqrt(piece area) from x (TR13 / 4 x 4 Gauss per piece), with no
+ * cap short of depth 30.  A point within about 2^-30 element sizes of the surface (on it, in particular) gets NaN for every
+ * solution; the other points of the call are not affected.  At points where every pair is regular on a Tri3 mesh the result
+ * is bemb200_scattered_field's up to summation order.
+ * surface_pressure / surface_velocity (may be NULL: v = 0): [nsol * num_dofs] complex128 in DOF order, host (on_device = 0)
+ * or device memory of the staged mesh's device (on_device = 1).  out [nsol * n_eval] complex128 (host), solution-major.
+ * Row s has the bits of the nsol = 1 call on solution s, for host and device input alike.  Bad arguments return
+ * BEMB200_EINVAL before the staged mesh or a device is touched. */
+int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                           const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, double* out);
 
 /* ---- room-acoustics dense path (SURVEY 8f rank 3): math-bem/src/room_acoustics/solver.rs -------
  * Point collocation on a RoomMesh (math-xem-common/src/types.rs:185-192): nodes [n_nodes*3],

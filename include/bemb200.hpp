@@ -832,6 +832,23 @@ inline std::vector<Complex64> compute_far_field(const StagedMesh& mesh, const st
           mesh.context().handle());
     return out;
 }
+// Accurate scattered pressure (bemb200_evaluate_field) at n x 3 eval_points: whole elements (Quad4: the bilinear map) and
+// adaptive quadrature near the surface; surface_velocity (v = dp/dn) may be empty.  Points on the surface are NaN.
+inline std::vector<Complex64> evaluate_field(const StagedMesh& mesh, const std::vector<double>& eval_points,
+                                             const std::vector<Complex64>& surface_pressure,
+                                             const std::vector<Complex64>& surface_velocity, const PhysicsParams& physics) {
+    if (eval_points.empty() || eval_points.size() % 3 != 0) throw std::invalid_argument("evaluate_field: eval_points must be n x 3, n >= 1");
+    if (surface_pressure.size() != mesh.num_dofs() || (!surface_velocity.empty() && surface_velocity.size() != mesh.num_dofs()))
+        throw std::invalid_argument("evaluate_field: surface vectors must have num_dofs entries");
+    const bemb200_physics phys = physics_abi(physics);
+    std::vector<Complex64> out(eval_points.size() / 3);
+    const std::vector<Complex64> ps = mesh.in_dof_order(surface_pressure), vs = mesh.in_dof_order(surface_velocity);
+    check(bemb200_evaluate_field(mesh.handle(), &phys, 1, reinterpret_cast<const double*>(ps.data()),
+                                 vs.empty() ? nullptr : reinterpret_cast<const double*>(vs.data()), 0, out.size(), eval_points.data(),
+                                 reinterpret_cast<double*>(out.data())),
+          mesh.context().handle());
+    return out;
+}
 
 struct LuError : std::runtime_error {  // lu.rs:15-21
     enum Kind { SingularMatrix, DimensionMismatch } kind;

@@ -771,6 +771,40 @@ def compute_far_field(directions, staged: StagedMesh, surface_pressure, surface_
     return out[0] if single else out
 
 
+def evaluate_field(eval_points, staged: StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                   nsol: Optional[int] = None) -> np.ndarray:
+    """Accurate scattered (or radiated) pressure at the (M, 3) ``eval_points`` (DESIGN.md 4.10): the representation
+    ``compute_scattered_field`` evaluates, over the whole element (Quad4: its bilinear map), with adaptive subdivision of
+    the elements near a point, so it holds close to the surface.  ``compute_far_field`` is its R -> infinity limit.  A point
+    on the surface (within about 2^-30 element sizes of it) is NaN for every solution.
+
+    Surface values as ``compute_far_field`` takes them: a 1-D ``surface_pressure`` (num_dofs,) returns (M,) complex; an
+    (nsol, num_dofs) array, or a device pointer (int) to nsol DOF-ordered vectors with ``nsol``, returns (nsol, M), row s
+    with the bits of the single call on solution s.  ``surface_velocity`` (v = dp/dn) is given the same way, or None."""
+    single = not isinstance(surface_pressure, (int, np.integer)) and np.ndim(surface_pressure) == 1
+    if single:
+        surface_pressure = np.reshape(surface_pressure, (1, -1))
+        if surface_velocity is not None:
+            if isinstance(surface_velocity, (int, np.integer)) or np.ndim(surface_velocity) != 1:
+                raise ValueError("a 1-D surface_pressure needs a 1-D surface_velocity (or None)")
+            surface_velocity = np.reshape(surface_velocity, (1, -1))
+    ps, nsol, on_dev = _solutions_arg(surface_pressure, staged, nsol, "surface_pressure")
+    vs, _, v_dev = _solutions_arg(surface_velocity, staged, nsol, "surface_velocity", allow_none=True)
+    if vs is not None and v_dev != on_dev:
+        raise ValueError("surface_pressure and surface_velocity must both be host arrays or both device pointers")
+    pts = np.ascontiguousarray(eval_points, dtype=np.float64)
+    if pts.ndim != 2 or pts.shape[1] != 3 or not 1 <= pts.shape[0] < 2 ** 31:
+        raise ValueError("eval_points must be an (M, 3) array with 1 <= M < 2^31")
+    if not np.all(np.isfinite(pts)):
+        raise ValueError("eval_points must be finite")
+    out = np.empty((nsol, pts.shape[0]), dtype=np.complex128)
+    ph = _cphys(physics)
+    vptr = None if vs is None else (vs if on_dev else _capi.ptr(vs))
+    _capi.check(_capi.lib().bemb200_evaluate_field(staged._h, C.byref(ph), nsol, ps if on_dev else _capi.ptr(ps), vptr,
+                                                   1 if on_dev else 0, pts.shape[0], _capi.ptr(pts), _capi.ptr(out)), staged.ctx._h)
+    return out[0] if single else out
+
+
 class IdentityPreconditioner:
     """traits.rs:377-385."""
 

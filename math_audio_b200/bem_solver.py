@@ -137,11 +137,13 @@ class BemSolution:
             self.staged = bem.StagedMesh(self.mesh)
         return self.staged
 
-    def evaluate_pressure_field(self, points) -> List[FieldPoint]:
+    def evaluate_pressure_field(self, points, accurate: bool = False) -> List[FieldPoint]:
         """compute_total_field (pressure.rs:273-309): incident + scattered (device field kernel).  With an admittance or a
-        prescribed velocity the scattered field takes the surface velocity v = v_bar + Y p."""
+        prescribed velocity the scattered field takes the surface velocity v = v_bar + Y p.  ``accurate``: the scattered
+        field over whole elements with adaptive quadrature near the surface (``evaluate_field``, DESIGN.md 4.10) instead
+        of the reference's rule; points on the surface are NaN."""
         return compute_total_field(points, self._staged(), self.surface_pressure, self._velocity_or_none(), self.incident_field,
-                                   self.physics)
+                                   self.physics, accurate)
 
     def far_field(self, directions) -> np.ndarray:
         """Complex far-field amplitude F of the scattered / radiated field in the (M, 3) unit ``directions``:
@@ -153,8 +155,8 @@ class BemSolution:
         minus the absorbed power of an absorbing body (host, O(N); DESIGN.md 4.9)."""
         return surface_power(self.mesh, self.surface_pressure, self.surface_velocity, self.physics)
 
-    def evaluate_pressure(self, point) -> complex:
-        return self.evaluate_pressure_field(np.asarray(point, dtype=np.float64).reshape(1, 3))[0].p_total
+    def evaluate_pressure(self, point, accurate: bool = False) -> complex:
+        return self.evaluate_pressure_field(np.asarray(point, dtype=np.float64).reshape(1, 3), accurate)[0].p_total
 
     def max_surface_pressure(self) -> float:
         return float(np.abs(self.surface_pressure).max())

@@ -442,6 +442,356 @@ __global__ void far_field_reduce_kernel(const cplx* __restrict__ part, uint32_t 
     out[i] = t / (4.0 * PI);
 }
 
+// ---- accurate field evaluation (DESIGN.md section 4.10) ------------------------------------------------------------------
+// p_sc(x) = sum_j p_j int_{E_j} dG/dn_y - v_j int_{E_j} G over the whole element (Tri3: the flat triangle; Quad4: the bilinear
+// map with its Jacobian and normal, as far_field_point), G = exp(i w r) / (4 pi r).  A (point, element) pair is regular when
+// |x - c_e| >= FE_ETA rho_e (c_e: node mean, rho_e: largest centroid-to-node distance) and takes far_field_point's rule.  A
+// near pair is split 4 ways in the element's parameter domain until |x - y(sub-centre)| >= FE_ACCEPT sqrt(sub-area); accepted
+// pieces take TR13 (Tri3) or 4 x 4 Gauss-Legendre (Quad4).  A piece still refused at depth FE_LMAX means the point lies within
+// about 2^-FE_LMAX element sizes of the surface: that pair's integrals are NaN, and so is the point's value for every solution.
+constexpr double FE_ETA = 4.0;     // regular pair: |x - c_e|^2 >= FE_ETA^2 rho_e^2
+constexpr double FE_ACCEPT = 3.0;  // accepted piece: |x - y(sub-centre)|^2 >= FE_ACCEPT^2 sub-area
+constexpr int FE_LMAX = 30;        // subdivision depth limit (2 bits per level of the piece's path fit a uint64)
+constexpr int FE_POINTS = 8;       // evaluation points per block of the regular pass: warp w serves point FE_POINTS * blockIdx.x + w
+
+// elem[j] = (node mean, FE_ETA^2 x largest squared centroid-to-node distance) of element j
+__global__ void field_element_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, uint32_t n,
+                                     double4* __restrict__ elem) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const double* c = coords + 12ull * j;
+    const int et = etype[j];
+    double m[3];
+    for (int k = 0; k < 3; ++k) m[k] = ((et == 4 ? (c[k] + c[3 + k]) + c[6 + k] + c[9 + k] : (c[k] + c[3 + k]) + c[6 + k])) / et;
+    double rho2 = 0.0;
+    for (int v = 0; v < et; ++v) {
+        const double d0 = c[3 * v] - m[0], d1 = c[3 * v + 1] - m[1], d2 = c[3 * v + 2] - m[2];
+        rho2 = fmax(rho2, d0 * d0 + d1 * d1 + d2 * d2);
+    }
+    elem[j] = make_double4(m[0], m[1], m[2], FE_ETA * FE_ETA * rho2);
+}
+
+__device__ __forceinline__ bool field_pair_regular(double x0, double x1, double x2, double4 e) {
+    const double d0 = x0 - e.x, d1 = x1 - e.y, d2 = x2 - e.z;
+    return d0 * d0 + d1 * d1 + d2 * d2 >= e.w;
+}
+
+// counts[m] = number of near pairs of point m (one warp per point)
+__global__ void field_near_count_kernel(const double4* __restrict__ elem, uint32_t n, const double* __restrict__ eval, uint32_t n_eval,
+                                        uint32_t* __restrict__ counts) {
+    const uint32_t m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (m >= n_eval) return;
+    const double x0 = eval[3ull * m], x1 = eval[3ull * m + 1], x2 = eval[3ull * m + 2];
+    uint32_t cnt = 0;
+    for (uint32_t j = lane; j < n; j += 32) cnt += field_pair_regular(x0, x1, x2, elem[j]) ? 0u : 1u;
+    for (int o = 16; o >= 1; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if (lane == 0) counts[m] = cnt;
+}
+
+// the near pairs of point m at [off[m], off[m + 1]), elements ascending (one warp per point)
+__global__ void field_near_fill_kernel(const double4* __restrict__ elem, uint32_t n, const double* __restrict__ eval, uint32_t n_eval,
+                                       const uint64_t* __restrict__ off, uint32_t* __restrict__ pair_pt, uint32_t* __restrict__ pair_el) {
+    const uint32_t m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (m >= n_eval) return;
+    const double x0 = eval[3ull * m], x1 = eval[3ull * m + 1], x2 = eval[3ull * m + 2];
+    uint64_t at = off[m];
+    for (uint32_t t0 = 0; t0 < n; t0 += 32) {
+        const uint32_t j = t0 + lane;
+        const bool near = j < n && !field_pair_regular(x0, x1, x2, elem[j]);
+        const uint32_t mask = __ballot_sync(0xffffffffu, near);
+        if (near) {
+            const uint64_t i = at + __popc(mask & ((1u << lane) - 1u));
+            pair_pt[i] = m;
+            pair_el[i] = j;
+        }
+        at += __popc(mask);
+    }
+}
+
+// Regular pass: partial fields of elements [per_split * blockIdx.z, +per_split) for solutions [SOL_CHUNK * blockIdx.y, +SOL_CHUNK)
+// and points [FE_POINTS * blockIdx.x, +FE_POINTS): part[z][s][m].  The layout of far_field_kernel: the block stages a tile's
+// quadrature points, element data and the chunk's surface values in shared memory; lane e of warp w forms the geometry-only
+// a = sum w J G and b = sum w dG/dn_y of (point w, element e) when the pair is regular, and each solution adds p b - v a.
+__global__ void __launch_bounds__(256)
+field_regular_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, const double4* __restrict__ elem, uint32_t n,
+                     uint32_t per_split, const double* __restrict__ eval, uint32_t n_eval, uint32_t nsol, const cplx* __restrict__ ps,
+                     const cplx* __restrict__ vs, double wavruim, cplx* __restrict__ part) {
+    __shared__ double sy[3][FF_NQ * FF_TILE], swj[FF_NQ * FF_TILE], swn[3][FF_NQ * FF_TILE];
+    __shared__ double4 sel[FF_TILE];
+    __shared__ cplx sp[SOL_CHUNK][FF_TILE], sv[SOL_CHUNK][FF_TILE];
+    __shared__ int snq[FF_TILE];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t m = blockIdx.x * FE_POINTS + warp;
+    const bool pt_ok = m < n_eval;
+    const double x0 = pt_ok ? eval[3ull * m] : 0.0, x1 = pt_ok ? eval[3ull * m + 1] : 0.0, x2 = pt_ok ? eval[3ull * m + 2] : 0.0;
+    const uint32_t s0 = blockIdx.y * SOL_CHUNK;
+    const int cnt = (int)min((uint32_t)SOL_CHUNK, nsol - s0);
+    const uint32_t j_begin = blockIdx.z * per_split, j_end = min(n, j_begin + per_split);
+    cplx acc[SOL_CHUNK];
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) acc[c] = C(0, 0);
+    for (uint32_t t0 = j_begin; t0 < j_end; t0 += FF_TILE) {
+        for (int i = threadIdx.x; i < FF_NQ * FF_TILE; i += blockDim.x) {
+            const int q = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            double y[3] = {0.0, 0.0, 0.0}, wj = 0.0, wn[3] = {0.0, 0.0, 0.0};
+            const int et = j < j_end ? etype[j] : 3;
+            if (j < j_end && (et == 4 || q < 7)) far_field_point(coords + 12ull * j, et, q, y, wj, wn);
+            if (q == 0) {
+                snq[e] = et == 4 ? 9 : 7;
+                sel[e] = j < j_end ? elem[j] : make_double4(0.0, 0.0, 0.0, 0.0);
+            }
+            for (int k = 0; k < 3; ++k) { sy[k][i] = y[k]; swn[k][i] = wn[k]; }
+            swj[i] = wj;
+        }
+        for (int i = threadIdx.x; i < SOL_CHUNK * FF_TILE; i += blockDim.x) {
+            const int c = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            const bool ok = c < cnt && j < j_end;
+            const uint64_t at = (uint64_t)(s0 + c) * n + j;
+            sp[c][e] = ok ? ps[at] : C(0, 0);
+            sv[c][e] = (ok && vs) ? vs[at] : C(0, 0);
+        }
+        __syncthreads();
+        if (pt_ok && t0 + lane < j_end && field_pair_regular(x0, x1, x2, sel[lane])) {
+            double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+            const int nq = snq[lane];
+            for (int q = 0; q < nq; ++q) {
+                const int at = q * FF_TILE + lane;
+                const double rv[3] = {sy[0][at] - x0, sy[1][at] - x1, sy[2][at] - x2};
+                const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
+                double sn, cs;
+                sincos(wavruim * r, &sn, &cs);
+                const double re1 = 4.0 * PI * r;
+                const cplx zg = C(cs / re1, sn / re1);
+                const cplx zgikr = zg * C(-1.0 / r, wavruim);
+                const double wj = swj[at], dn = (rv[0] * swn[0][at] + rv[1] * swn[1][at] + rv[2] * swn[2][at]) / r;
+                ar += wj * zg.re;
+                ai += wj * zg.im;
+                br += dn * zgikr.re;
+                bi += dn * zgikr.im;
+            }
+            const cplx a = C(ar, ai), b = C(br, bi);
+#pragma unroll
+            for (int c = 0; c < SOL_CHUNK; ++c) {
+                if (c < cnt) {
+                    acc[c] += sp[c][lane] * b;
+                    if (vs) acc[c] -= sv[c][lane] * a;
+                }
+            }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int c = 0; c < SOL_CHUNK; ++c) {
+#pragma unroll
+        for (int o = 16; o >= 1; o >>= 1) {
+            acc[c].re += __shfl_xor_sync(0xffffffffu, acc[c].re, o);
+            acc[c].im += __shfl_xor_sync(0xffffffffu, acc[c].im, o);
+        }
+    }
+    if (lane == 0 && pt_ok) {
+        const uint64_t base = (uint64_t)blockIdx.z * nsol;
+#pragma unroll
+        for (int c = 0; c < SOL_CHUNK; ++c)
+            if (c < cnt) part[(base + s0 + c) * n_eval + m] = acc[c];
+    }
+}
+
+// A piece of a near pair: Tri3 -- its vertices in the parameter triangle (u[0..5], (xi, eta) per vertex); Quad4 -- its
+// sub-square [u0, u0 + u2] x [u1, u1 + u2] of [-1, 1]^2.  The piece at depth `lvl` is reached from the whole element by the
+// children path[2 (l - 1) .. 2 l) of levels l = 1..lvl: Tri3 children are the corner triangles at vertices 0, 1, 2 and the
+// centre triangle; Quad4 children the sub-squares (xi low, eta low), (high, low), (low, high), (high, high).  Every parameter
+// coordinate is a multiple of 2^-FE_LMAX, so the pieces are exact.
+struct FieldPiece {
+    double u[6];
+    int lvl;
+};
+
+__device__ __forceinline__ FieldPiece field_piece(int et, uint64_t path, int lvl) {
+    FieldPiece p;
+    p.lvl = lvl;
+    if (et == 3) {
+        double u[6] = {0.0, 0.0, 1.0, 0.0, 0.0, 1.0};
+        for (int l = 0; l < lvl; ++l) {
+            const int ch = (int)((path >> (2 * l)) & 3u);
+            const double m01[2] = {(u[0] + u[2]) / 2, (u[1] + u[3]) / 2}, m12[2] = {(u[2] + u[4]) / 2, (u[3] + u[5]) / 2},
+                         m20[2] = {(u[4] + u[0]) / 2, (u[5] + u[1]) / 2};
+            if (ch == 0) { u[2] = m01[0]; u[3] = m01[1]; u[4] = m20[0]; u[5] = m20[1]; }
+            else if (ch == 1) { u[0] = m01[0]; u[1] = m01[1]; u[4] = m12[0]; u[5] = m12[1]; }
+            else if (ch == 2) { u[0] = m20[0]; u[1] = m20[1]; u[2] = m12[0]; u[3] = m12[1]; }
+            else { u[0] = m01[0]; u[1] = m01[1]; u[2] = m12[0]; u[3] = m12[1]; u[4] = m20[0]; u[5] = m20[1]; }
+        }
+        for (int k = 0; k < 6; ++k) p.u[k] = u[k];
+    } else {
+        double xi0 = -1.0, eta0 = -1.0, h = 2.0;
+        for (int l = 0; l < lvl; ++l) {
+            const int ch = (int)((path >> (2 * l)) & 3u);
+            h *= 0.5;
+            if (ch & 1) xi0 += h;
+            if (ch & 2) eta0 += h;
+        }
+        p.u[0] = xi0; p.u[1] = eta0; p.u[2] = h;
+        p.u[3] = p.u[4] = p.u[5] = 0.0;
+    }
+    return p;
+}
+
+// position y and N = dy/dxi x dy/deta of the bilinear map at (xi, eta) (far_field_point's expressions)
+__device__ __forceinline__ void quad_map(const double* c, double xi, double eta, double y[3], double nv[3]) {
+    const double n0 = 0.25 * (1.0 - xi) * (1.0 - eta), n1 = 0.25 * (1.0 + xi) * (1.0 - eta);
+    const double n2 = 0.25 * (1.0 + xi) * (1.0 + eta), n3 = 0.25 * (1.0 - xi) * (1.0 + eta);
+    double dxi[3], deta[3];
+    for (int k = 0; k < 3; ++k) {
+        y[k] = n0 * c[k] + n1 * c[3 + k] + n2 * c[6 + k] + n3 * c[9 + k];
+        dxi[k] = 0.25 * ((1.0 - eta) * (c[3 + k] - c[k]) + (1.0 + eta) * (c[6 + k] - c[9 + k]));
+        deta[k] = 0.25 * ((1.0 - xi) * (c[9 + k] - c[k]) + (1.0 + xi) * (c[6 + k] - c[3 + k]));
+    }
+    nv[0] = dxi[1] * deta[2] - dxi[2] * deta[1];
+    nv[1] = dxi[2] * deta[0] - dxi[0] * deta[2];
+    nv[2] = dxi[0] * deta[1] - dxi[1] * deta[0];
+}
+
+// Is the piece far enough from x for its rule: |x - y(sub-centre)|^2 >= FE_ACCEPT^2 sub-area (Tri3: area / 4^lvl; Quad4: the
+// map's |N| at the sub-centre x side^2, the exact area of a sub-parallelogram)?  tri_area: the Tri3 element's area.
+__device__ __forceinline__ bool field_piece_accepted(const double* c, int et, const FieldPiece& p, double tri_area, const double x[3]) {
+    double y[3], sub_area;
+    if (et == 3) {
+        const double a = (p.u[0] + p.u[2] + p.u[4]) / 3.0, b = (p.u[1] + p.u[3] + p.u[5]) / 3.0, l0 = 1.0 - a - b;
+        for (int k = 0; k < 3; ++k) y[k] = l0 * c[k] + a * c[3 + k] + b * c[6 + k];
+        sub_area = tri_area * ldexp(1.0, -2 * p.lvl);
+    } else {
+        double nv[3];
+        quad_map(c, p.u[0] + 0.5 * p.u[2], p.u[1] + 0.5 * p.u[2], y, nv);
+        sub_area = sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]) * p.u[2] * p.u[2];
+    }
+    const double d0 = y[0] - x[0], d1 = y[1] - x[1], d2 = y[2] - x[2];
+    return d0 * d0 + d1 * d1 + d2 * d2 >= FE_ACCEPT * FE_ACCEPT * sub_area;
+}
+
+// Adds quadrature point q (TR13: q < 13; 4 x 4 Gauss: q < 16) of piece p to the lane's (int G, int dG/dn_y) sums.
+// en, jac: the Tri3 element's unit normal and |e1 x e2|.
+__device__ __forceinline__ void field_piece_point(const double* c, int et, const FieldPiece& p, int q, const double en[3], double jac,
+                                                  const double x[3], double wavruim, double& ar, double& ai, double& br, double& bi) {
+    double y[3], wj, wn[3];
+    if (et == 3) {
+        const double xi = BEMQ_TR13[q][0], eta = BEMQ_TR13[q][1];
+        const double a = p.u[0] + xi * (p.u[2] - p.u[0]) + eta * (p.u[4] - p.u[0]);
+        const double b = p.u[1] + xi * (p.u[3] - p.u[1]) + eta * (p.u[5] - p.u[1]);
+        const double l0 = 1.0 - a - b;
+        for (int k = 0; k < 3; ++k) y[k] = l0 * c[k] + a * c[3 + k] + b * c[6 + k];
+        wj = BEMQ_TR13[q][2] * 0.5 * (jac * ldexp(1.0, -2 * p.lvl));
+        for (int k = 0; k < 3; ++k) wn[k] = wj * en[k];
+    } else {
+        const double g = 0.5 * p.u[2];
+        const double w = BEMQ_GL4_W[q >> 2] * BEMQ_GL4_W[q & 3] * g * g;
+        double nv[3];
+        quad_map(c, p.u[0] + g + g * BEMQ_GL4_X[q >> 2], p.u[1] + g + g * BEMQ_GL4_X[q & 3], y, nv);
+        wj = w * sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]);
+        for (int k = 0; k < 3; ++k) wn[k] = w * nv[k];
+    }
+    const double rv[3] = {y[0] - x[0], y[1] - x[1], y[2] - x[2]};
+    const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
+    double sn, cs;
+    sincos(wavruim * r, &sn, &cs);
+    const double re1 = 4.0 * PI * r;
+    const cplx zg = C(cs / re1, sn / re1);
+    const cplx zgikr = zg * C(-1.0 / r, wavruim);
+    const double dn = (rv[0] * wn[0] + rv[1] * wn[1] + rv[2] * wn[2]) / r;
+    ar += wj * zg.re;
+    ai += wj * zg.im;
+    br += dn * zgikr.re;
+    bi += dn * zgikr.im;
+}
+
+// Near pass: one warp per near pair i walks the subdivision tree of its element depth first (children in order), every lane
+// taking the same decisions, without a stack: the current piece is (path, depth).  Accepted pieces are evaluated two at a time,
+// the earlier on lanes 0-15 and the later on lanes 16-31, one quadrature point per lane; a fixed butterfly reduces the lanes.
+// ab[i] = (int G, int dG/dn_y) of the pair, NaN when a piece reaches FE_LMAX unaccepted.
+__global__ void __launch_bounds__(256)
+field_near_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, const double* __restrict__ eval,
+                  const uint32_t* __restrict__ pair_pt, const uint32_t* __restrict__ pair_el, uint64_t npairs, double wavruim,
+                  cplx* __restrict__ ab) {
+    const uint64_t i = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (i >= npairs) return;
+    const uint32_t m = pair_pt[i], j = pair_el[i];
+    const double x[3] = {eval[3ull * m], eval[3ull * m + 1], eval[3ull * m + 2]};
+    double c[12];
+    for (int k = 0; k < 12; ++k) c[k] = coords[12ull * j + k];
+    const int et = etype[j];
+    double en[3] = {0.0, 0.0, 0.0}, jac = 0.0;
+    if (et == 3) {
+        const double e1[3] = {c[3] - c[0], c[4] - c[1], c[5] - c[2]};
+        const double e2[3] = {c[6] - c[0], c[7] - c[1], c[8] - c[2]};
+        const double nv[3] = {e1[1] * e2[2] - e1[2] * e2[1], e1[2] * e2[0] - e1[0] * e2[2], e1[0] * e2[1] - e1[1] * e2[0]};
+        jac = sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]);
+        for (int k = 0; k < 3; ++k) en[k] = nv[k] / jac;
+    }
+    const int nq = et == 3 ? 13 : 16;
+    const int half = lane >> 4, q = lane & 15;
+    double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+    bool failed = false, have_pending = false;
+    FieldPiece pending{};
+    uint64_t path = 0;
+    int lvl = 0;
+    for (;;) {
+        const FieldPiece cur = field_piece(et, path, lvl);
+        if (field_piece_accepted(c, et, cur, 0.5 * jac, x)) {
+            if (have_pending) {
+                if (q < nq) field_piece_point(c, et, half ? cur : pending, q, en, jac, x, wavruim, ar, ai, br, bi);
+                have_pending = false;
+            } else {
+                pending = cur;
+                have_pending = true;
+            }
+            // next piece: the next sibling, or that of the nearest ancestor that has one
+            while (lvl > 0 && ((path >> (2 * (lvl - 1))) & 3u) == 3u) {
+                path &= ~(3ull << (2 * (lvl - 1)));
+                --lvl;
+            }
+            if (lvl == 0) break;
+            path += 1ull << (2 * (lvl - 1));
+        } else if (lvl == FE_LMAX) {
+            failed = true;
+            break;
+        } else {
+            ++lvl;  // first child: digit 0
+        }
+    }
+    if (have_pending && !failed && half == 0 && q < nq) field_piece_point(c, et, pending, q, en, jac, x, wavruim, ar, ai, br, bi);
+    for (int o = 16; o >= 1; o >>= 1) {
+        ar += __shfl_xor_sync(0xffffffffu, ar, o);
+        ai += __shfl_xor_sync(0xffffffffu, ai, o);
+        br += __shfl_xor_sync(0xffffffffu, br, o);
+        bi += __shfl_xor_sync(0xffffffffu, bi, o);
+    }
+    if (lane == 0) {
+        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+        ab[2 * i] = failed ? C(nan, nan) : C(ar, ai);
+        ab[2 * i + 1] = failed ? C(nan, nan) : C(br, bi);
+    }
+}
+
+// out[s][m] = (sum over the element splits z in order of part[z][s][m]) + sum over the near pairs of m in list order of
+// p_j int dG/dn_y - v_j int G
+__global__ void field_combine_kernel(const cplx* __restrict__ part, uint32_t nsplit, uint32_t nsol, uint32_t n_eval, uint32_t n,
+                                     const uint64_t* __restrict__ off, const uint32_t* __restrict__ pair_el, const cplx* __restrict__ ab,
+                                     const cplx* __restrict__ ps, const cplx* __restrict__ vs, cplx* __restrict__ out) {
+    const uint64_t total = (uint64_t)nsol * n_eval;
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const uint64_t s = i / n_eval, m = i % n_eval;
+    cplx t = part[i];
+    for (uint32_t z = 1; z < nsplit; ++z) t += part[z * total + i];
+    for (uint64_t k = off[m]; k < off[m + 1]; ++k) {
+        const uint64_t at = s * n + pair_el[k];
+        t += ps[at] * ab[2 * k + 1];
+        if (vs) t -= vs[at] * ab[2 * k];
+    }
+    out[i] = t;
+}
+
 // b[s] = sys + inc[s] for the nrhs columns of a block (in place: out may be inc), the one IEEE add of bemb200_sweep_next
 __global__ void add_system_rhs_kernel(const cplx* __restrict__ sys, const cplx* inc, uint64_t n, uint64_t total, cplx* out) {
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x)
@@ -776,5 +1126,109 @@ extern "C" int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_ph
     if (tmp_p) cudaFreeAsync(tmp_p, s);
     if (tmp_v) cudaFreeAsync(tmp_v, s);
     if (e != cudaSuccess) return cuda_fail(ctx, e, "far_field");
+    return BEMB200_OK;
+}
+
+extern "C" int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                                      const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, double* out) {
+    // every argument is checked before a device is touched (the staged mesh last, so each check answers for itself)
+    bemb200_ctx* ctx = sm ? sm->ctx : nullptr;
+    if (!phys || !surface_pressure || !eval_pts || !out) return set_error(ctx, BEMB200_EINVAL, "NULL argument");
+    if (nsol == 0 || nsol > 4096) return set_error(ctx, BEMB200_EINVAL, "need 1..4096 solutions");
+    if (on_device != 0 && on_device != 1) return set_error(ctx, BEMB200_EINVAL, "on_device must be 0 (host arrays) or 1 (device arrays)");
+    if (n_eval == 0 || n_eval > 0x7fffffffull) return set_error(ctx, BEMB200_EINVAL, "need 1..2^31-1 evaluation points");
+    for (uint64_t m = 0; m < 3 * n_eval; ++m)
+        if (!std::isfinite(eval_pts[m])) return set_error(ctx, BEMB200_EINVAL, "evaluation point " + std::to_string(m / 3) + " is not finite");
+    if (!sm) return set_error(nullptr, BEMB200_EINVAL, "NULL staged mesh");
+    if (on_device && (!device_ptr_on(ctx->device, surface_pressure) || (surface_velocity && !device_ptr_on(ctx->device, surface_velocity))))
+        return set_error(ctx, BEMB200_EINVAL, "surface values are not device memory of the staged mesh's device");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const uint32_t n = sm->dm.n, ne = (uint32_t)n_eval;
+    const double wavruim = phys->wave_number * phys->harmonic_factor;
+    cudaStream_t s = ctx->stream;
+    struct Allocs {  // stream-ordered frees after the last kernel, on every return path
+        cudaStream_t s;
+        std::vector<void*> p;
+        cudaError_t get(void** out, size_t bytes) {
+            cudaError_t e = cudaMallocAsync(out, bytes ? bytes : 1, s);
+            if (e == cudaSuccess) p.push_back(*out);
+            return e;
+        }
+        ~Allocs() { for (void* q : p) cudaFreeAsync(q, s); }
+    } mem{s, {}};
+    // The regular pass splits the elements as far_field does (depending on n_eval and n only, so a solution's bits do not
+    // depend on nsol).
+    const uint32_t pt_blocks = (ne + FE_POINTS - 1) / FE_POINTS, tiles = (n + FF_TILE - 1) / FF_TILE;
+    uint32_t nsplit = (1184u + pt_blocks - 1) / pt_blocks;
+    nsplit = std::max(1u, std::min({nsplit, 32u, tiles}));
+    const uint32_t per_split = std::max(1u, (tiles + nsplit - 1) / nsplit) * FF_TILE;
+    nsplit = std::max(1u, (n + per_split - 1) / per_split);
+    const size_t nout = (size_t)nsol * ne;
+    double *dev = nullptr;
+    double4* elem = nullptr;
+    uint32_t* counts = nullptr;
+    cplx *part = nullptr, *dout = nullptr, *tmp_p = nullptr, *tmp_v = nullptr;
+    const cplx *dps = nullptr, *dvs = nullptr;
+    cudaError_t e = mem.get((void**)&dev, (size_t)ne * 3 * sizeof(double));
+    if (e == cudaSuccess) e = mem.get((void**)&elem, (size_t)n * sizeof(double4));
+    if (e == cudaSuccess) e = mem.get((void**)&counts, (size_t)ne * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dev, eval_pts, (size_t)ne * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && n) {
+        field_element_kernel<<<(n + 255) / 256, 256, 0, s>>>(sm->dm.coords, sm->dm.etype, n, elem);
+        e = cudaGetLastError();
+    }
+    const unsigned warp_blocks = (unsigned)(((uint64_t)ne * 32 + 255) / 256);
+    if (e == cudaSuccess) {
+        field_near_count_kernel<<<warp_blocks, 256, 0, s>>>(elem, n, dev, ne, counts);
+        e = cudaGetLastError();
+    }
+    // near list sized exactly: counts -> host prefix sum -> offsets
+    std::vector<uint32_t> hcount(ne);
+    std::vector<uint64_t> hoff((size_t)ne + 1, 0);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(hcount.data(), counts, (size_t)ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "evaluate_field (near count)");
+    for (uint32_t m = 0; m < ne; ++m) hoff[m + 1] = hoff[m] + hcount[m];
+    const uint64_t npairs = hoff[ne];
+    uint64_t* off = nullptr;
+    uint32_t *pair_pt = nullptr, *pair_el = nullptr;
+    cplx* ab = nullptr;
+    e = mem.get((void**)&off, hoff.size() * sizeof(uint64_t));
+    if (e == cudaSuccess) e = mem.get((void**)&pair_pt, npairs * sizeof(uint32_t));
+    if (e == cudaSuccess) e = mem.get((void**)&pair_el, npairs * sizeof(uint32_t));
+    if (e == cudaSuccess) e = mem.get((void**)&ab, 2 * npairs * sizeof(cplx));
+    if (e == cudaSuccess) e = mem.get((void**)&part, nout * nsplit * sizeof(cplx));
+    if (e == cudaSuccess) e = mem.get((void**)&dout, nout * sizeof(cplx));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(off, hoff.data(), hoff.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && npairs) {
+        field_near_fill_kernel<<<warp_blocks, 256, 0, s>>>(elem, n, dev, ne, off, pair_pt, pair_el);
+        e = cudaGetLastError();
+        if (e == cudaSuccess) {
+            field_near_kernel<<<(unsigned)((npairs * 32 + 255) / 256), 256, 0, s>>>(sm->dm.coords, sm->dm.etype, dev, pair_pt, pair_el,
+                                                                                  npairs, wavruim, ab);
+            e = cudaGetLastError();
+        }
+    }
+    if (e == cudaSuccess) {
+        e = solutions_on_device(surface_pressure, on_device, (size_t)nsol * n, s, &tmp_p, &dps);
+        if (tmp_p) mem.p.push_back(tmp_p);
+    }
+    if (e == cudaSuccess && surface_velocity) {
+        e = solutions_on_device(surface_velocity, on_device, (size_t)nsol * n, s, &tmp_v, &dvs);
+        if (tmp_v) mem.p.push_back(tmp_v);
+    }
+    if (e == cudaSuccess) {
+        field_regular_kernel<<<dim3(pt_blocks, (nsol + SOL_CHUNK - 1) / SOL_CHUNK, nsplit), 256, 0, s>>>(
+            sm->dm.coords, sm->dm.etype, elem, n, per_split, dev, ne, nsol, dps, dvs, wavruim, part);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) {
+        field_combine_kernel<<<(unsigned)((nout + 255) / 256), 256, 0, s>>>(part, nsplit, nsol, ne, n, off, pair_el, ab, dps, dvs, dout);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "evaluate_field");
     return BEMB200_OK;
 }

@@ -86,12 +86,22 @@ def compute_scattered_field(eval_points, staged: bem.StagedMesh, surface_pressur
     return bem.compute_scattered_field(eval_points, staged, surface_pressure, surface_velocity, physics)
 
 
+def evaluate_field(eval_points, staged: bem.StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                   nsol: Optional[int] = None) -> np.ndarray:
+    """Accurate scattered pressure, whole elements and adaptive near-surface quadrature (device; ``bem.evaluate_field``)."""
+    return bem.evaluate_field(eval_points, staged, surface_pressure, surface_velocity, physics, nsol)
+
+
 def compute_total_field(eval_points, staged: bem.StagedMesh, surface_pressure, surface_velocity: Optional[np.ndarray],
-                        incident_field: IncidentField, physics: PhysicsParams) -> List[FieldPoint]:
-    """pressure.rs:273-309: incident (host, O(M)) + scattered (device, O(M N))."""
+                        incident_field: IncidentField, physics: PhysicsParams, accurate: bool = False) -> List[FieldPoint]:
+    """pressure.rs:273-309: incident (host, O(M)) + scattered (device, O(M N)).  ``accurate``: the scattered part from
+    ``evaluate_field`` (whole elements, adaptive near the surface) instead of the reference's rule."""
     pts = np.ascontiguousarray(eval_points, dtype=np.float64).reshape(-1, 3)
     p_inc = incident_field.evaluate_pressure(pts, physics)
-    p_sc = bem.compute_scattered_field(pts, staged, surface_pressure, surface_velocity, physics)
+    if accurate:
+        p_sc = bem.evaluate_field(pts, staged, surface_pressure, surface_velocity, physics)
+    else:
+        p_sc = bem.compute_scattered_field(pts, staged, surface_pressure, surface_velocity, physics)
     return [FieldPoint(pts[i].copy(), complex(p_inc[i]), complex(p_sc[i])) for i in range(pts.shape[0])]
 
 
