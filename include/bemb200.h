@@ -370,6 +370,19 @@ int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys
  * BEMB200_EINVAL before the staged mesh or a device is touched. */
 int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
                            const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, double* out);
+/* x-gradient of the field of bemb200_evaluate_field, on the same elements, pairs, subdivision and rules:
+ *   grad p_sc(x) = sum_j p_j int_{E_j} grad_x dG/dn_y dS - v_j int_{E_j} grad_x G dS
+ * with rv = y - x, r = |rv|, w = s k, G' = (i w - 1/r) G, G'' = ((i w - 1/r)^2 + 1/r^2) G:
+ *   grad_x G = -G' rv / r,   grad_x dG/dn_y = -(G'/r) n - (G'' - G'/r) (rv.n) rv / r^2.
+ * Arguments, limits and checks are those of bemb200_evaluate_field.  out_grad [nsol * n_eval * 3] complex128 (host),
+ * solution-major, (d/dx, d/dy, d/dz) per point.  out_p (may be NULL) [nsol * n_eval] complex128 (host) receives the pressure
+ * with the bits of bemb200_evaluate_field for the same arguments.  A point within about 2^-30 element sizes of the surface (on
+ * it, in particular) gets NaN in the pressure and in all three components for every solution; the other points of the call
+ * are not affected.  Row s has the bits of the nsol = 1 call on solution s, for host and device input alike.  The particle
+ * velocity is grad p_total / (i s omega rho). */
+int bemb200_evaluate_field_gradient(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                                    const double* surface_pressure, const double* surface_velocity, int on_device,
+                                    uint64_t n_eval, const double* eval_pts, double* out_p, double* out_grad);
 
 /* ---- room-acoustics dense path (SURVEY 8f rank 3): math-bem/src/room_acoustics/solver.rs -------
  * Point collocation on a RoomMesh (math-xem-common/src/types.rs:185-192): nodes [n_nodes*3],

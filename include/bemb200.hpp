@@ -849,6 +849,29 @@ inline std::vector<Complex64> evaluate_field(const StagedMesh& mesh, const std::
           mesh.context().handle());
     return out;
 }
+// Gradient of the accurate scattered pressure (bemb200_evaluate_field_gradient) at n x 3 eval_points: n x 3 values
+// (d/dx, d/dy, d/dz per point); surface_velocity (v = dp/dn) may be empty.  pressure (may be null) receives the n values of
+// evaluate_field.  Points on the surface are NaN.
+inline std::vector<Complex64> evaluate_field_gradient(const StagedMesh& mesh, const std::vector<double>& eval_points,
+                                                      const std::vector<Complex64>& surface_pressure,
+                                                      const std::vector<Complex64>& surface_velocity, const PhysicsParams& physics,
+                                                      std::vector<Complex64>* pressure = nullptr) {
+    if (eval_points.empty() || eval_points.size() % 3 != 0)
+        throw std::invalid_argument("evaluate_field_gradient: eval_points must be n x 3, n >= 1");
+    if (surface_pressure.size() != mesh.num_dofs() || (!surface_velocity.empty() && surface_velocity.size() != mesh.num_dofs()))
+        throw std::invalid_argument("evaluate_field_gradient: surface vectors must have num_dofs entries");
+    const bemb200_physics phys = physics_abi(physics);
+    const size_t n = eval_points.size() / 3;
+    std::vector<Complex64> grad(3 * n);
+    if (pressure) pressure->assign(n, Complex64{});
+    const std::vector<Complex64> ps = mesh.in_dof_order(surface_pressure), vs = mesh.in_dof_order(surface_velocity);
+    check(bemb200_evaluate_field_gradient(mesh.handle(), &phys, 1, reinterpret_cast<const double*>(ps.data()),
+                                          vs.empty() ? nullptr : reinterpret_cast<const double*>(vs.data()), 0, n, eval_points.data(),
+                                          pressure ? reinterpret_cast<double*>(pressure->data()) : nullptr,
+                                          reinterpret_cast<double*>(grad.data())),
+          mesh.context().handle());
+    return grad;
+}
 
 struct LuError : std::runtime_error {  // lu.rs:15-21
     enum Kind { SingularMatrix, DimensionMismatch } kind;

@@ -130,6 +130,7 @@ SYMBOLS = {
     "bemb200_scattered_field_batch": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, C.c_int, C.c_uint64, _VP, _VP]),
     "bemb200_far_field": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, C.c_int, C.c_uint32, _VP, _VP]),
     "bemb200_evaluate_field": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, C.c_int, C.c_uint64, _VP, _VP]),
+    "bemb200_evaluate_field_gradient": (C.c_int, [_VP, C.POINTER(CPhysics), C.c_uint32, _VP, _VP, C.c_int, C.c_uint64, _VP, _VP, _VP]),
     "bemb200_bicgstab": (C.c_int, [_VP, _VP, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo)]),
     "bemb200_cgs": (C.c_int, [_VP, _VP, C.c_uint32, C.c_double, _VP, C.POINTER(CGmresInfo)]),
     "bemb200_lu_solve": (C.c_int, [_VP, _VP, _VP, C.c_int, C.POINTER(C.c_double)]),

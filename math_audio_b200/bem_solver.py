@@ -22,7 +22,8 @@ import numpy as np
 
 from . import bem
 from .incident import IncidentField
-from .postprocess import FieldPoint, compute_far_field, compute_total_field, surface_power
+from .postprocess import (FieldPoint, compute_far_field, compute_total_field, compute_total_field_gradient, particle_velocity,
+                          sound_intensity, surface_power)
 from .mesh import BC_PRESSURE, BC_VELOCITY, Mesh, generate_icosphere_mesh, generate_sphere_mesh
 from .types import PhysicsParams
 
@@ -144,6 +145,21 @@ class BemSolution:
         of the reference's rule; points on the surface are NaN."""
         return compute_total_field(points, self._staged(), self.surface_pressure, self._velocity_or_none(), self.incident_field,
                                    self.physics, accurate)
+
+    def evaluate_particle_velocity(self, points) -> np.ndarray:
+        """(M, 3) total particle velocity u = grad p_total / (i s omega rho) at the (M, 3) points: the incident gradient plus
+        the gradient of the accurate scattered field (``evaluate_field_gradient``, DESIGN.md 4.11) with the surface velocity
+        v_bar + Y p.  Points on the surface are NaN."""
+        _, g = compute_total_field_gradient(points, self._staged(), self.surface_pressure, self._velocity_or_none(),
+                                            self.incident_field, self.physics)
+        return particle_velocity(g, self.physics)
+
+    def evaluate_sound_intensity(self, points) -> np.ndarray:
+        """(M, 3) active intensity I = 1/2 Re(p_total conj(u)) of the total field at the (M, 3) points, from the accurate
+        evaluation as ``evaluate_particle_velocity``.  Points on the surface are NaN."""
+        p, g = compute_total_field_gradient(points, self._staged(), self.surface_pressure, self._velocity_or_none(),
+                                            self.incident_field, self.physics)
+        return sound_intensity(p, g, self.physics)
 
     def far_field(self, directions) -> np.ndarray:
         """Complex far-field amplitude F of the scattered / radiated field in the (M, 3) unit ``directions``:

@@ -669,11 +669,10 @@ __device__ __forceinline__ bool field_piece_accepted(const double* c, int et, co
     return d0 * d0 + d1 * d1 + d2 * d2 >= FE_ACCEPT * FE_ACCEPT * sub_area;
 }
 
-// Adds quadrature point q (TR13: q < 13; 4 x 4 Gauss: q < 16) of piece p to the lane's (int G, int dG/dn_y) sums.
+// Quadrature point q (TR13: q < 13; 4 x 4 Gauss: q < 16) of piece p: position y, weight x Jacobian wj and weight x normal wn.
 // en, jac: the Tri3 element's unit normal and |e1 x e2|.
-__device__ __forceinline__ void field_piece_point(const double* c, int et, const FieldPiece& p, int q, const double en[3], double jac,
-                                                  const double x[3], double wavruim, double& ar, double& ai, double& br, double& bi) {
-    double y[3], wj, wn[3];
+__device__ __forceinline__ void field_piece_geometry(const double* c, int et, const FieldPiece& p, int q, const double en[3], double jac,
+                                                     double y[3], double& wj, double wn[3]) {
     if (et == 3) {
         const double xi = BEMQ_TR13[q][0], eta = BEMQ_TR13[q][1];
         const double a = p.u[0] + xi * (p.u[2] - p.u[0]) + eta * (p.u[4] - p.u[0]);
@@ -690,6 +689,13 @@ __device__ __forceinline__ void field_piece_point(const double* c, int et, const
         wj = w * sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]);
         for (int k = 0; k < 3; ++k) wn[k] = w * nv[k];
     }
+}
+
+// Adds quadrature point q of piece p to the lane's (int G, int dG/dn_y) sums.
+__device__ __forceinline__ void field_piece_point(const double* c, int et, const FieldPiece& p, int q, const double en[3], double jac,
+                                                  const double x[3], double wavruim, double& ar, double& ai, double& br, double& bi) {
+    double y[3], wj, wn[3];
+    field_piece_geometry(c, et, p, q, en, jac, y, wj, wn);
     const double rv[3] = {y[0] - x[0], y[1] - x[1], y[2] - x[2]};
     const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
     double sn, cs;
@@ -790,6 +796,262 @@ __global__ void field_combine_kernel(const cplx* __restrict__ part, uint32_t nsp
         if (vs) t -= vs[at] * ab[2 * k];
     }
     out[i] = t;
+}
+
+// ---- field gradient (DESIGN.md section 4.11) ------------------------------------------------------------------------------
+// grad p_sc(x) = sum_j p_j int_{E_j} grad_x dG/dn_y dS - v_j int_{E_j} grad_x G dS, the x-gradient of the representation
+// above on the same pairs, pieces and rules.  With rv = y - x, G' = (i w - 1/r) G and G'' = ((i w - 1/r)^2 + 1/r^2) G:
+//   grad_x G = -G' rv / r,   grad_x dG/dn_y = -(G'/r) n - (G'' - G'/r) (rv.n) rv / r^2,  G'' - G'/r = (3/r^2 - 3 i w/r - w^2) G.
+// The (int G, int dG/dn_y) sums keep the pressure kernels' expressions, so the pressure has the bits of evaluate_field.
+constexpr int GRAD_CHUNK = 4;  // solutions per block of the gradient's regular pass (four complex accumulators each)
+
+// Adds the quadrature point's wj grad_x G to ga and grad_x dG/dn_y (normal wn) to gb, (re, im) per component.
+// zg = G, zgikr = G', dn = rv.wn / r.
+__device__ __forceinline__ void field_gradient_point(const double rv[3], double r, double wavruim, cplx zg, cplx zgikr, double wj,
+                                                     const double wn[3], double dn, double ga[6], double gb[6]) {
+    const double ir = 1.0 / r;
+    const cplx ca = zgikr * (wj * ir);                                                 // G' wj / r
+    const cplx g1 = zgikr * ir;                                                        // G' / r
+    const cplx h = zg * C(3.0 * ir * ir - wavruim * wavruim, -3.0 * wavruim * ir) * (dn * ir);  // (G'' - G'/r) (rv.wn) / r^2
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        ga[2 * k] -= ca.re * rv[k];
+        ga[2 * k + 1] -= ca.im * rv[k];
+        gb[2 * k] -= g1.re * wn[k] + h.re * rv[k];
+        gb[2 * k + 1] -= g1.im * wn[k] + h.im * rv[k];
+    }
+}
+
+// Regular pass of the gradient: field_regular_kernel's layout, tile and q order, for solutions [GRAD_CHUNK * blockIdx.y,
+// +GRAD_CHUNK).  Lane e forms a and b of (point w, element e) with field_regular_kernel's expressions and the geometry-only
+// grad a = sum wJ grad_x G, grad b = sum grad_x dG/dn_y w; each solution adds p b - v a and p grad b - v grad a.
+// part[z][s][m][c]: c = 0 the pressure, 1..3 the gradient's components.
+__global__ void __launch_bounds__(256)
+field_gradient_regular_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, const double4* __restrict__ elem,
+                              uint32_t n, uint32_t per_split, const double* __restrict__ eval, uint32_t n_eval, uint32_t nsol,
+                              const cplx* __restrict__ ps, const cplx* __restrict__ vs, double wavruim, cplx* __restrict__ part) {
+    __shared__ double sy[3][FF_NQ * FF_TILE], swj[FF_NQ * FF_TILE], swn[3][FF_NQ * FF_TILE];
+    __shared__ double4 sel[FF_TILE];
+    __shared__ cplx sp[GRAD_CHUNK][FF_TILE], sv[GRAD_CHUNK][FF_TILE];
+    __shared__ int snq[FF_TILE];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t m = blockIdx.x * FE_POINTS + warp;
+    const bool pt_ok = m < n_eval;
+    const double x0 = pt_ok ? eval[3ull * m] : 0.0, x1 = pt_ok ? eval[3ull * m + 1] : 0.0, x2 = pt_ok ? eval[3ull * m + 2] : 0.0;
+    const uint32_t s0 = blockIdx.y * GRAD_CHUNK;
+    const int cnt = (int)min((uint32_t)GRAD_CHUNK, nsol - s0);
+    const uint32_t j_begin = blockIdx.z * per_split, j_end = min(n, j_begin + per_split);
+    cplx acc[GRAD_CHUNK][4];
+#pragma unroll
+    for (int c = 0; c < GRAD_CHUNK; ++c)
+#pragma unroll
+        for (int d = 0; d < 4; ++d) acc[c][d] = C(0, 0);
+    for (uint32_t t0 = j_begin; t0 < j_end; t0 += FF_TILE) {
+        for (int i = threadIdx.x; i < FF_NQ * FF_TILE; i += blockDim.x) {
+            const int q = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            double y[3] = {0.0, 0.0, 0.0}, wj = 0.0, wn[3] = {0.0, 0.0, 0.0};
+            const int et = j < j_end ? etype[j] : 3;
+            if (j < j_end && (et == 4 || q < 7)) far_field_point(coords + 12ull * j, et, q, y, wj, wn);
+            if (q == 0) {
+                snq[e] = et == 4 ? 9 : 7;
+                sel[e] = j < j_end ? elem[j] : make_double4(0.0, 0.0, 0.0, 0.0);
+            }
+            for (int k = 0; k < 3; ++k) { sy[k][i] = y[k]; swn[k][i] = wn[k]; }
+            swj[i] = wj;
+        }
+        for (int i = threadIdx.x; i < GRAD_CHUNK * FF_TILE; i += blockDim.x) {
+            const int c = i / FF_TILE, e = i % FF_TILE;
+            const uint32_t j = t0 + e;
+            const bool ok = c < cnt && j < j_end;
+            const uint64_t at = (uint64_t)(s0 + c) * n + j;
+            sp[c][e] = ok ? ps[at] : C(0, 0);
+            sv[c][e] = (ok && vs) ? vs[at] : C(0, 0);
+        }
+        __syncthreads();
+        if (pt_ok && t0 + lane < j_end && field_pair_regular(x0, x1, x2, sel[lane])) {
+            double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+            double ga[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, gb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+            const int nq = snq[lane];
+            for (int q = 0; q < nq; ++q) {
+                const int at = q * FF_TILE + lane;
+                const double rv[3] = {sy[0][at] - x0, sy[1][at] - x1, sy[2][at] - x2};
+                const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
+                double sn, cs;
+                sincos(wavruim * r, &sn, &cs);
+                const double re1 = 4.0 * PI * r;
+                const cplx zg = C(cs / re1, sn / re1);
+                const cplx zgikr = zg * C(-1.0 / r, wavruim);
+                const double wn[3] = {swn[0][at], swn[1][at], swn[2][at]};
+                const double wj = swj[at], dn = (rv[0] * wn[0] + rv[1] * wn[1] + rv[2] * wn[2]) / r;
+                ar += wj * zg.re;
+                ai += wj * zg.im;
+                br += dn * zgikr.re;
+                bi += dn * zgikr.im;
+                field_gradient_point(rv, r, wavruim, zg, zgikr, wj, wn, dn, ga, gb);
+            }
+            const cplx a = C(ar, ai), b = C(br, bi);
+#pragma unroll
+            for (int c = 0; c < GRAD_CHUNK; ++c) {
+                if (c < cnt) {
+                    acc[c][0] += sp[c][lane] * b;
+                    if (vs) acc[c][0] -= sv[c][lane] * a;
+#pragma unroll
+                    for (int d = 0; d < 3; ++d) {
+                        acc[c][1 + d] += sp[c][lane] * C(gb[2 * d], gb[2 * d + 1]);
+                        if (vs) acc[c][1 + d] -= sv[c][lane] * C(ga[2 * d], ga[2 * d + 1]);
+                    }
+                }
+            }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int c = 0; c < GRAD_CHUNK; ++c) {
+#pragma unroll
+        for (int d = 0; d < 4; ++d) {
+#pragma unroll
+            for (int o = 16; o >= 1; o >>= 1) {
+                acc[c][d].re += __shfl_xor_sync(0xffffffffu, acc[c][d].re, o);
+                acc[c][d].im += __shfl_xor_sync(0xffffffffu, acc[c][d].im, o);
+            }
+        }
+    }
+    if (lane == 0 && pt_ok) {
+        const uint64_t base = (uint64_t)blockIdx.z * nsol;
+#pragma unroll
+        for (int c = 0; c < GRAD_CHUNK; ++c)
+            if (c < cnt)
+#pragma unroll
+                for (int d = 0; d < 4; ++d) part[((base + s0 + c) * n_eval + m) * 4 + d] = acc[c][d];
+    }
+}
+
+// Adds quadrature point q of piece p to the lane's (int G, int dG/dn_y) sums, with field_piece_point's expressions, and to
+// its gradient sums ga, gb.
+__device__ __forceinline__ void field_gradient_piece_point(const double* c, int et, const FieldPiece& p, int q, const double en[3],
+                                                           double jac, const double x[3], double wavruim, double& ar, double& ai,
+                                                           double& br, double& bi, double ga[6], double gb[6]) {
+    double y[3], wj, wn[3];
+    field_piece_geometry(c, et, p, q, en, jac, y, wj, wn);
+    const double rv[3] = {y[0] - x[0], y[1] - x[1], y[2] - x[2]};
+    const double r = sqrt(rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2]);
+    double sn, cs;
+    sincos(wavruim * r, &sn, &cs);
+    const double re1 = 4.0 * PI * r;
+    const cplx zg = C(cs / re1, sn / re1);
+    const cplx zgikr = zg * C(-1.0 / r, wavruim);
+    const double dn = (rv[0] * wn[0] + rv[1] * wn[1] + rv[2] * wn[2]) / r;
+    ar += wj * zg.re;
+    ai += wj * zg.im;
+    br += dn * zgikr.re;
+    bi += dn * zgikr.im;
+    field_gradient_point(rv, r, wavruim, zg, zgikr, wj, wn, dn, ga, gb);
+}
+
+// Near pass of the gradient: field_near_kernel's walk, piece pairing on half-warps and butterfly.  ab[8 i ..] = (int G,
+// int dG/dn_y, int grad_x G (3), int grad_x dG/dn_y (3)) of pair i, all NaN when a piece reaches FE_LMAX unaccepted.
+__global__ void __launch_bounds__(256)
+field_gradient_near_kernel(const double* __restrict__ coords, const uint8_t* __restrict__ etype, const double* __restrict__ eval,
+                           const uint32_t* __restrict__ pair_pt, const uint32_t* __restrict__ pair_el, uint64_t npairs, double wavruim,
+                           cplx* __restrict__ ab) {
+    const uint64_t i = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (i >= npairs) return;
+    const uint32_t m = pair_pt[i], j = pair_el[i];
+    const double x[3] = {eval[3ull * m], eval[3ull * m + 1], eval[3ull * m + 2]};
+    double c[12];
+    for (int k = 0; k < 12; ++k) c[k] = coords[12ull * j + k];
+    const int et = etype[j];
+    double en[3] = {0.0, 0.0, 0.0}, jac = 0.0;
+    if (et == 3) {
+        const double e1[3] = {c[3] - c[0], c[4] - c[1], c[5] - c[2]};
+        const double e2[3] = {c[6] - c[0], c[7] - c[1], c[8] - c[2]};
+        const double nv[3] = {e1[1] * e2[2] - e1[2] * e2[1], e1[2] * e2[0] - e1[0] * e2[2], e1[0] * e2[1] - e1[1] * e2[0]};
+        jac = sqrt(nv[0] * nv[0] + nv[1] * nv[1] + nv[2] * nv[2]);
+        for (int k = 0; k < 3; ++k) en[k] = nv[k] / jac;
+    }
+    const int nq = et == 3 ? 13 : 16;
+    const int half = lane >> 4, q = lane & 15;
+    double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+    double ga[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, gb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    bool failed = false, have_pending = false;
+    FieldPiece pending{};
+    uint64_t path = 0;
+    int lvl = 0;
+    for (;;) {
+        const FieldPiece cur = field_piece(et, path, lvl);
+        if (field_piece_accepted(c, et, cur, 0.5 * jac, x)) {
+            if (have_pending) {
+                if (q < nq) field_gradient_piece_point(c, et, half ? cur : pending, q, en, jac, x, wavruim, ar, ai, br, bi, ga, gb);
+                have_pending = false;
+            } else {
+                pending = cur;
+                have_pending = true;
+            }
+            while (lvl > 0 && ((path >> (2 * (lvl - 1))) & 3u) == 3u) {
+                path &= ~(3ull << (2 * (lvl - 1)));
+                --lvl;
+            }
+            if (lvl == 0) break;
+            path += 1ull << (2 * (lvl - 1));
+        } else if (lvl == FE_LMAX) {
+            failed = true;
+            break;
+        } else {
+            ++lvl;
+        }
+    }
+    if (have_pending && !failed && half == 0 && q < nq)
+        field_gradient_piece_point(c, et, pending, q, en, jac, x, wavruim, ar, ai, br, bi, ga, gb);
+    for (int o = 16; o >= 1; o >>= 1) {
+        ar += __shfl_xor_sync(0xffffffffu, ar, o);
+        ai += __shfl_xor_sync(0xffffffffu, ai, o);
+        br += __shfl_xor_sync(0xffffffffu, br, o);
+        bi += __shfl_xor_sync(0xffffffffu, bi, o);
+#pragma unroll
+        for (int k = 0; k < 6; ++k) {
+            ga[k] += __shfl_xor_sync(0xffffffffu, ga[k], o);
+            gb[k] += __shfl_xor_sync(0xffffffffu, gb[k], o);
+        }
+    }
+    if (lane == 0) {
+        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+        cplx* o = ab + 8 * i;
+        o[0] = failed ? C(nan, nan) : C(ar, ai);
+        o[1] = failed ? C(nan, nan) : C(br, bi);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            o[2 + k] = failed ? C(nan, nan) : C(ga[2 * k], ga[2 * k + 1]);
+            o[5 + k] = failed ? C(nan, nan) : C(gb[2 * k], gb[2 * k + 1]);
+        }
+    }
+}
+
+// field_combine_kernel for the four components: (s, m, c) = the split ranges of part in order, then the near pairs of m in
+// list order, p_j (int dG/dn_y, int grad_x dG/dn_y) - v_j (int G, int grad_x G).  c = 0 goes to out_p[s][m] (when given),
+// c = 1..3 to out_grad[s][m][c - 1].
+__global__ void field_gradient_combine_kernel(const cplx* __restrict__ part, uint32_t nsplit, uint32_t nsol, uint32_t n_eval, uint32_t n,
+                                              const uint64_t* __restrict__ off, const uint32_t* __restrict__ pair_el,
+                                              const cplx* __restrict__ ab, const cplx* __restrict__ ps, const cplx* __restrict__ vs,
+                                              cplx* __restrict__ out_p, cplx* __restrict__ out_grad) {
+    const uint64_t total = (uint64_t)nsol * n_eval * 4;
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const uint64_t sm = i >> 2, s = sm / n_eval, m = sm % n_eval;
+    const int c = (int)(i & 3u), ib = c == 0 ? 1 : 4 + c, ia = c == 0 ? 0 : 1 + c;
+    cplx t = part[i];
+    for (uint32_t z = 1; z < nsplit; ++z) t += part[z * total + i];
+    for (uint64_t k = off[m]; k < off[m + 1]; ++k) {
+        const uint64_t at = s * n + pair_el[k];
+        t += ps[at] * ab[8 * k + ib];
+        if (vs) t -= vs[at] * ab[8 * k + ia];
+    }
+    if (c == 0) {
+        if (out_p) out_p[sm] = t;
+    } else {
+        out_grad[3 * sm + c - 1] = t;
+    }
 }
 
 // b[s] = sys + inc[s] for the nrhs columns of a block (in place: out may be inc), the one IEEE add of bemb200_sweep_next
@@ -1129,8 +1391,36 @@ extern "C" int bemb200_far_field(const bemb200_staged_mesh* sm, const bemb200_ph
     return BEMB200_OK;
 }
 
-extern "C" int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
-                                      const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, double* out) {
+namespace {
+
+// What bemb200_evaluate_field and bemb200_evaluate_field_gradient share: the argument checks, then, under the context's lock,
+// the point upload, the element data, the exactly sized near list and the split of the elements for the regular pass.
+struct FieldSetup {
+    std::unique_lock<std::mutex> lk;
+    struct Allocs {  // stream-ordered frees after the last kernel, on every return path (before the lock is released)
+        cudaStream_t s = nullptr;
+        std::vector<void*> p;
+        cudaError_t get(void** out, size_t bytes) {
+            cudaError_t e = cudaMallocAsync(out, bytes ? bytes : 1, s);
+            if (e == cudaSuccess) p.push_back(*out);
+            return e;
+        }
+        ~Allocs() { for (void* q : p) cudaFreeAsync(q, s); }
+    } mem;
+    uint32_t n = 0, ne = 0, pt_blocks = 0, nsplit = 0, per_split = 0;
+    double wavruim = 0.0;
+    double* dev = nullptr;                // the points, [ne][3]
+    double4* elem = nullptr;              // field_element_kernel's element data
+    uint64_t npairs = 0;
+    uint64_t* off = nullptr;              // near pairs of point m at [off[m], off[m + 1])
+    uint32_t *pair_pt = nullptr, *pair_el = nullptr;
+};
+
+// Checks the arguments (out: the output the entry requires) before a device is touched, then sets fs up.  what: the entry's
+// name for error messages.
+int field_setup(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, const double* out,
+                const char* what, FieldSetup& fs) {
     // every argument is checked before a device is touched (the staged mesh last, so each check answers for itself)
     bemb200_ctx* ctx = sm ? sm->ctx : nullptr;
     if (!phys || !surface_pressure || !eval_pts || !out) return set_error(ctx, BEMB200_EINVAL, "NULL argument");
@@ -1142,45 +1432,35 @@ extern "C" int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb2
     if (!sm) return set_error(nullptr, BEMB200_EINVAL, "NULL staged mesh");
     if (on_device && (!device_ptr_on(ctx->device, surface_pressure) || (surface_velocity && !device_ptr_on(ctx->device, surface_velocity))))
         return set_error(ctx, BEMB200_EINVAL, "surface values are not device memory of the staged mesh's device");
-    std::lock_guard<std::mutex> lk(ctx->mu);
+    fs.lk = std::unique_lock<std::mutex>(ctx->mu);
     BEMB_CUDA(ctx, cudaSetDevice(ctx->device));
-    const uint32_t n = sm->dm.n, ne = (uint32_t)n_eval;
-    const double wavruim = phys->wave_number * phys->harmonic_factor;
     cudaStream_t s = ctx->stream;
-    struct Allocs {  // stream-ordered frees after the last kernel, on every return path
-        cudaStream_t s;
-        std::vector<void*> p;
-        cudaError_t get(void** out, size_t bytes) {
-            cudaError_t e = cudaMallocAsync(out, bytes ? bytes : 1, s);
-            if (e == cudaSuccess) p.push_back(*out);
-            return e;
-        }
-        ~Allocs() { for (void* q : p) cudaFreeAsync(q, s); }
-    } mem{s, {}};
+    fs.mem.s = s;
+    const uint32_t n = sm->dm.n, ne = (uint32_t)n_eval;
+    fs.n = n;
+    fs.ne = ne;
+    fs.wavruim = phys->wave_number * phys->harmonic_factor;
     // The regular pass splits the elements as far_field does (depending on n_eval and n only, so a solution's bits do not
     // depend on nsol).
     const uint32_t pt_blocks = (ne + FE_POINTS - 1) / FE_POINTS, tiles = (n + FF_TILE - 1) / FF_TILE;
     uint32_t nsplit = (1184u + pt_blocks - 1) / pt_blocks;
     nsplit = std::max(1u, std::min({nsplit, 32u, tiles}));
     const uint32_t per_split = std::max(1u, (tiles + nsplit - 1) / nsplit) * FF_TILE;
-    nsplit = std::max(1u, (n + per_split - 1) / per_split);
-    const size_t nout = (size_t)nsol * ne;
-    double *dev = nullptr;
-    double4* elem = nullptr;
+    fs.pt_blocks = pt_blocks;
+    fs.nsplit = std::max(1u, (n + per_split - 1) / per_split);
+    fs.per_split = per_split;
     uint32_t* counts = nullptr;
-    cplx *part = nullptr, *dout = nullptr, *tmp_p = nullptr, *tmp_v = nullptr;
-    const cplx *dps = nullptr, *dvs = nullptr;
-    cudaError_t e = mem.get((void**)&dev, (size_t)ne * 3 * sizeof(double));
-    if (e == cudaSuccess) e = mem.get((void**)&elem, (size_t)n * sizeof(double4));
-    if (e == cudaSuccess) e = mem.get((void**)&counts, (size_t)ne * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dev, eval_pts, (size_t)ne * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
+    cudaError_t e = fs.mem.get((void**)&fs.dev, (size_t)ne * 3 * sizeof(double));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&fs.elem, (size_t)n * sizeof(double4));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&counts, (size_t)ne * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(fs.dev, eval_pts, (size_t)ne * 3 * sizeof(double), cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess && n) {
-        field_element_kernel<<<(n + 255) / 256, 256, 0, s>>>(sm->dm.coords, sm->dm.etype, n, elem);
+        field_element_kernel<<<(n + 255) / 256, 256, 0, s>>>(sm->dm.coords, sm->dm.etype, n, fs.elem);
         e = cudaGetLastError();
     }
     const unsigned warp_blocks = (unsigned)(((uint64_t)ne * 32 + 255) / 256);
     if (e == cudaSuccess) {
-        field_near_count_kernel<<<warp_blocks, 256, 0, s>>>(elem, n, dev, ne, counts);
+        field_near_count_kernel<<<warp_blocks, 256, 0, s>>>(fs.elem, n, fs.dev, ne, counts);
         e = cudaGetLastError();
     }
     // near list sized exactly: counts -> host prefix sum -> offsets
@@ -1188,47 +1468,108 @@ extern "C" int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb2
     std::vector<uint64_t> hoff((size_t)ne + 1, 0);
     if (e == cudaSuccess) e = cudaMemcpyAsync(hcount.data(), counts, (size_t)ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) return cuda_fail(ctx, e, "evaluate_field (near count)");
+    if (e != cudaSuccess) return cuda_fail(ctx, e, (std::string(what) + " (near count)").c_str());
     for (uint32_t m = 0; m < ne; ++m) hoff[m + 1] = hoff[m] + hcount[m];
-    const uint64_t npairs = hoff[ne];
-    uint64_t* off = nullptr;
-    uint32_t *pair_pt = nullptr, *pair_el = nullptr;
-    cplx* ab = nullptr;
-    e = mem.get((void**)&off, hoff.size() * sizeof(uint64_t));
-    if (e == cudaSuccess) e = mem.get((void**)&pair_pt, npairs * sizeof(uint32_t));
-    if (e == cudaSuccess) e = mem.get((void**)&pair_el, npairs * sizeof(uint32_t));
-    if (e == cudaSuccess) e = mem.get((void**)&ab, 2 * npairs * sizeof(cplx));
-    if (e == cudaSuccess) e = mem.get((void**)&part, nout * nsplit * sizeof(cplx));
-    if (e == cudaSuccess) e = mem.get((void**)&dout, nout * sizeof(cplx));
-    if (e == cudaSuccess) e = cudaMemcpyAsync(off, hoff.data(), hoff.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess && npairs) {
-        field_near_fill_kernel<<<warp_blocks, 256, 0, s>>>(elem, n, dev, ne, off, pair_pt, pair_el);
+    fs.npairs = hoff[ne];
+    e = fs.mem.get((void**)&fs.off, hoff.size() * sizeof(uint64_t));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&fs.pair_pt, fs.npairs * sizeof(uint32_t));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&fs.pair_el, fs.npairs * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(fs.off, hoff.data(), hoff.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && fs.npairs) {
+        field_near_fill_kernel<<<warp_blocks, 256, 0, s>>>(fs.elem, n, fs.dev, ne, fs.off, fs.pair_pt, fs.pair_el);
         e = cudaGetLastError();
-        if (e == cudaSuccess) {
-            field_near_kernel<<<(unsigned)((npairs * 32 + 255) / 256), 256, 0, s>>>(sm->dm.coords, sm->dm.etype, dev, pair_pt, pair_el,
-                                                                                  npairs, wavruim, ab);
-            e = cudaGetLastError();
-        }
     }
-    if (e == cudaSuccess) {
-        e = solutions_on_device(surface_pressure, on_device, (size_t)nsol * n, s, &tmp_p, &dps);
-        if (tmp_p) mem.p.push_back(tmp_p);
-    }
+    if (e != cudaSuccess) return cuda_fail(ctx, e, what);
+    return BEMB200_OK;
+}
+
+// The surface values of the call on the device (uploads owned by fs).
+cudaError_t field_solutions(FieldSetup& fs, const double* surface_pressure, const double* surface_velocity, int on_device, size_t count,
+                            const cplx** dps, const cplx** dvs) {
+    cplx *tmp_p = nullptr, *tmp_v = nullptr;
+    cudaError_t e = solutions_on_device(surface_pressure, on_device, count, fs.mem.s, &tmp_p, dps);
+    if (tmp_p) fs.mem.p.push_back(tmp_p);
     if (e == cudaSuccess && surface_velocity) {
-        e = solutions_on_device(surface_velocity, on_device, (size_t)nsol * n, s, &tmp_v, &dvs);
-        if (tmp_v) mem.p.push_back(tmp_v);
+        e = solutions_on_device(surface_velocity, on_device, count, fs.mem.s, &tmp_v, dvs);
+        if (tmp_v) fs.mem.p.push_back(tmp_v);
     }
+    return e;
+}
+
+}  // namespace
+
+extern "C" int bemb200_evaluate_field(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol, const double* surface_pressure,
+                                      const double* surface_velocity, int on_device, uint64_t n_eval, const double* eval_pts, double* out) {
+    FieldSetup fs;
+    const int rc = field_setup(sm, phys, nsol, surface_pressure, surface_velocity, on_device, n_eval, eval_pts, out, "evaluate_field", fs);
+    if (rc != BEMB200_OK) return rc;
+    bemb200_ctx* ctx = sm->ctx;
+    cudaStream_t s = ctx->stream;
+    const uint32_t n = fs.n, ne = fs.ne;
+    const size_t nout = (size_t)nsol * ne;
+    cplx *ab = nullptr, *part = nullptr, *dout = nullptr;
+    const cplx *dps = nullptr, *dvs = nullptr;
+    cudaError_t e = fs.mem.get((void**)&ab, 2 * fs.npairs * sizeof(cplx));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&part, nout * fs.nsplit * sizeof(cplx));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&dout, nout * sizeof(cplx));
+    if (e == cudaSuccess && fs.npairs) {
+        field_near_kernel<<<(unsigned)((fs.npairs * 32 + 255) / 256), 256, 0, s>>>(sm->dm.coords, sm->dm.etype, fs.dev, fs.pair_pt,
+                                                                                     fs.pair_el, fs.npairs, fs.wavruim, ab);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = field_solutions(fs, surface_pressure, surface_velocity, on_device, (size_t)nsol * n, &dps, &dvs);
     if (e == cudaSuccess) {
-        field_regular_kernel<<<dim3(pt_blocks, (nsol + SOL_CHUNK - 1) / SOL_CHUNK, nsplit), 256, 0, s>>>(
-            sm->dm.coords, sm->dm.etype, elem, n, per_split, dev, ne, nsol, dps, dvs, wavruim, part);
+        field_regular_kernel<<<dim3(fs.pt_blocks, (nsol + SOL_CHUNK - 1) / SOL_CHUNK, fs.nsplit), 256, 0, s>>>(
+            sm->dm.coords, sm->dm.etype, fs.elem, n, fs.per_split, fs.dev, ne, nsol, dps, dvs, fs.wavruim, part);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) {
-        field_combine_kernel<<<(unsigned)((nout + 255) / 256), 256, 0, s>>>(part, nsplit, nsol, ne, n, off, pair_el, ab, dps, dvs, dout);
+        field_combine_kernel<<<(unsigned)((nout + 255) / 256), 256, 0, s>>>(part, fs.nsplit, nsol, ne, n, fs.off, fs.pair_el, ab, dps, dvs,
+                                                                            dout);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     if (e != cudaSuccess) return cuda_fail(ctx, e, "evaluate_field");
+    return BEMB200_OK;
+}
+
+extern "C" int bemb200_evaluate_field_gradient(const bemb200_staged_mesh* sm, const bemb200_physics* phys, uint32_t nsol,
+                                               const double* surface_pressure, const double* surface_velocity, int on_device,
+                                               uint64_t n_eval, const double* eval_pts, double* out_p, double* out_grad) {
+    FieldSetup fs;
+    const int rc = field_setup(sm, phys, nsol, surface_pressure, surface_velocity, on_device, n_eval, eval_pts, out_grad,
+                               "evaluate_field_gradient", fs);
+    if (rc != BEMB200_OK) return rc;
+    bemb200_ctx* ctx = sm->ctx;
+    cudaStream_t s = ctx->stream;
+    const uint32_t n = fs.n, ne = fs.ne;
+    const size_t nout = (size_t)nsol * ne;
+    cplx *ab = nullptr, *part = nullptr, *dp = nullptr, *dgrad = nullptr;
+    const cplx *dps = nullptr, *dvs = nullptr;
+    cudaError_t e = fs.mem.get((void**)&ab, 8 * fs.npairs * sizeof(cplx));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&part, 4 * nout * fs.nsplit * sizeof(cplx));
+    if (e == cudaSuccess) e = fs.mem.get((void**)&dgrad, 3 * nout * sizeof(cplx));
+    if (e == cudaSuccess && out_p) e = fs.mem.get((void**)&dp, nout * sizeof(cplx));
+    if (e == cudaSuccess && fs.npairs) {
+        field_gradient_near_kernel<<<(unsigned)((fs.npairs * 32 + 255) / 256), 256, 0, s>>>(sm->dm.coords, sm->dm.etype, fs.dev, fs.pair_pt,
+                                                                                              fs.pair_el, fs.npairs, fs.wavruim, ab);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = field_solutions(fs, surface_pressure, surface_velocity, on_device, (size_t)nsol * n, &dps, &dvs);
+    if (e == cudaSuccess) {
+        field_gradient_regular_kernel<<<dim3(fs.pt_blocks, (nsol + GRAD_CHUNK - 1) / GRAD_CHUNK, fs.nsplit), 256, 0, s>>>(
+            sm->dm.coords, sm->dm.etype, fs.elem, n, fs.per_split, fs.dev, ne, nsol, dps, dvs, fs.wavruim, part);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) {
+        field_gradient_combine_kernel<<<(unsigned)((4 * nout + 255) / 256), 256, 0, s>>>(part, fs.nsplit, nsol, ne, n, fs.off, fs.pair_el,
+                                                                                         ab, dps, dvs, dp, dgrad);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_grad, dgrad, 3 * nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && out_p) e = cudaMemcpyAsync(out_p, dp, nout * sizeof(cplx), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "evaluate_field_gradient");
     return BEMB200_OK;
 }

@@ -54,6 +54,25 @@ class IncidentField:
             p[ok] += s * g
         return p
 
+    def evaluate_gradient(self, points: np.ndarray, physics: PhysicsParams) -> np.ndarray:
+        """(M, 3) gradient of ``evaluate_pressure`` as written (wave number k): i k d p for a plane wave, s (i k - 1/r) G
+        (x - x_s) / r for a point source (0 where ``evaluate_pressure`` skips the source, r <= 1e-10)."""
+        k = physics.wave_number
+        points = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+        g = np.zeros(points.shape, dtype=np.complex128)
+        for d, amp in self.plane_waves:
+            kdotx = k * (d[0] * points[:, 0] + d[1] * points[:, 1] + d[2] * points[:, 2])
+            p = amp * (np.cos(kdotx) + 1j * np.sin(kdotx))
+            g += (1j * k * p)[:, None] * np.asarray(d, dtype=np.float64)[None, :]
+        for pos, s in self.point_sources:
+            dv = points - np.asarray(pos, dtype=np.float64)[None, :]
+            r = np.sqrt(dv[:, 0] * dv[:, 0] + dv[:, 1] * dv[:, 1] + dv[:, 2] * dv[:, 2])
+            ok = r > 1e-10
+            kr = k * r[ok]
+            gr = (np.cos(kr) + 1j * np.sin(kr)) / (4.0 * math.pi * r[ok])
+            g[ok] += (s * (1j * k - 1.0 / r[ok]) * gr / r[ok])[:, None] * dv[ok]
+        return g
+
     def evaluate_normal_derivative(self, points: np.ndarray, normals: np.ndarray, physics: PhysicsParams) -> np.ndarray:
         k = physics.wave_number
         out = np.zeros(points.shape[0], dtype=np.complex128)

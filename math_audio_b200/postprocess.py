@@ -5,7 +5,8 @@
 
 Beyond the reference: the complex far-field amplitude with the surface-velocity term (``compute_far_field``, device) and the
 host-side quantities built on it -- ``sphere_quadrature``, ``far_field_power``, ``surface_power`` and ``directivity_index``
-(DESIGN.md 4.9)."""
+(DESIGN.md 4.9); the gradient of the accurate field (``evaluate_field_gradient``, device) and the particle velocity and
+active intensity derived from it (DESIGN.md 4.11)."""
 from __future__ import annotations
 
 import math
@@ -103,6 +104,34 @@ def compute_total_field(eval_points, staged: bem.StagedMesh, surface_pressure, s
     else:
         p_sc = bem.compute_scattered_field(pts, staged, surface_pressure, surface_velocity, physics)
     return [FieldPoint(pts[i].copy(), complex(p_inc[i]), complex(p_sc[i])) for i in range(pts.shape[0])]
+
+
+def evaluate_field_gradient(eval_points, staged: bem.StagedMesh, surface_pressure, surface_velocity, physics: PhysicsParams,
+                            nsol: Optional[int] = None, with_pressure: bool = False):
+    """Gradient of the accurate scattered pressure (device; ``bem.evaluate_field_gradient``)."""
+    return bem.evaluate_field_gradient(eval_points, staged, surface_pressure, surface_velocity, physics, nsol, with_pressure)
+
+
+def compute_total_field_gradient(eval_points, staged: bem.StagedMesh, surface_pressure, surface_velocity: Optional[np.ndarray],
+                                 incident_field: IncidentField, physics: PhysicsParams):
+    """(p_total (M,), grad p_total (M, 3)) at the (M, 3) points: the incident field and its gradient (host, O(M)) plus the
+    accurate scattered field and its gradient (device, ``evaluate_field_gradient``)."""
+    pts = np.ascontiguousarray(eval_points, dtype=np.float64).reshape(-1, 3)
+    p_sc, g_sc = bem.evaluate_field_gradient(pts, staged, surface_pressure, surface_velocity, physics, with_pressure=True)
+    return incident_field.evaluate_pressure(pts, physics) + p_sc, incident_field.evaluate_gradient(pts, physics) + g_sc
+
+
+def particle_velocity(grad_p, physics: PhysicsParams) -> np.ndarray:
+    """Particle velocity u = grad p / (i s omega rho) (Euler's equation; s = harmonic_factor, time factor exp(-i s omega t))
+    of complex pressure gradients (..., 3)."""
+    return np.asarray(grad_p, dtype=np.complex128) / (1j * physics.harmonic_factor * physics.omega * physics.density)
+
+
+def sound_intensity(p, grad_p, physics: PhysicsParams) -> np.ndarray:
+    """Active (time-averaged) intensity I = 1/2 Re(p conj(u)) (..., 3) of pressures p (...) and their gradients (..., 3);
+    on the surface I.n = -(s / (2 omega rho)) Im(p conj(dp/dn)), the sign of ``surface_power``."""
+    u = particle_velocity(grad_p, physics)
+    return 0.5 * np.real(np.asarray(p, dtype=np.complex128)[..., None] * np.conj(u))
 
 
 def compute_rcs(surface_pressure, staged: bem.StagedMesh, direction, physics: PhysicsParams):

@@ -117,6 +117,9 @@ extern "C" {
                              surface_velocity: *const f64, on_device: c_int, n_dirs: u32, dirs: *const f64, out: *mut f64) -> c_int;
     pub fn bemb200_evaluate_field(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, nsol: u32, surface_pressure: *const f64,
                                   surface_velocity: *const f64, on_device: c_int, n_eval: u64, eval_pts: *const f64, out: *mut f64) -> c_int;
+    pub fn bemb200_evaluate_field_gradient(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, nsol: u32,
+                                           surface_pressure: *const f64, surface_velocity: *const f64, on_device: c_int, n_eval: u64,
+                                           eval_pts: *const f64, out_p: *mut f64, out_grad: *mut f64) -> c_int;
     pub fn bemb200_incident_rhs(sm: *const bemb200_staged_mesh, phys: *const bemb200_physics, beta_re: f64, beta_im: f64,
                                 n_sources: u32, kinds: *const i32, vecs: *const f64, amps: *const f64, rhs_host: *mut f64,
                                 rhs_dev: *mut f64) -> c_int;
