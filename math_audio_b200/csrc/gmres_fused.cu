@@ -27,8 +27,8 @@
 // The convergence test of column j-1 is therefore taken one matvec late: a solve costs one A-product more
 // than the reference's count, the reported iteration/restart numbers are the reference's.
 #include <cooperative_groups.h>
-#include <atomic>
 #include <cstring>
+#include <mutex>
 
 #include "api_internal.h"
 #include "gmres_fused.h"
@@ -914,15 +914,23 @@ uint32_t fused_pick_rblk(uint32_t S) {
 }
 
 cudaError_t launch_gmres_fused(const FusedParams& p, int grid, size_t smem, bool polite, cudaStream_t s) {
-    static std::atomic<unsigned long long> attr_done[64];
+    // The shared-memory limit is an attribute of the kernel on the device, and the ranks of a group that share a device
+    // launch from their own host threads, each with its own split and so its own size.  Raised under a lock and never
+    // lowered: an unlocked check-then-set let one rank lower the limit below what another had just checked, that rank's
+    // launch failed, and the ranks already launched waited for it until the peer timeout.
+    static std::mutex attr_mu[64];
+    static size_t attr_done[64];
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64) dev = 63;
-    if (attr_done[dev].load() < smem) {
-        cudaError_t e = cudaFuncSetAttribute(gmres_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gmres_fused_kernel_polite, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr_done[dev].store(smem);
+    {
+        std::lock_guard<std::mutex> lk(attr_mu[dev]);
+        if (attr_done[dev] < smem) {
+            cudaError_t e = cudaFuncSetAttribute(gmres_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(gmres_fused_kernel_polite, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+            attr_done[dev] = smem;
+        }
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid, 1, 1);
